@@ -1,7 +1,10 @@
 #!/usr/bin/env python
 """Benchmark of the GNAN hot path (BASELINE.json metric: fwd+bwd graphs/s on graph tasks & nodes/s on node tasks, 1-8 B200).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload mol|mutag|cora|pubmed|arxiv] [--impl reference] ...
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload mol|mutag|cora|pubmed|arxiv] [--impl reference] [--dump-outputs DIR] ...
+
+`--steps K` is the number of timed steps of both GPU legs (device-resident and e2e) of every workload; the per-kernel attribution
+pass runs min(K, 10) steps, and the CPU reference arm runs at least 2 steps within its time budget.
 
 A step is forward + loss + backward + Adam step (trainer.py:48-67). Workloads = BASELINE.json configs:
   mol     configs[4]  32768 molecule-shaped graphs (10-100 nodes) per step and rank, GPU all-pairs hop preprocessing of the
@@ -440,7 +443,29 @@ KERNEL_NAMES = {
 COLLECTIVES = ("allgather_rows", "reduce_scatter_rows", "allreduce_gradients")
 
 
-def run_workload(args, env, name, *, steps, warmup, classes=0, compare_legs=False, cpu_budget_s=60.0):
+DUMP_SAMPLE = 1 << 20   # elements kept of a larger dumped array
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each tensor as <out_dir>/<name>.npy, float64 as float64 and anything else as float32. An array of more than DUMP_SAMPLE
+    elements is reduced to a fixed seeded sample of its flattened values: the same positions in every run, so that two builds can be
+    compared output for output. Refuses to write more than DUMP_MAX_BYTES in all."""
+    out = {}
+    for nm, t in arrays.items():
+        a = t.detach().cpu().numpy().astype(np.float64 if t.dtype == torch.float64 else np.float32)
+        if a.size > DUMP_SAMPLE:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))]
+        out[nm] = a
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_MAX_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for nm, a in out.items():
+        np.save(os.path.join(out_dir, nm + ".npy"), a)
+
+
+def run_workload(args, env, name, *, steps, warmup, classes=0, compare_legs=False, cpu_budget_s=60.0, dump_dir=None):
     import torch.distributed as dist
     from gnan_b200 import ops
     from gnan_b200 import dist as gdist
@@ -468,6 +493,7 @@ def run_workload(args, env, name, *, steps, warmup, classes=0, compare_legs=Fals
     scaling = "strong" if sharded else "weak"
     fg = gdist.FlatGradients(model.parameters()) if world > 1 and wl.name != "cora" else None
     zero_grads = (lambda: fg.zero()) if fg is not None else (lambda: opt.zero_grad(set_to_none=True))
+    last_out = [None]                                           # the model output of the latest step (a captured step rewrites it)
 
     # ---- device-resident inputs and the step ------------------------------------------------------------------------
     if wl.kind == "node":
@@ -512,6 +538,7 @@ def run_workload(args, env, name, *, steps, warmup, classes=0, compare_legs=Fals
                 out = gdist.row_sharded_forward(model, data.x, data.hop_data, sizes, x_compressed=data.x_compressed)
             else:
                 out = model.forward(data)
+            last_out[0] = out.detach()
             # masked cross entropy: value and the [N,C] output gradient from one kernel (trainer.py:52-66)
             return ops.cross_entropy_rows(out, yl_d, rows=idx_d, scale=1.0 / n_train)
         after_bwd = (lambda: fg.all_reduce()) if sharded else None
@@ -586,7 +613,9 @@ def run_workload(args, env, name, *, steps, warmup, classes=0, compare_legs=Fals
                                     rscale=not pair_stats, pair_stats=pair_stats)
                 data.x_compressed = c
                 apsp_status[:] = [data.status]
-            return ops.bce_with_logits(model(data).flatten(), data.y)   # model(data): [B,1]; BCEWithLogitsLoss, value + gradient in one kernel
+            out = model(data)
+            last_out[0] = out.detach()
+            return ops.bce_with_logits(out.flatten(), data.y)           # model(data): [B,1]; BCEWithLogitsLoss, value + gradient in one kernel
         after_bwd = (lambda: fg.all_reduce(average=True)) if world > 1 else None
         rows_local = wl.n
         n_train_local = None
@@ -686,8 +715,12 @@ def run_workload(args, env, name, *, steps, warmup, classes=0, compare_legs=Fals
     barrier(); torch.cuda.synchronize()
     for a, b in ev:
         flush.fill_(1)                                              # evict L2 (126 MB) between timed steps
-        a.record(); run_step(data_d); b.record()
+        a.record(); loss = run_step(data_d); b.record()
     torch.cuda.synchronize(); barrier()
+    if dump_dir is not None and rank == 0:                          # before the passes below move the weights again
+        named = list(model.named_parameters())
+        dump_outputs(dump_dir, {"loss": loss, "output": last_out[0], **{f"grad.{k}": p.grad for k, p in named if p.grad is not None},
+                                **{f"param.{k}": p for k, p in named}})
     launches = lib.gnan_launch_count() - launches0
     if graphed is not None:
         launches = launches_per_step * steps                        # replayed launches are not seen by the library's counter
@@ -816,16 +849,14 @@ def run_workload(args, env, name, *, steps, warmup, classes=0, compare_legs=Fals
 
     e2e_loop(3)
     barrier(); torch.cuda.synchronize()
-    # sub-millisecond steps: at least 100 of them (20 steps of 1 ms are 20 ms of wall clock: host scheduling noise of +-20 %)
-    e2e_steps = steps if ms_per_step >= 5.0 else max(steps, 100)
     a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     a.record()
-    e2e_loop(e2e_steps)
+    e2e_loop(steps)
     b.record(); torch.cuda.synchronize(); barrier()
     t = torch.tensor([a.elapsed_time(b)], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
-    e2e_val = total_units * e2e_steps / (float(t.item()) / 1e3)
+    e2e_val = total_units * steps / (float(t.item()) / 1e3)
 
     rec = None
     if rank == 0:
@@ -899,7 +930,7 @@ def run_workload(args, env, name, *, steps, warmup, classes=0, compare_legs=Fals
                 "LocalEdges (uint8 endpoints inside their graph + per-graph edge offsets): the BFS kernel builds each graph's adjacency itself"
                 + (" and accumulates the pair statistics of the graph readout (undirected graphs)" if pair_stats else "")
                 if local_edges else "int64 [2,E] edge_index: gnan_build_csr + BFS")} if in_step_apsp else {})),
-            "e2e": {"value": e2e_val, "unit": wl.unit, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": 4, "steps": e2e_steps,
+            "e2e": {"value": e2e_val, "unit": wl.unit, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": 4, "steps": steps,
                     "note": "hop matrix kept device-resident in the e2e leg (too large to stage in pinned host memory)" if (wl.kind == "node" and big) else None},
             "gpu_launches": int(launches), "cuda_graph": graphed is not None,
             "roofline": roof, "aggregation": agg, "strict_fp32": strict, "dense_kernels": dense,
@@ -1010,6 +1041,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-cuda-graph", action="store_true", help="run the step eagerly instead of replaying a captured CUDA graph")
     ap.add_argument("--subs", default=None, help="comma-separated sub-record workloads (default: cora,mutag,pubmed,arxiv at N=1; arxiv at N>1)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps of the headline workload, write what its last timed step computed (loss, model output, "
+                         "parameter gradients, updated parameters) as DIR/<name>.npy; arrays over 1 Mi elements as a fixed seeded sample; "
+                         "with row-sharded ranks, the output is rank 0's rows, as row_sharded_forward returns them there")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -1029,13 +1064,13 @@ def main():
 
     primary = args.workload or "mol"
     line = run_workload(args, env, primary, steps=args.steps, warmup=args.warmup, classes=args.classes,
-                        compare_legs=(primary == "cora" and not args.headline_only), cpu_budget_s=90.0)
+                        compare_legs=(primary == "cora" and not args.headline_only), cpu_budget_s=90.0, dump_dir=args.dump_outputs)
     subs, parity = {}, None
     if args.workload is None and not args.headline_only:
         names = (args.subs.split(",") if args.subs else (["cora", "mutag", "pubmed", "arxiv"] if world == 1 else ["arxiv"]))
         for nm in [n for n in names if n]:
             try:
-                subs[nm] = run_workload(args, env, nm, steps=min(args.steps, 10), warmup=3, compare_legs=(nm == "cora"), cpu_budget_s=45.0)
+                subs[nm] = run_workload(args, env, nm, steps=args.steps, warmup=3, compare_legs=(nm == "cora"), cpu_budget_s=45.0)
             except Exception as exc:                                # pragma: no cover
                 print(f"[bench] sub-record {nm} failed: {exc!r}", file=sys.stderr)
                 subs[nm] = {"error": repr(exc)}

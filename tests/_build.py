@@ -2,7 +2,7 @@
 import torch
 
 
-def build_module(z, device=None):
+def build_module(z, device=None, load=True):
     v = z["variant"]
     sd = {k: torch.tensor(val) for k, val in z["sd"].items()}
     if v == "batched":
@@ -21,7 +21,8 @@ def build_module(z, device=None):
         from gnan_b200.models import GNAN
         m = GNAN(z["K"], z["C"], num_layers=z["L"], hidden_channels=z["H"], bias=z["bias"],
                  normalize_rho=z["normalize_rho"], rho_per_feature=z["rho_per_feature"])
-    m.load_state_dict(sd, strict=True)
+    if load:
+        m.load_state_dict(sd, strict=True)
     if device is not None:
         m = m.to(device)
     return m

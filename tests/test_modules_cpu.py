@@ -378,48 +378,30 @@ def test_reference_format_inputs_are_converted_once_and_again_after_an_in_place_
         _inputs.resolve(SimpleNamespace(x=torch.rand(4, 2)), "cpu")
 
 
-@pytest.mark.skipif(not __import__("os").path.exists("/root/reference/GNAN.py"), reason="the unmodified reference is only present in the build container")
-@pytest.mark.parametrize("variant", ["gnanpy_tensor_node", "gnanpy_tensor_graph", "gnanpy_gnan", "gnanpy_gnan_rho_per_feature", "models_tensor_readout",
-                                     "models_tensor_node", "models_gnan", "batched"])
-def test_checkpoints_round_trip_with_the_unmodified_reference_modules(variant):
-    """A checkpoint written by a gnan_b200 module loads STRICTLY into the unmodified reference class built with the same arguments
-    (and back), and the reference's per-feature sub-modules then evaluate like ours: the drop-in claim for state_dicts in both directions
-    (the golden-file test covers reference -> gnan_b200 only)."""
-    from oracle import pyg_shim
-    gnan_py, models_py, _, batched_cls = pyg_shim.import_reference("/root/reference")
-    from gnan_b200 import GNAN as g, batched as b, models as mo
-    K, C, L, H = 5, 3, 3, 8
-    ours_cls, ref_cls, kw = {
-        "gnanpy_tensor_node": (g.TensorGNAN, gnan_py.TensorGNAN, dict(in_channels=K, out_channels=C, n_layers=L, hidden_channels=H, is_graph_task=False)),
-        "gnanpy_tensor_graph": (g.TensorGNAN, gnan_py.TensorGNAN, dict(in_channels=K, out_channels=1, n_layers=L, hidden_channels=H, is_graph_task=True, bias=False)),
-        "gnanpy_gnan": (g.GNAN, gnan_py.GNAN, dict(in_channels=K, out_channels=C, n_layers=4, hidden_channels=H)),
-        "gnanpy_gnan_rho_per_feature": (g.GNAN, gnan_py.GNAN, dict(in_channels=K, out_channels=C, n_layers=L, hidden_channels=H, rho_per_feature=True)),
-        "models_tensor_readout": (mo.TensorGNAN, models_py.TensorGNAN, dict(in_channels=K, out_channels=2, n_layers=L, hidden_channels=H, is_graph_task=True, readout_n_layers=2)),
-        "models_tensor_node": (mo.TensorGNAN, models_py.TensorGNAN, dict(in_channels=K, out_channels=C, n_layers=1, hidden_channels=H, rho_per_feature=True)),
-        "models_gnan": (mo.GNAN, models_py.GNAN, dict(in_channels=K, out_channels=C, num_layers=L, hidden_channels=H)),
-        "batched": (b.TensorGNAN, batched_cls, dict(in_channels=K, out_channels=C, n_layers=L, hidden_channels=H, dropout=0.0)),
-    }[variant]
-    torch.manual_seed(0)
-    ours, ref = ours_cls(**kw), ref_cls(**kw)
-    with torch.no_grad():
-        for p in ours.parameters():
-            p.normal_()
-    sd = ours.state_dict()
-    assert sorted(sd) == sorted(ref.state_dict())
-    ref.load_state_dict(sd, strict=True)                                     # gnan_b200 checkpoint -> unmodified reference
-    ours.eval(); ref.eval()
+@pytest.mark.parametrize("name", G.MODEL_CASES + G.BATCHED_CASES)
+def test_checkpoints_keep_the_reference_layout_in_both_directions(name):
+    """The gnan_b200 -> reference direction of test_loads_reference_state_dict: a FRESH module of a golden case's configuration (no
+    reference weights loaded) writes exactly the keys, shapes and dtypes the reference module wrote for that case (the sd.* arrays), so
+    its checkpoint loads strictly into the reference class. After the strict load of the reference's checkpoint, the per-feature
+    accessors `fs[k]` / `rho` evaluate the reference's Sequential (oracle/gnan_port.scalar_mlp, float64) on the stored weights."""
+    from gnan_b200 import GNAN as g
+    z = G.load(name)
+    ref = {k: torch.from_numpy(v) for k, v in z["sd"].items()}
+    fresh = [build_module(z, load=False)]
+    if z["variant"] == "gnan_loop":                      # both copies of the reference's GNAN class write the same layout
+        fresh.append(g.GNAN(z["K"], z["C"], n_layers=z["L"], hidden_channels=z["H"], bias=z["bias"], normalize_rho=z["normalize_rho"],
+                            rho_per_feature=z["rho_per_feature"]))
+    for m in fresh:
+        sd = m.state_dict()
+        assert sorted(sd) == sorted(ref), (type(m).__module__, sorted(set(sd) ^ set(ref)))
+        for k, v in sd.items():
+            assert v.shape == ref[k].shape and v.dtype == ref[k].dtype, k
+    m = build_module(z).eval()
     t = torch.linspace(-1.5, 1.5, 7).view(-1, 1)
-    for k in range(K):
-        assert torch.allclose(ref.fs[k](t), ours.fs[k](t), atol=1e-6), k
-    ref_rho = ref.rho if not isinstance(ref.rho, torch.nn.ModuleList) else ref.rho[0]
-    assert torch.allclose(ref_rho(t), ours.rho(t), atol=1e-6)
-    with torch.no_grad():
-        for p in ref.parameters():
-            p.add_(1.0)
-    ours.load_state_dict(ref.state_dict(), strict=True)                      # and back
-    back = ours.state_dict()
-    for k_, v in ref.state_dict().items():
-        assert torch.equal(back[k_], v), k_
+    fs, rho = gnan_port.to_torch(z["fs"], torch.float64), gnan_port.to_torch(z["rho"], torch.float64)
+    for k in range(z["K"]):
+        assert torch.allclose(m.fs[k](t).double(), gnan_port.scalar_mlp(fs, k, t.double()), rtol=1e-5, atol=1e-5), k
+    assert torch.allclose(m.rho(t).double(), gnan_port.scalar_mlp(rho, 0, t.double()), rtol=1e-5, atol=1e-5)
 
 
 def test_product_package_never_imports_the_oracle_or_the_tests():

@@ -129,37 +129,6 @@ def test_apsp_oracle_bit_exact(name):
     del node_task
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/GNAN.py"), reason="the unmodified reference is only present in the build container")
-def test_golden_files_regenerate_bit_exactly_from_the_reference(tmp_path):
-    """The committed fixtures ARE the reference's outputs: oracle/make_golden.py (unmodified GNAN.py / models.py / pre_process_datasets.py /
-    trainer.py through the torch_geometric stub) rewrites every file of tests/golden/ bit for bit."""
-    import contextlib
-    import glob
-    import io
-
-    import oracle.make_golden as mg
-    old = mg.OUT
-    mg.OUT = str(tmp_path)
-    try:
-        with contextlib.redirect_stdout(io.StringIO()):
-            mg.main()
-            mg.trainer_cases()
-    finally:
-        mg.OUT = old
-    files = sorted(glob.glob(os.path.join(old, "*.npz")))
-    assert len(files) >= 23
-    for f in files:
-        g = os.path.join(str(tmp_path), os.path.basename(f))
-        assert os.path.exists(g), f"{os.path.basename(f)} is not produced by make_golden.py"
-        a, b = np.load(f, allow_pickle=True), np.load(g, allow_pickle=True)
-        assert set(a.files) == set(b.files), os.path.basename(f)
-        for k in a.files:
-            if a[k].dtype == object:
-                assert str(a[k]) == str(b[k]), (os.path.basename(f), k)
-            else:
-                assert a[k].dtype == b[k].dtype and np.array_equal(a[k], b[k]), (os.path.basename(f), k)
-
-
 @pytest.mark.parametrize("seed", range(12))
 def test_apsp_oracle_matches_scipy_dijkstra_on_random_graphs(seed):
     """The C oracle against the library call the reference makes (scipy.sparse.csgraph.dijkstra on the unit-weight directed adjacency,
@@ -194,50 +163,101 @@ def test_apsp_oracle_matches_scipy_dijkstra_on_random_graphs(seed):
     assert np.array_equal(oapsp.apsp_rows(ei, n, rows), np.asarray(hop)[:rows])
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/GNAN.py"), reason="the unmodified reference is only present in the build container")
-@pytest.mark.parametrize("seed", [1, 2, 3, 4, 5, 6, 7, 8, 14, 33])     # 14 and 33: ill-conditioned draws (see below)
-def test_oracle_matches_the_live_reference_on_fresh_random_cases(tmp_path, monkeypatch, seed):
-    """Beyond the committed fixtures: NEW random configurations (sizes, widths, depths, switches drawn from the seed) are run through the
-    unmodified reference classes here, and both restatements (fp32 port in the reference's op order, float64 table form) must reproduce
-    outputs and all parameter gradients — the oracle is pinned to the reference itself, not only to 23 files."""
-    import contextlib
-    import io
+def _random_weights(model, seed):
+    """The golden generator's re-draw (oracle/make_golden.reinit), applied through the module's reference-format state_dict."""
+    g = torch.Generator().manual_seed(seed)
+    sd = {k: torch.randn(v.shape, generator=g) * ((1.2 / max(v.shape[1], 1) ** 0.5) if k.endswith("weight") else 0.3)
+          for k, v in model.state_dict().items()}
+    model.load_state_dict(sd, strict=True)
+    return {f"sd.{k}": v.numpy() for k, v in model.state_dict().items()}
 
+
+def _random_model_case(out_dir, name, cls, variant, rng, *, N, K_raw, C, H, L, is_graph_task, normalize_rho, rho_per_feature=False,
+                       n_isolated=0, node_ids=None, directed=False, layers_kw="n_layers", bias=True):
+    """oracle/make_golden.model_case with the same random draws, minus the reference: the weights are written by the gnan_b200 module
+    of that configuration (the reference's state_dict layout) and the inputs by the C BFS in the reference's fp32 format (bit-exact
+    to its pre_process: test_apsp_oracle_bit_exact, test_apsp_oracle_matches_scipy_dijkstra_on_random_graphs)."""
     import oracle.make_golden as mg
-    gnan_py, models_py, pre_py, batched_cls = mg.import_reference()
+    ei = mg.random_graph(rng, N, n_isolated=n_isolated, directed=directed)
+    x = ((rng.random((N, K_raw)) < 0.5) * rng.normal(size=(N, K_raw))).astype(np.float32)
+    hop = oapsp.apsp(ei, N)
+    nd, nm = oapsp.reference_format(hop, oapsp.level_counts(hop))
+    x = np.concatenate([x, np.ones((N, 1), np.float32)], 1)                 # pre_process_datasets.py:108
+    K = K_raw + 1
+    kw = dict(in_channels=K, out_channels=C, hidden_channels=H, bias=bias, dropout=0.0, normalize_rho=normalize_rho,
+              rho_per_feature=rho_per_feature, **{layers_kw: L})
+    if variant != "gnan_loop":
+        kw["is_graph_task"] = is_graph_task
+    if variant == "models_tensor":
+        kw["readout_n_layers"] = 0
+    sd = _random_weights(cls(**kw), int(rng.integers(0, 2 ** 31)))
+    rho_has_bias = bias if variant == "gnan_loop" else (not is_graph_task)
+    meta = np.array([N, K, C, H, L, int(is_graph_task), int(normalize_rho), int(rho_per_feature), 0, int(rho_has_bias), int(bias)])
+    extra = {} if node_ids is None else {"node_ids": np.array(node_ids, dtype=np.int64)}
+    np.savez(os.path.join(out_dir, name + ".npz"), x=x, edge_index=ei, node_distances=nd, normalization_matrix=nm, meta=meta, **extra, **sd)
+
+
+def _random_batched_case(out_dir, name, rng, *, B, K, C, H, is_graph_task):
+    """oracle/make_golden.batched_case with the same random draws: per-graph hop matrices from the C BFS (-1 unreachable, as the
+    networkx BFS of batched_pyg_main.py:39-44), weights written by gnan_b200's batched module."""
+    import oracle.make_golden as mg
+    from gnan_b200 import batched
+    xs, dists, bv = [], [], []
+    for g_ in range(B):
+        n = int(rng.integers(3, 12))
+        ei = mg.random_graph(rng, n, n_isolated=1 if g_ % 3 == 0 and n > 4 else 0)
+        dists.append(np.asarray(oapsp.apsp(ei, n), dtype=np.float32))
+        xs.append(rng.normal(size=(n, K)).astype(np.float32)); bv += [g_] * n
+    tot = len(bv)
+    dist_batch = np.full((tot, tot), -1, dtype=np.float32)
+    o = 0
+    for dm in dists:
+        dist_batch[o:o + dm.shape[0], o:o + dm.shape[0]] = dm; o += dm.shape[0]
+    model = batched.TensorGNAN(in_channels=K, out_channels=C, n_layers=2, hidden_channels=H, is_graph_task=is_graph_task)
+    sd = _random_weights(model, int(rng.integers(0, 2 ** 31)))
+    np.savez(os.path.join(out_dir, name + ".npz"), x=np.concatenate(xs), dist_batch=dist_batch, batch_vector=np.array(bv, dtype=np.int64),
+             meta=np.array([tot, K, C, H, 2, int(is_graph_task)]), **sd)
+
+
+@pytest.mark.parametrize("seed", [1, 2, 3, 4, 5, 6, 7, 8, 14, 33])     # 14 and 33: ill-conditioned draws (see below)
+def test_table_restatement_matches_the_port_on_fresh_random_cases(tmp_path, monkeypatch, seed):
+    """Beyond the committed fixtures: NEW random configurations (sizes, widths, depths 1-4, directed graphs, isolated nodes, bias and
+    normalisation switches, row subsets, all four variants), drawn from the seed as oracle/make_golden.py draws them. Both restatements
+    must agree on outputs and all parameter gradients: the float64 table form (gnan_lut) and the fp32 port's op order carried in float64
+    (gnan_port). The port itself is pinned to the reference's outputs by test_port_matches_reference."""
+    from gnan_b200 import GNAN as gnan_py, models as models_py
     rng = np.random.default_rng(9000 + seed)
-    monkeypatch.setattr(mg, "OUT", str(tmp_path))
     monkeypatch.setattr(G, "GOLDEN_DIR", str(tmp_path))
     pick = lambda *v: v[int(rng.integers(0, len(v)))]
     names = []
-    with contextlib.redirect_stdout(io.StringIO()):
-        for variant, cls, kw in (("gnanpy_tensor", gnan_py.TensorGNAN, {}), ("models_tensor", models_py.TensorGNAN, {}),
-                                 ("gnan_loop", pick(gnan_py.GNAN, models_py.GNAN), {})):
-            graph = bool(rng.integers(0, 2)) and variant != "gnan_loop"
-            name = f"{variant if variant != 'gnan_loop' else 'gnan_loop'}_live{seed}"
-            if variant == "gnan_loop":
-                kw = dict(layers_kw="n_layers" if cls is gnan_py.GNAN else "num_layers", rho_per_feature=bool(rng.integers(0, 2)),
-                          node_ids=pick(None, [2, 0, 5]))
-            elif variant == "models_tensor":
-                kw = dict(rho_per_feature=bool(rng.integers(0, 2)) and not graph)
-            mg.model_case(name, cls, variant, rng, pre_py, N=int(rng.integers(8, 30)), K_raw=int(rng.integers(2, 7)),
-                          C=1 if graph else int(rng.integers(1, 6)), H=pick(8, 16, 32, 64), L=pick(1, 2, 3, 4) if variant == "gnanpy_tensor" else pick(2, 3),
-                          is_graph_task=graph, normalize_rho=bool(rng.integers(0, 2)), n_isolated=int(rng.integers(0, 3)),
-                          directed=bool(rng.integers(0, 2)), bias=bool(rng.integers(0, 4)), **kw)
-            names.append(name)
-        mg.batched_case(f"batched_live{seed}", batched_cls, rng, B=int(rng.integers(2, 6)), K=int(rng.integers(2, 6)), C=int(rng.integers(1, 5)),
-                        H=pick(8, 16), is_graph_task=bool(rng.integers(0, 2)))
-        names.append(f"batched_live{seed}")
-    for name in names:
-        test_port_matches_reference(name)                    # fp32 port in the reference's op order == the fp32 reference
-        # the table form against the SAME op order carried in float64: a random case may be ill-conditioned (outputs that are small
-        # differences of O(1) terms), where the reference's own fp32 rounding exceeds any fixed bound against float64; the algebra
-        # is checked where rounding does not enter (left: the fp32 rounding of the 1/(1+d) inputs the port is fed, 6e-8, which such a
-        # case amplifies: hence 1e-6 on outputs and 2e-5 on gradients; 40 seeds were tried when the test was written)
+    for variant, cls, kw in (("gnanpy_tensor", gnan_py.TensorGNAN, {}), ("models_tensor", models_py.TensorGNAN, {}),
+                             ("gnan_loop", pick(gnan_py.GNAN, models_py.GNAN), {})):
+        graph = bool(rng.integers(0, 2)) and variant != "gnan_loop"
+        name = f"{variant}_live{seed}"
+        if variant == "gnan_loop":
+            kw = dict(layers_kw="n_layers" if cls is gnan_py.GNAN else "num_layers", rho_per_feature=bool(rng.integers(0, 2)),
+                      node_ids=pick(None, [2, 0, 5]))
+        elif variant == "models_tensor":
+            kw = dict(rho_per_feature=bool(rng.integers(0, 2)) and not graph)
+        _random_model_case(str(tmp_path), name, cls, variant, rng, N=int(rng.integers(8, 30)), K_raw=int(rng.integers(2, 7)),
+                           C=1 if graph else int(rng.integers(1, 6)), H=pick(8, 16, 32, 64), L=pick(1, 2, 3, 4) if variant == "gnanpy_tensor" else pick(2, 3),
+                           is_graph_task=graph, normalize_rho=bool(rng.integers(0, 2)), n_isolated=int(rng.integers(0, 3)),
+                           directed=bool(rng.integers(0, 2)), bias=bool(rng.integers(0, 4)), **kw)
+        names.append(name)
+    _random_batched_case(str(tmp_path), f"batched_live{seed}", rng, B=int(rng.integers(2, 6)), K=int(rng.integers(2, 6)), C=int(rng.integers(1, 5)),
+                         H=pick(8, 16), is_graph_task=bool(rng.integers(0, 2)))
+    names.append(f"batched_live{seed}")
+    for i, name in enumerate(names):
         z = G.load(name)
+        z["out_weight"] = np.float64(1.0)
+        shape = run_port(z, torch.float64)[0].shape
+        z["out_weight"] = torch.randn(shape, generator=torch.Generator().manual_seed(seed * 10 + i), dtype=torch.float64).numpy()
+        # a random case may be ill-conditioned (outputs that are small differences of O(1) terms), where fp32 rounding exceeds any fixed
+        # bound against float64; the algebra is checked where rounding does not enter (left: the fp32 rounding of the 1/(1+d) inputs
+        # the port is fed, 6e-8, which such a case amplifies: hence 1e-6 on outputs and 2e-5 on gradients)
         out_l, fs_l, rho_l = run_lut(z)
         out_p, fs_p, rho_p, _ = run_port(z, torch.float64)
-        assert G.rel_err(out_l.detach().numpy(), out_p.detach().numpy()) < 1e-6, name
+        assert out_l.shape == out_p.shape and G.rel_err(out_l.detach().numpy(), out_p.detach().numpy()) < 1e-6, name
         for got, want in ((fs_l, fs_p), (rho_l, rho_p)):
             for k in ("w1", "b1", "wh", "bh", "wo", "bo"):
                 if want[k] is None or want[k].grad is None or got[k].grad is None or float(want[k].grad.norm()) == 0:
