@@ -84,6 +84,8 @@ SIGNATURES = {
                                              c_void_p, c_void_p, c_int32, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "gnan_apsp_bfs_batched_local": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_void_p, c_void_p,
                                             c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "gnan_bfs_graph_readout_fwd": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p, c_int32, c_void_p,
+                                           c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "gnan_edges_from_local": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int64, c_void_p, c_void_p]),
     "gnan_build_csr_workspace_bytes": (c_size_t, [c_int32, c_int64]),
     "gnan_build_csr": (c_int, [c_void_p, c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),

@@ -5,6 +5,7 @@
 // Output: uint8 hop matrix (level, 255 = unreachable) and int32 level sizes cnt[i,d]; the reference's two fp32 [N,N]
 // matrices are node_distances = 1/(1+hop) and normalization_matrix = cnt[i, hop[i,j]] (gnan_hops_to_reference).
 #include <algorithm>
+#include <type_traits>
 #include <cub/block/block_scan.cuh>
 
 #include <cstdlib>
@@ -402,6 +403,60 @@ __host__ __device__ inline size_t bv3_need(int cap, int W, int nbins, bool level
     return bv3_hop_bytes(cap) + bv3_fr_bytes(cap, W, local, pst) + (levels ? bv2_round16((size_t)cap * nbins) : 0);
 }
 
+// up to 8 out-neighbours of a vertex travel with it as bytes of two registers (lo, hi), dg of them
+__device__ __forceinline__ void bv3_keep(uint32_t &lo, uint32_t &hi, int &dg, uint32_t u)
+{
+    const int sh = 8 * (dg & 3);
+    if (dg < 4) lo = (lo & ~(0xffu << sh)) | (u << sh);
+    else hi = (hi & ~(0xffu << sh)) | (u << sh);
+    ++dg;
+}
+// LOCAL: the out-neighbours of a vertex from its adjacency row; more than 8: many = 1 and the level loop walks the row instead
+template <int W>
+__device__ __forceinline__ void bv3_local_nbrs(const uint32_t *arow, uint32_t &lo, uint32_t &hi, int &dg, int &many)
+{
+    int deg = 0;
+#pragma unroll
+    for (int ww = 0; ww < W; ++ww) deg += __popc(arow[ww]);
+    if (deg <= 8) {
+#pragma unroll
+        for (int ww = 0; ww < W; ++ww) {
+            uint32_t m = arow[ww];
+            while (m) {
+                bv3_keep(lo, hi, dg, (uint32_t)(ww * 32 + __ffs(m) - 1));
+                m &= m - 1;
+            }
+        }
+    } else {
+        many = 1;
+    }
+}
+// acc |= the frontier rows fc [n][WS] of the dg kept neighbours
+template <int W>
+__device__ __forceinline__ void bv3_pull_kept(const uint32_t *fc, uint32_t lo, uint32_t hi, int dg, uint32_t (&acc)[W])
+{
+#pragma unroll
+    for (int t = 0; t < 8; ++t) {
+        if (t < dg) {
+            const uint32_t u = ((t < 4 ? lo : hi) >> (8 * (t & 3))) & 0xffu;
+            bv3_or_row<W>(fc + u * bv3_ws(W), acc);
+        }
+    }
+}
+// acc |= the frontier rows of every neighbour in the adjacency row arow (rows with more than 8 neighbours)
+template <int W>
+__device__ __forceinline__ void bv3_pull_row(const uint32_t *fc, const uint32_t *arow, uint32_t (&acc)[W])
+{
+#pragma unroll
+    for (int ww = 0; ww < W; ++ww) {
+        uint32_t m = arow[ww];
+        while (m) {
+            bv3_or_row<W>(fc + (ww * 32 + __ffs(m) - 1) * bv3_ws(W), acc);
+            m &= m - 1;
+        }
+    }
+}
+
 template <int G>
 __device__ __forceinline__ void bv3_sync(int bar)
 {
@@ -444,34 +499,14 @@ __device__ __forceinline__ int bv3_graph(const int32_t *__restrict__ rowptr, con
 #pragma unroll
     for (int ww = 0; ww < W; ++ww) vis[ww] = 0u;
     if (mine) {
-        auto keep = [&](uint32_t u) {
-            const int sh = 8 * (dg & 3);
-            if (dg < 4) nb_lo = (nb_lo & ~(0xffu << sh)) | (u << sh);
-            else nb_hi = (nb_hi & ~(0xffu << sh)) | (u << sh);
-            ++dg;
-        };
         if (LOCAL) {
-            int deg = 0;
-#pragma unroll
-            for (int ww = 0; ww < W; ++ww) deg += __popc(adj[v * WS + ww]);
-            if (deg <= 8) {
-#pragma unroll
-                for (int ww = 0; ww < W; ++ww) {
-                    uint32_t m = adj[v * WS + ww];
-                    while (m) {
-                        keep((uint32_t)(ww * 32 + __ffs(m) - 1));
-                        m &= m - 1;
-                    }
-                }
-            } else {
-                e1 = 1;                                              // more than 8 neighbours: the level loop walks the adjacency row
-            }
+            bv3_local_nbrs<W>(adj + v * WS, nb_lo, nb_hi, dg, e1);  // e1 = 1: more than 8 neighbours
         } else {
             const int eb = rowptr[n0 + v], ee = rowptr[n0 + v + 1];
             int e = eb;
             for (; e < ee && dg < 8; ++e) {                          // neighbours outside the graph are ignored
                 const int u = __ldg(col + e) - n0;
-                if (u >= 0 && u < n) keep((uint32_t)u);
+                if (u >= 0 && u < n) bv3_keep(nb_lo, nb_hi, dg, (uint32_t)u);
             }
             e8 = e; e1 = ee;
         }
@@ -494,24 +529,9 @@ __device__ __forceinline__ int bv3_graph(const int32_t *__restrict__ rowptr, con
             uint32_t acc[W];
 #pragma unroll
             for (int ww = 0; ww < W; ++ww) acc[ww] = 0u;
-#pragma unroll
-            for (int t = 0; t < 8; ++t) {
-                if (t < dg) {
-                    const uint32_t u = ((t < 4 ? nb_lo : nb_hi) >> (8 * (t & 3))) & 0xffu;
-                    bv3_or_row<W>(fc + u * WS, acc);
-                }
-            }
+            bv3_pull_kept<W>(fc, nb_lo, nb_hi, dg, acc);
             if (LOCAL) {
-                if (e1) {                                            // rows with more than 8 neighbours
-#pragma unroll
-                    for (int ww = 0; ww < W; ++ww) {
-                        uint32_t m = adj[v * WS + ww];
-                        while (m) {
-                            bv3_or_row<W>(fc + (ww * 32 + __ffs(m) - 1) * WS, acc);
-                            m &= m - 1;
-                        }
-                    }
-                }
+                if (e1) bv3_pull_row<W>(fc, adj + v * WS, acc);      // rows with more than 8 neighbours
             } else {
                 for (int e = e8; e < e1; ++e) {                      // rows with more than 8 neighbours
                     const int u = __ldg(col + e) - n0;
@@ -718,6 +738,216 @@ __device__ __forceinline__ int bv3_run(const int32_t *__restrict__ rowptr, const
     return lm;
 }
 
+// ---- the batched BFS fused with the output-normalised graph readout (LOCAL edges; models.py:366-384) -------------------------
+// agg_bd_graph_fwd_kernel (csrc/agg_bd.cu) computes out / colw / Q from the hop bytes and the normaliser table that the BFS wrote.
+// Here the BFS folds the pair statistics P[j,d] = sum_{i: hop(i,j) = d} 1/count(i,d) straight into them, level by level:
+// colw[j,c'] += T[d,c'] P[j,d] in lane j's registers, Q[b,d,c] += S[j,c] P[j,d] as one warp sum per level into the warp's own
+// [nbins][C] slot of shared memory (the slots are added in warp order at the end: no float atomics, fixed order). Neither hop
+// bytes, nor a level table, nor P reach global memory. P[.,d] after the barrier of level d, summed over i in ascending order:
+// on a symmetric graph the i at distance d from j are j's own new sources of the level, and count(i,d) is i's popcount (rcl,
+// published by every lane before the barrier); on a directed graph lane j walks the new-frontier rows of all n vertices for
+// bit j instead (slower, same result). Levels >= nbins-1 only set the overflow flag (the level table's contract).
+struct Bv3Readout {
+    const float *T;      // [nbins][Cr]
+    const float *S;      // [sumN][C]
+    int Cr, C;
+    float *out, *colw, *Q;   // [B][C], [sumN][Cr], [B][nbins][C]
+};
+
+// frontier rows [2][cap][WS], adjacency [cap][WS], 1/count [2][cap], per-warp Q [G][nbins][CC] + per-warp out [G][CC]
+__host__ __device__ inline size_t bv3_ro_need(int cap, int W, int G, int nbins, int CC)
+{
+    return bv2_round16((size_t)3 * cap * bv3_ws(W) * 4 + (size_t)2 * cap * 4 + (size_t)G * (nbins + 1) * CC * 4);
+}
+
+// lane's share of bin d: colw += T[d,:] p, the warp's Q slot [d,:] = sum over the warp's lanes of S[v,:] p (all 32 lanes call it)
+template <int CC>
+__device__ __forceinline__ void bv3_ro_fold(int d, float p, const float (&s)[CC], float (&cw)[CC], float *sqw, const Bv3Readout &r,
+                                            int lane)
+{
+#pragma unroll
+    for (int c = 0; c < CC; ++c) {
+        if (c < r.Cr) cw[c] = fmaf(__ldg(r.T + d * r.Cr + c), p, cw[c]);
+        if (c < r.C) {
+            float q = s[c] * p;
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) q += __shfl_xor_sync(0xffffffffu, q, o);
+            if (lane == 0) sqw[d * CC + c] = q;
+        }
+    }
+}
+
+template <int W, int G, int CC>
+__device__ __forceinline__ int bv3_readout_run(const int32_t *__restrict__ node_off, int64_t b, int ts, int bar, uint8_t *slice,
+                                               const Bv3Out &o, const Bv3Readout &r, int32_t *overflow)
+{
+    constexpr int T = 32 * G, WS = bv3_ws(W);
+    const int n0 = node_off[b], n = node_off[b + 1] - n0, nbins = o.nbins, nq = nbins * CC;
+    const int v = ts, lane = ts & 31, wsub = ts >> 5;
+    const bool mine = v < n;
+    uint32_t *frs = reinterpret_cast<uint32_t *>(slice);                       // [2][n][WS]
+    uint32_t *adj = frs + 2 * n * WS;                                          // [n][WS]
+    float *rcl = reinterpret_cast<float *>(adj + n * WS);                      // [2][n] 1/count of the current level (by parity)
+    float *sq = rcl + 2 * n, *so = sq + G * nq;                                // [G][nbins][CC], [G][CC]
+    float *sqw = sq + wsub * nq;
+    for (int t = ts; t < n * WS; t += T) adj[t] = 0u;
+    for (int t = ts; t < G * (nq + CC); t += T) sq[t] = 0.f;
+    bv3_sync<G>(bar);
+    const int e0 = o.edge_off[b], e1 = o.edge_off[b + 1];
+    int flags = 0;                                                             // status bits as gnan_apsp_bfs_batched_local
+    for (int e = e0 + ts; e < e1; e += T) {
+        const uint32_t s = o.lsrc[e], d = o.ldst[e];
+        if (s < (uint32_t)n && d < (uint32_t)n) {
+            const uint32_t bit = 1u << (d & 31);
+            if (atomicOr(adj + s * WS + (d >> 5), bit) & bit) flags |= 2;
+        } else {
+            flags |= 1;
+        }
+    }
+    if (flags) atomicOr(o.status, flags);
+    bv3_sync<G>(bar);
+    bool asym = false;
+    for (int e = e0 + ts; e < e1; e += T) {
+        const uint32_t s = o.lsrc[e], d = o.ldst[e];
+        if (s < (uint32_t)n && d < (uint32_t)n && !((adj[d * WS + (s >> 5)] >> (s & 31)) & 1u)) asym = true;
+    }
+    const bool sym = !bv3_any<G>(bar, asym);
+
+    float s[CC], cw[CC];
+#pragma unroll
+    for (int c = 0; c < CC; ++c) {
+        s[c] = (mine && c < r.C) ? r.S[(int64_t)(n0 + v) * r.C + c] : 0.f;
+        cw[c] = 0.f;
+    }
+    uint32_t vis[W], nb_lo = 0xffffffffu, nb_hi = 0xffffffffu;
+    int dg = 0, many = 0;
+#pragma unroll
+    for (int ww = 0; ww < W; ++ww) vis[ww] = 0u;
+    if (mine) {
+        bv3_local_nbrs<W>(adj + v * WS, nb_lo, nb_hi, dg, many);
+#pragma unroll
+        for (int ww = 0; ww < W; ++ww) vis[ww] = ww == wsub ? 1u << lane : 0u;
+        bv3_store_row<W>(frs + v * WS, vis);
+    }
+    bv3_ro_fold<CC>(0, mine ? 1.f : 0.f, s, cw, sqw, r, lane);                 // level 0: v itself, count 1
+    bv3_sync<G>(bar);
+    int lvl_max = 0;
+    for (int level = 1; level <= n; ++level) {
+        const uint32_t *fc = frs + ((level - 1) & 1) * n * WS;
+        uint32_t *fn = frs + (level & 1) * n * WS;
+        float *rc = rcl + (level & 1) * n;
+        bool any = false;
+        uint32_t nw[W];
+        if (mine) {
+#pragma unroll
+            for (int ww = 0; ww < W; ++ww) nw[ww] = 0u;
+            bv3_pull_kept<W>(fc, nb_lo, nb_hi, dg, nw);
+            if (many) bv3_pull_row<W>(fc, adj + v * WS, nw);
+            int newc = 0;
+#pragma unroll
+            for (int ww = 0; ww < W; ++ww) {
+                nw[ww] &= ~vis[ww];
+                vis[ww] |= nw[ww];
+                newc += __popc(nw[ww]);
+            }
+            bv3_store_row<W>(fn + v * WS, nw);
+            rc[v] = newc ? __frcp_rn((float)newc) : 0.f;
+            if (newc) {
+                any = true;
+                if (level >= nbins - 1) atomicExch(overflow, 1);
+            }
+        }
+        if (!bv3_any<G>(bar, any)) break;
+        lvl_max = level;
+        float p = 0.f;                                                         // P[v, level]
+        if (mine) {
+            if (sym) {                      // v's new sources (one channel: reloaded from fn, 5 groups per CTA fit 48 registers)
+#pragma unroll
+                for (int ww = 0; ww < W; ++ww) {
+                    uint32_t m = CC == 1 ? fn[v * WS + ww] : nw[ww];
+                    while (m) {
+                        p += rc[ww * 32 + __ffs(m) - 1];
+                        m &= m - 1;
+                    }
+                }
+            } else {
+                for (int i = 0; i < n; ++i)
+                    if ((fn[i * WS + wsub] >> lane) & 1u) p += rc[i];
+            }
+        }
+        if (level < nbins - 1) bv3_ro_fold<CC>(level, p, s, cw, sqw, r, lane);
+    }
+    // unreachable bin: sum over the i that do not reach v of 1/(i's unreachable count); skipped for connected graphs
+    int reached = 0;
+#pragma unroll
+    for (int ww = 0; ww < W; ++ww) reached += __popc(vis[ww]);
+    if (bv3_any<G>(bar, mine && reached < n)) {                                // (both frontier / 1/count buffers are free now)
+        if (mine) {
+            rcl[v] = reached < n ? __frcp_rn((float)(n - reached)) : 0.f;
+            if (!sym) bv3_store_row<W>(frs + v * WS, vis);
+        }
+        bv3_sync<G>(bar);
+        float U = 0.f;
+        if (mine) {
+            if (sym) {
+#pragma unroll
+                for (int ww = 0; ww < W; ++ww) {
+                    const int left = n - ww * 32;
+                    uint32_t m = ~vis[ww] & (left >= 32 ? 0xffffffffu : (left > 0 ? (1u << left) - 1u : 0u));
+                    while (m) {
+                        U += rcl[ww * 32 + __ffs(m) - 1];
+                        m &= m - 1;
+                    }
+                }
+            } else {
+                for (int i = 0; i < n; ++i)
+                    if (!((frs[i * WS + wsub] >> lane) & 1u)) U += rcl[i];
+            }
+        }
+        bv3_ro_fold<CC>(nbins - 1, U, s, cw, sqw, r, lane);
+    }
+    if (mine) {
+#pragma unroll
+        for (int c = 0; c < CC; ++c)
+            if (c < r.Cr) r.colw[(int64_t)(n0 + v) * r.Cr + c] = cw[c];
+    }
+    // out[b,c] = sum_v S[v,c] colw[v,c']: a warp sum each, then the warps in order
+#pragma unroll
+    for (int c = 0; c < CC; ++c) {
+        if (c < r.C) {
+            float q = s[c] * cw[r.Cr == 1 ? 0 : c];
+#pragma unroll
+            for (int off = 16; off > 0; off >>= 1) q += __shfl_xor_sync(0xffffffffu, q, off);
+            if (lane == 0) so[wsub * CC + c] = q;
+        }
+    }
+    bv3_sync<G>(bar);
+    for (int t = ts; t < nbins * r.C; t += T) {                                // Q[b] in full (empty bins: 0), coalesced
+        const int d = t / r.C, c = t - d * r.C;
+        float q = 0.f;
+#pragma unroll
+        for (int w = 0; w < G; ++w) q += sq[w * nq + d * CC + c];
+        r.Q[(int64_t)b * nbins * r.C + t] = q;
+    }
+    if (ts < r.C) {
+        float q = 0.f;
+#pragma unroll
+        for (int w = 0; w < G; ++w) q += so[w * CC + ts];
+        r.out[b * r.C + ts] = q;
+    }
+    return lvl_max;
+}
+
+// one work item of the v3 kernel: the BFS of bv3_run, or (CC > 0) the BFS fused with the graph readout
+template <int W, int G, bool LOCAL, bool PST, int CC>
+__device__ __forceinline__ int bv3_item(const int32_t *__restrict__ rowptr, const int32_t *__restrict__ col,
+                                        const int32_t *__restrict__ node_off, const int64_t *__restrict__ hop_off, int64_t b, int cap,
+                                        int ts, int bar, uint8_t *slice, const Bv3Out &o, const Bv3Readout &r, bool levels, int32_t *overflow)
+{
+    if constexpr (CC > 0) return bv3_readout_run<W, G, CC>(node_off, b, ts, bar, slice, o, r, overflow);
+    else return bv3_run<W, G, LOCAL, PST>(rowptr, col, node_off, hop_off, b, cap, ts, bar, slice, o, levels, overflow);
+}
+
 // the batch's edge list in its transfer form (LOCAL instantiation: no CSR; rowptr / col are NULL)
 struct Bv3Edges {
     const uint8_t *src, *dst;
@@ -728,13 +958,15 @@ struct Bv3Edges {
 };
 
 // order = the output of bv3_classify_kernel
-// (the pair-statistics instantiation keeps the level's new bits across the barrier: 4 groups per CTA give it 64 registers)
-template <bool LOCAL, bool PST>
-__global__ void __launch_bounds__(32 * BV3_GW * (PST ? BV3_MAX_GROUPS - 1 : BV3_MAX_GROUPS), 2)
+// (the pair-statistics and the multi-channel readout instantiations keep the level's new bits across the barrier: 4 groups per
+// CTA give them 64 registers)
+constexpr int bv3_max_groups(bool pst, int cc) { return pst || cc > 1 ? BV3_MAX_GROUPS - 1 : BV3_MAX_GROUPS; }
+template <bool LOCAL, bool PST, int CC = 0>
+__global__ void __launch_bounds__(32 * BV3_GW * bv3_max_groups(PST, CC), 2)
 apsp_batched_v3_kernel(const int32_t *__restrict__ rowptr, const int32_t *__restrict__ col, const int32_t *__restrict__ node_off,
                        const int64_t *__restrict__ hop_off, int B, int max_n, int groups_per_cta, int slice_bytes, uint8_t *__restrict__ hop,
                        int32_t *__restrict__ cnt, float *__restrict__ rscale, int nbins, int32_t *__restrict__ overflow,
-                       int32_t *__restrict__ max_level, const int32_t *__restrict__ order, Bv3Edges le)
+                       int32_t *__restrict__ max_level, const int32_t *__restrict__ order, Bv3Edges le, Bv3Readout ro)
 {
     extern __shared__ __align__(16) uint8_t sm3[];
     __shared__ float rcp_tab[256];
@@ -759,20 +991,20 @@ apsp_batched_v3_kernel(const int32_t *__restrict__ rowptr, const int32_t *__rest
             const int64_t b = t < c0 ? ord0[t] : ord1[t - c0];
             const int n = node_off[b + 1] - node_off[b];
             const int ts = wq * 32 + lane;
-            const int lm = n <= 96 ? bv3_run<3, 4, LOCAL, PST>(rowptr, col, node_off, hop_off, b, max_n, ts, bar_group, gslice, out, levels, overflow)
-                                   : bv3_run<4, 4, LOCAL, PST>(rowptr, col, node_off, hop_off, b, max_n, ts, bar_group, gslice, out, levels, overflow);
+            const int lm = n <= 96 ? bv3_item<3, 4, LOCAL, PST, CC>(rowptr, col, node_off, hop_off, b, max_n, ts, bar_group, gslice, out, ro, levels, overflow)
+                                   : bv3_item<4, 4, LOCAL, PST, CC>(rowptr, col, node_off, hop_off, b, max_n, ts, bar_group, gslice, out, ro, levels, overflow);
             lvl_max = max(lvl_max, lm);
         } else if (t < c_big + items2) {                             // 33..64 nodes: two graphs on the two warp pairs
             const int pr = wq >> 1;
             const int64_t idx = 2 * (t - c_big) + pr;
             if (idx < c2)
-                lvl_max = max(lvl_max, bv3_run<2, 2, LOCAL, PST>(rowptr, col, node_off, hop_off, ord2[idx], cap2, (wq & 1) * 32 + lane,
-                                                     bar_group + 1 + pr, gslice + (size_t)pr * half, out, levels, overflow));
+                lvl_max = max(lvl_max, bv3_item<2, 2, LOCAL, PST, CC>(rowptr, col, node_off, hop_off, ord2[idx], cap2, (wq & 1) * 32 + lane,
+                                                          bar_group + 1 + pr, gslice + (size_t)pr * half, out, ro, levels, overflow));
         } else {                                                     // up to 32 nodes: four graphs, a warp each
             const int64_t idx = 4 * (t - c_big - items2) + wq;
             if (idx < c3)
-                lvl_max = max(lvl_max, bv3_run<1, 1, LOCAL, PST>(rowptr, col, node_off, hop_off, ord3[idx], cap1, lane, 0,
-                                                     gslice + (size_t)wq * quarter, out, levels, overflow));
+                lvl_max = max(lvl_max, bv3_item<1, 1, LOCAL, PST, CC>(rowptr, col, node_off, hop_off, ord3[idx], cap1, lane, 0,
+                                                          gslice + (size_t)wq * quarter, out, ro, levels, overflow));
         }
         bv3_sync<BV3_GW>(bar_group);                                 // the slice is re-partitioned / refilled by the next item
     }
@@ -1078,31 +1310,36 @@ extern "C" int gnan_apsp_msbfs(const int32_t *rowptr, const int32_t *col, int32_
 }
 
 // v3 launch: groups of 4 warps; the group's slice holds one graph of 65..128 nodes, two of 33..64 or four of up to 32
-template <bool LOCAL, bool PST>
+// CC > 0: the BFS fused with the graph readout (bv3_readout_run; ro holds its tensors, hop / cnt / rscale are NULL)
+template <bool LOCAL, bool PST, int CC = 0>
 static int launch_bv3(const int32_t *rowptr, const int32_t *col, const int32_t *node_off, const int64_t *hop_off, int32_t B, int32_t max_n,
                       uint8_t *hop, int32_t *cnt, float *rscale, int nb, bool levels, int32_t *overflow_flag, int32_t *max_level,
-                      int32_t *order_ws, Bv3Edges le, cudaStream_t st)
+                      int32_t *order_ws, Bv3Edges le, cudaStream_t st, Bv3Readout ro = Bv3Readout{})
 {
     const int Wmax = (max_n + 31) / 32;
-    size_t slice = 4 * bv3_need(std::min(max_n, 32), 1, nb, levels, LOCAL, PST);
-    if (Wmax >= 2) slice = std::max(slice, 2 * bv3_need(std::min(max_n, 64), 2, nb, levels, LOCAL, PST));
-    if (Wmax >= 3) slice = std::max(slice, bv3_need(max_n, Wmax, nb, levels, LOCAL, PST));
-    const int gpc = (int)std::min<size_t>(PST ? BV3_MAX_GROUPS - 1 : BV3_MAX_GROUPS, (112 * 1024) / slice);     // two CTAs per SM
+    auto need = [&](int cap, int W, int G) {
+        return CC > 0 ? bv3_ro_need(cap, W, G, nb, CC) : bv3_need(cap, W, nb, levels, LOCAL, PST);
+    };
+    size_t slice = 4 * need(std::min(max_n, 32), 1, 1);
+    if (Wmax >= 2) slice = std::max(slice, 2 * need(std::min(max_n, 64), 2, 2));
+    if (Wmax >= 3) slice = std::max(slice, need(max_n, Wmax, 4));
+    const int gpc = (int)std::min<size_t>(bv3_max_groups(PST, CC), (112 * 1024) / slice);     // two CTAs per SM
     if (gpc < 1) return GNAN_ERR_UNSUPPORTED;
     const size_t smem3 = slice * gpc;
+    auto kernel = apsp_batched_v3_kernel<LOCAL, PST, CC>;
     static thread_local size_t cached_smem3 = 0;
     static thread_local int cached_gpc = 0, cached_per_sm3 = 0;
     if (cached_smem3 != smem3 || cached_gpc != gpc || cached_per_sm3 == 0) {
-        GNAN_CUDA(cudaFuncSetAttribute(apsp_batched_v3_kernel<LOCAL, PST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem3));
-        GNAN_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cached_per_sm3, apsp_batched_v3_kernel<LOCAL, PST>, 32 * BV3_GW * gpc, smem3));
+        GNAN_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem3));
+        GNAN_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cached_per_sm3, kernel, 32 * BV3_GW * gpc, smem3));
         cached_smem3 = smem3; cached_gpc = gpc;
     }
     const int blocks3 = (int)std::min<int64_t>(ceil_div64(B, gpc), (int64_t)std::max(cached_per_sm3, 1) * gnan_sm_count());
     GNAN_CUDA(cudaMemsetAsync(order_ws, 0, 4 * sizeof(int32_t), st));
     bv3_classify_kernel<<<(unsigned)ceil_div64(B, 256), 256, 0, st>>>(node_off, B, order_ws);
     GNAN_LAUNCH_OK();
-    apsp_batched_v3_kernel<LOCAL, PST><<<blocks3, 32 * BV3_GW * gpc, smem3, st>>>(rowptr, col, node_off, hop_off, B, max_n, gpc, (int)slice, hop, cnt,
-                                                                            rscale, nb, overflow_flag, max_level, order_ws, le);
+    kernel<<<blocks3, 32 * BV3_GW * gpc, smem3, st>>>(rowptr, col, node_off, hop_off, B, max_n, gpc, (int)slice, hop, cnt, rscale, nb,
+                                                      overflow_flag, max_level, order_ws, le, ro);
     GNAN_LAUNCH_OK();
     return GNAN_OK;
 }
@@ -1216,6 +1453,39 @@ extern "C" int gnan_apsp_bfs_batched_local(const uint8_t *src, const uint8_t *ds
                          : launch_bv3<true, false>(nullptr, nullptr, node_off, hop_off, B, max_n, hop, cnt, rscale, nb, levels, overflow_flag,
                                                    max_level, order_ws, le, st);
     if (rc == GNAN_ERR_UNSUPPORTED) gnan_set_error("apsp_bfs_batched_local: level table too wide for the shared-memory slice");
+    return rc;
+}
+
+// The batched BFS fused with the output-normalised graph readout, straight from the batch's edge list: see include/gnan_b200.h
+extern "C" int gnan_bfs_graph_readout_fwd(const uint8_t *src, const uint8_t *dst, const int32_t *edge_off, const int32_t *node_off,
+                                          int32_t B, int32_t max_n, int32_t nbins, const float *T, int32_t Cr, const float *S, int32_t C,
+                                          float *out, float *colw, float *Q, int32_t *status, int32_t *overflow_flag, int32_t *max_level,
+                                          int32_t *order_ws, gnan_stream_t stream)
+{
+    GNAN_REQUIRE(B >= 0, "bfs_graph_readout_fwd: negative batch");
+    GNAN_REQUIRE(status != nullptr, "bfs_graph_readout_fwd: NULL status");
+    if (!gnan_aggregate_blockdiag_graph_supported(nbins, Cr, C)) {
+        gnan_set_error("bfs_graph_readout_fwd: needs 2 <= nbins <= 64, C <= 4, Cr in {1,C} (nbins=%d Cr=%d C=%d)", nbins, Cr, C);
+        return GNAN_ERR_UNSUPPORTED;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    GNAN_CUDA(cudaMemsetAsync(status, 0, sizeof(int32_t), st));
+    if (B == 0) return GNAN_OK;
+    GNAN_REQUIRE(src && dst && edge_off && node_off && T && S && out && colw && Q && overflow_flag && order_ws,
+                 "bfs_graph_readout_fwd: NULL pointer");
+    if (max_n < 1 || max_n > 32 * BV2_W) {
+        gnan_set_error("bfs_graph_readout_fwd: graphs with %d nodes unsupported (1..%d)", max_n, 32 * BV2_W);
+        return GNAN_ERR_UNSUPPORTED;
+    }
+    const Bv3Edges le{src, dst, edge_off, status, nullptr, nullptr};
+    const Bv3Readout ro{T, S, Cr, C, out, colw, Q};
+    auto launch = [&](auto cc) {
+        return launch_bv3<true, false, decltype(cc)::value>(nullptr, nullptr, node_off, nullptr, B, max_n, nullptr, nullptr, nullptr, nbins,
+                                                            false, overflow_flag, max_level, order_ws, le, st, ro);
+    };
+    const int rc = C == 1 ? launch(std::integral_constant<int, 1>{}) : C == 2 ? launch(std::integral_constant<int, 2>{})
+                                                                             : launch(std::integral_constant<int, 4>{});
+    if (rc == GNAN_ERR_UNSUPPORTED) gnan_set_error("bfs_graph_readout_fwd: per-graph state too large for the shared-memory slice");
     return rc;
 }
 

@@ -93,10 +93,16 @@ class TensorGNAN(_Base):
     def forward_packed(self, pk):
         """Many graphs in one call (extension; see gnan_b200.GNAN.TensorGNAN.forward_packed): [B,C] for graph tasks."""
         dev = self._device()
-        if pk.hop.device != dev:
+        if pk.node_off.device != dev:
             pk = pk.to(dev)
         S = self._per_feature(pk.x.float().contiguous()) if self._readout else self._feature_sums(*self._features(pk))
         T = self._table(ops.rho_table_inputs(pk.nbins, dev))
+        if (pk.deferred and self.normalize_rho and self.is_graph_task and T.dim() == 2 and ops.BLOCKDIAG_GRAPH_KERNEL
+                and ops.load().gnan_aggregate_blockdiag_graph_supported(T.shape[0], T.shape[1], S.shape[1])):
+            # distances not computed yet (preprocess.apsp_batched on a LocalEdges batch): the BFS and this readout run as one
+            # kernel, neither the hop bytes nor the normaliser table are ever written (models.py:366-384)
+            out = ops.bfs_graph_readout(pk.edges, pk.node_off, pk.max_nodes, T, S, pk.status)
+            return self.readout_nam(out) if self._readout else out
         if getattr(pk, "pair_stats", None) is not None and self.normalize_rho and self.is_graph_task and T.dim() == 2:
             # the batched BFS accumulated the pair statistics of this readout itself: no pass over the hop bytes (models.py:366-384)
             out = ops.aggregate_blockdiag_pairs(pk.pair_stats, pk.pair_depth, pk.node_off, T, S)

@@ -546,6 +546,51 @@ def aggregate_blockdiag_pairs(pstat, pdepth, node_off, T, S):
     return agg_bd_graph_pairs_fwd(pstat, pdepth, node_off, T, S)[0]
 
 
+def bfs_graph_readout_fwd(edges, node_off: Tensor, max_n: int, T: Tensor, S: Tensor, status: Tensor) -> Tuple[Tensor, Tensor, Tensor]:
+    """The batched BFS of a LocalEdges batch fused with the output-normalised graph readout (gnan_bfs_graph_readout_fwd): the
+    (out, colw, Q) of agg_bd_graph_fwd on the batch's hop bytes and normaliser table, without writing either. status: the batch's
+    device int32 [3] (edge status bits, overflow flag, largest hop), filled as apsp_batched's BFS fills it."""
+    lib = load()
+    T, S = _f32(T, "T"), _f32(S, "S")
+    if node_off.dtype != torch.int32 or status.dtype != torch.int32 or status.numel() != 3:
+        raise TypeError("node_off int32 [B+1] and status int32 [3] expected")
+    B = node_off.numel() - 1
+    N, C = S.shape
+    nbins, Cr = T.shape
+    out = torch.empty(B, C, dtype=torch.float32, device=S.device)
+    colw = torch.empty(N, Cr, dtype=torch.float32, device=S.device)
+    Q = torch.empty(B, nbins, C, dtype=torch.float32, device=S.device)
+    order_ws = torch.empty(4 * B + 4, dtype=torch.int32, device=S.device)
+    with _timed("bfs_graph_readout_fwd"):
+        check(lib.gnan_bfs_graph_readout_fwd(ptr(edges.src), ptr(edges.dst), ptr(edges.edge_off), ptr(node_off), B, int(max_n), nbins, ptr(T),
+                                             Cr, ptr(S), C, ptr(out), ptr(colw), ptr(Q), status.data_ptr(), status.data_ptr() + 4,
+                                             status.data_ptr() + 8, ptr(order_ws), stream_handle()), "gnan_bfs_graph_readout_fwd")
+    return out, colw, Q
+
+
+class _BfsGraphReadout(torch.autograd.Function):
+    """out = the graph readout of a LocalEdges batch whose distances were never materialised; backward = agg_bd_graph_bwd."""
+
+    @staticmethod
+    def forward(ctx, T, S, edges, node_off, max_n, status):
+        out, colw, Q = bfs_graph_readout_fwd(edges, node_off, max_n, T, S, status)
+        ctx.save_for_backward(node_off, colw, Q)
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        node_off, colw, Q = ctx.saved_tensors
+        dS, dT = agg_bd_graph_bwd(node_off, g.contiguous(), colw, Q)
+        return dT, dS, None, None, None, None
+
+
+def bfs_graph_readout(edges, node_off, max_n, T, S, status):
+    """[B,C] output-normalised graph readout straight from the batch's edge list (preprocess.apsp_batched's deferred batches)"""
+    if T.dim() != 2 or not load().gnan_aggregate_blockdiag_graph_supported(T.shape[0], T.shape[1], S.shape[1]):
+        raise NotImplementedError("the fused BFS readout covers a global table with nbins <= 64 and C <= 4")
+    return _BfsGraphReadout.apply(T, S, edges, node_off, max_n, status)
+
+
 BLOCKDIAG_GRAPH_KERNEL = True     # tests switch it off to compare the two kernel families
 
 

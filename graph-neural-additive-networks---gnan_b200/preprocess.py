@@ -262,6 +262,8 @@ class PackedBatch:
         # output-normalised graph readout needs nothing else.
         self.pair_stats, self.pair_depth = pair_stats, pair_depth
 
+    deferred = False    # see _DeferredBatch
+
     @property
     def num_graphs(self):
         return self.node_off.numel() - 1
@@ -287,6 +289,49 @@ class PackedBatch:
         pm = lambda t: None if t is None else t.pin_memory()
         return PackedBatch(pm(self.x), pm(self.hop), pm(self.hop_off), pm(self.node_off), pm(self.level_counts), pm(self.y),
                            self.max_nodes, pm(self.level_rscale), pm(self.pair_stats), pm(self.pair_depth))
+
+
+class _DeferredBatch(PackedBatch):
+    """What apsp_batched returns for the configuration of a training step that preprocesses its own batch (LocalEdges, nbins,
+    rscale=True, graphs of at most 128 nodes): the batched BFS has not run yet. models.TensorGNAN's output-normalised graph readout
+    consumes the edge segments `edges` directly (ops.bfs_graph_readout: the BFS and the readout in one kernel, neither hop bytes
+    nor a normaliser table in memory). The first read of `hop` or `level_rscale` runs the batched BFS once, exactly as
+    apsp_batched runs it otherwise, and keeps the result; `deferred` is False from then on."""
+
+    def __init__(self, x, hop_off, node_off, y, max_nodes, nbins, edges, materialise):
+        self._materialise, self._nbins, self.edges = materialise, nbins, edges
+        super().__init__(x, None, hop_off, node_off, None, y, max_nodes)
+
+    @property
+    def deferred(self):
+        return self._materialise is not None
+
+    def _distances(self):
+        if self._materialise is not None:
+            self._hop, self._level_rscale = self._materialise()
+            self._materialise = None
+
+    @property
+    def hop(self):
+        self._distances()
+        return self._hop
+
+    @hop.setter
+    def hop(self, v):
+        self._hop = v
+
+    @property
+    def level_rscale(self):
+        self._distances()
+        return self._level_rscale
+
+    @level_rscale.setter
+    def level_rscale(self, v):
+        self._level_rscale = v
+
+    @property
+    def nbins(self):
+        return self._nbins
 
 
 class LocalEdges:
@@ -352,7 +397,9 @@ class LocalEdges:
 
 def check_batched_status(status):
     """Raise for a status word returned by apsp_batched(..., nbins=...) (one device read; call it once per epoch or when a
-    result looks wrong, not once per step)."""
+    result looks wrong, not once per step). The status of a deferred batch (see apsp_batched) is filled by whichever kernel
+    consumes its edges first: the fused BFS + readout of the model's forward, or the BFS run by the first read of `hop` /
+    `level_rscale`; read it after that."""
     st, over, _ = (int(v) for v in status.tolist())
     _check_status(st)
     if st & 2:
@@ -379,6 +426,11 @@ def apsp_batched(edge_index, node_off, device="cuda", x=None, y=None, node_off_d
     rscale=True (fixed-width mode, graphs of at most 128 nodes): the BFS writes the output normaliser 1/level_counts
     (`PackedBatch.level_rscale`, fp32) INSTEAD of the int32 level counts, which the output-normalised models
     (models.TensorGNAN, normalize_rho=True) consume directly: one table written, none converted.
+    With a `LocalEdges` input (and pair_stats=False) the distances are DEFERRED: the call launches nothing and returns a batch
+    that holds the edge segments (`deferred` is True). models.TensorGNAN's output-normalised graph readout then runs the BFS and
+    the readout as one kernel (ops.bfs_graph_readout) and never materialises hop bytes or the normaliser table; the first read of
+    `hop` or `level_rscale` runs this BFS once and caches both. `status` is the same device word either way, filled by the
+    first kernel that consumes the edges (check it after the forward).
 
     pair_stats=True (fixed-width mode, `LocalEdges` input, UNDIRECTED graphs of at most 128 nodes): the BFS
     also accumulates the pair statistics of the output-normalised graph readout (`PackedBatch.pair_stats`; see PackedBatch), so
@@ -419,9 +471,8 @@ def apsp_batched(edge_index, node_off, device="cuda", x=None, y=None, node_off_d
             edge_index = edge_index.expand(node_off_d)
     if local is None:
         rowptr, col, _ = build_csr(edge_index, sumN, device, status=st[0:1])
-    hop = torch.empty(max(total, 1), dtype=torch.uint8, device=device)
 
-    def bfs(cnt_t, rs_t, order_ws, ps_t=None, pd_t=None):
+    def bfs(hop, cnt_t, rs_t, order_ws, ps_t=None, pd_t=None):
         if local is not None:
             check(lib.gnan_apsp_bfs_batched_local(ptr(local.src), ptr(local.dst), ptr(local.edge_off), ptr(node_off_d), ptr(hop_off), B, max_n,
                                                   ptr(hop), ptr(cnt_t), ptr(rs_t), ptr(ps_t), ptr(pd_t), nb, st.data_ptr(), st.data_ptr() + 4,
@@ -439,19 +490,32 @@ def apsp_batched(edge_index, node_off, device="cuda", x=None, y=None, node_off_d
     if rscale or pair_stats:
         if nbins is None or max_n > 128 or sumN == 0:
             raise ValueError("rscale=True needs the fixed-width mode (nbins=...) and graphs of at most 128 nodes")
+        if local is not None and not pair_stats:
+            def materialise():
+                hop = torch.empty(max(total, 1), dtype=torch.uint8, device=device)
+                rs = torch.empty(sumN, nb, dtype=torch.float32, device=device)
+                order_ws = torch.empty(4 * B + 4, dtype=torch.int32, device=device)
+                with _timed("apsp_bfs_batched"):
+                    bfs(hop, None, rs, order_ws)
+                return hop, rs
+            pk = _DeferredBatch(x, hop_off, node_off_d, y, max_n, nb, local, materialise)
+            pk.status = st
+            return pk
+        hop = torch.empty(max(total, 1), dtype=torch.uint8, device=device)
         rs = torch.empty(sumN, nb, dtype=torch.float32, device=device) if rscale else None
         ps = torch.empty(sumN, nb, dtype=torch.float32, device=device) if pair_stats else None
         pd = torch.empty(B, dtype=torch.int32, device=device) if pair_stats else None
         order_ws = torch.empty(4 * B + 4, dtype=torch.int32, device=device)
         with _timed("apsp_bfs_batched"):
-            bfs(None, rs, order_ws, ps, pd)
+            bfs(hop, None, rs, order_ws, ps, pd)
         pk = PackedBatch(x, hop, hop_off, node_off_d, None, y, max_n, level_rscale=rs, pair_stats=ps, pair_depth=pd)
         pk.status = st
         return pk
+    hop = torch.empty(max(total, 1), dtype=torch.uint8, device=device)
     cnt = torch.empty(sumN, nb, dtype=torch.int32, device=device)
     order_ws = torch.empty(4 * B + 4, dtype=torch.int32, device=device)     # graphs are processed grouped by size class
     with _timed("apsp_bfs_batched"):
-        bfs(cnt, None, order_ws)
+        bfs(hop, cnt, None, order_ws)
     if nbins is not None:
         pk = PackedBatch(x, hop, hop_off, node_off_d, cnt, y, max_n)
         pk.status = st

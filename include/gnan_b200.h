@@ -364,6 +364,17 @@ int gnan_apsp_bfs_batched_local(const uint8_t *src, const uint8_t *dst, const in
                                 float *pstat, int32_t *pdepth, int32_t nbins, int32_t *status, int32_t *overflow_flag,
                                 int32_t *max_level, int32_t *order_ws, gnan_stream_t stream);
 
+/* gnan_apsp_bfs_batched_local fused with gnan_aggregate_blockdiag_graph_fwd on the output-normaliser table (models.py:366-384 with
+ * normalize_rho, a global table T [nbins,Cr]): the same out [B,C], colw [sumN,Cr] and Q [B,nbins,C] (gnan_aggregate_blockdiag_graph_bwd
+ * is the backward), computed inside the BFS level loop. No hop bytes, level table or pair statistics are written. Directed graphs
+ * are exact too (a slower path per graph, chosen in the kernel). Same envelope as gnan_aggregate_blockdiag_graph_supported;
+ * graphs of at most 128 nodes; *status (zeroed here), *overflow_flag and *max_level (optional) as gnan_apsp_bfs_batched_local.
+ * Deterministic (fixed summation orders). */
+int gnan_bfs_graph_readout_fwd(const uint8_t *src, const uint8_t *dst, const int32_t *edge_off, const int32_t *node_off, int32_t B,
+                               int32_t max_n, int32_t nbins, const float *T, int32_t Cr, const float *S, int32_t C, float *out,
+                               float *colw, float *Q, int32_t *status, int32_t *overflow_flag, int32_t *max_level, int32_t *order_ws,
+                               gnan_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Deep graphs (csrc/wide.cu): hop distances > 254. The reference has no depth limit (pre_process_datasets.py:109-121), so the
  * same path exists with an int16 hop matrix (-1 = unreachable, levels 0..32766): warp-per-source BFS (no level table: the depth
