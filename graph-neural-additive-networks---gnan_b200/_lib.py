@@ -75,15 +75,13 @@ SIGNATURES = {
     "gnan_aggregate_blockdiag_graph_supported": (c_int, [c_int32, c_int32, c_int32]),
     "gnan_aggregate_blockdiag_graph_fwd": (c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_int32, c_int32, c_void_p, c_void_p,
                                                    c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
-    "gnan_aggregate_blockdiag_graph_fwd_pairs": (c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_int32, c_int32, c_void_p, c_int32,
-                                                         c_void_p, c_void_p, c_void_p, c_void_p]),
     "gnan_aggregate_blockdiag_graph_bwd_workspace_bytes": (c_size_t, [c_int32, c_int32]),
     "gnan_aggregate_blockdiag_graph_bwd": (c_int, [c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p,
                                                    c_void_p, c_void_p, c_size_t, c_void_p]),
     "gnan_aggregate_blockdiag_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_int, c_int32, c_int32,
                                              c_void_p, c_void_p, c_int32, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "gnan_apsp_bfs_batched_local": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_void_p, c_void_p,
-                                            c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+                                            c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "gnan_bfs_graph_readout_fwd": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p, c_int32, c_void_p,
                                            c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "gnan_edges_from_local": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int64, c_void_p, c_void_p]),
@@ -97,8 +95,6 @@ SIGNATURES = {
                                 c_void_p, c_size_t, c_void_p]),
     "gnan_apsp_bfs_batched": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_int32, c_void_p,
                                       c_void_p]),
-    "gnan_apsp_bfs_batched_n": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int64, c_int64, c_void_p, c_void_p,
-                                        c_int32, c_void_p, c_void_p, c_void_p]),
     "gnan_apsp_bfs_batched_ex": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int64, c_int64, c_void_p, c_void_p,
                                          c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_void_p]),
     "gnan_loss_workspace_bytes": (c_size_t, []),

@@ -275,98 +275,6 @@ agg_bd_graph_dt_final_kernel(int nslab, int nbins, int Cr, int C, const float *_
     if (lane == 0) dT[t] = s;
 }
 
-// Graph readout from pair statistics the batched BFS produced itself (gnan_apsp_bfs_batched_local: pstat, pdepth): no hop bytes,
-// no normaliser table. A warp per graph; the graph's level-major block P_b [nbins][n] is read once, 32 nodes at a time:
-// pass A (lane = node j): p = P_b[d][j] for the rows that exist (0..depth and nbins-1) -> colw[j,c'] = sum_d T[d,c'] p (lane-local),
-// the values parked in a padded shared-memory tile; pass B (lane = level d): Q[b,d,c] += sum_j S[j,c] tile[d][j]. Fixed order.
-constexpr int BDP_WARPS = 4;
-template <int CC>
-__global__ void __launch_bounds__(BDP_WARPS * 32)
-agg_bd_graph_pairs_fwd_kernel(const float *__restrict__ P, const int32_t *__restrict__ pdepth, const int32_t *__restrict__ node_off, int B,
-                              const float *__restrict__ T, int nbins, int Cr, const float *__restrict__ S, int C, float *__restrict__ out,
-                              float *__restrict__ colw, float *__restrict__ Q)
-{
-    __shared__ float sT[BDG_MAX_NBINS * 4];                          // [nbins][Cr]
-    __shared__ float tile[BDP_WARPS][BDG_MAX_NBINS][33];             // [level][node of the block], padded: conflict free both ways
-    __shared__ float sS[BDP_WARPS][32][CC];
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    for (int t = threadIdx.x; t < nbins * Cr; t += blockDim.x) sT[t] = T[t];
-    __syncthreads();
-    const int64_t warp = (int64_t)blockIdx.x * BDP_WARPS + w, nwarp = (int64_t)gridDim.x * BDP_WARPS;
-    const int nb1 = nbins - 1;
-    for (int64_t b = warp; b < B; b += nwarp) {
-        const int n0 = node_off[b], n = node_off[b + 1] - n0, depth = min(pdepth[b], nbins - 2);
-        const float *Pb = P + (int64_t)n0 * nbins;
-        float q0[CC], q1[CC], o[CC];
-#pragma unroll
-        for (int c = 0; c < CC; ++c) q0[c] = q1[c] = o[c] = 0.f;
-        for (int jq = 0; jq < n; jq += 32) {
-            const int j = jq + lane;
-            const bool jv = j < n;
-            float sv[CC], cw[CC];
-#pragma unroll
-            for (int c = 0; c < CC; ++c) {
-                sv[c] = (jv && c < C) ? S[(int64_t)(n0 + j) * C + c] : 0.f;
-                sS[w][lane][c] = sv[c];
-                cw[c] = 0.f;
-            }
-            // pass A: rows 0..depth, then the unreachable row; four loads in flight
-            for (int d = 0; d <= depth + 1; d += 4) {
-                int dd[4];
-                float p[4];
-#pragma unroll
-                for (int u = 0; u < 4; ++u) {
-                    dd[u] = d + u <= depth ? d + u : nb1;            // past the last row: the unreachable row again (harmless: skipped below)
-                    p[u] = (jv && d + u <= depth + 1) ? Pb[(int64_t)dd[u] * n + j] : 0.f;
-                }
-#pragma unroll
-                for (int u = 0; u < 4; ++u) {
-                    if (d + u <= depth + 1) {
-                        tile[w][dd[u]][lane] = p[u];
-#pragma unroll
-                        for (int c = 0; c < CC; ++c)
-                            if (c < Cr) cw[c] = fmaf(sT[dd[u] * Cr + c], p[u], cw[c]);
-                    }
-                }
-            }
-            if (jv) {
-#pragma unroll
-                for (int c = 0; c < CC; ++c)
-                    if (c < Cr) colw[(int64_t)(n0 + j) * Cr + c] = cw[c];
-            }
-#pragma unroll
-            for (int c = 0; c < CC; ++c) o[c] = fmaf(Cr == 1 ? cw[0] : cw[c], sv[c], o[c]);
-            __syncwarp();
-            // pass B: lane t owns levels t and t + 32
-            const bool a0 = lane <= depth || lane == nb1, a1 = lane + 32 <= depth || lane + 32 == nb1;
-            if (a0 || a1) {
-#pragma unroll 8
-                for (int jj = 0; jj < 32; ++jj) {
-                    const float p0 = a0 ? tile[w][lane][jj] : 0.f, p1 = a1 ? tile[w][lane + 32][jj] : 0.f;
-#pragma unroll
-                    for (int c = 0; c < CC; ++c) {
-                        const float s = sS[w][jj][c];
-                        q0[c] = fmaf(s, p0, q0[c]);
-                        q1[c] = fmaf(s, p1, q1[c]);
-                    }
-                }
-            }
-            __syncwarp();
-        }
-#pragma unroll
-        for (int c = 0; c < CC; ++c) {
-            float v = o[c];
-#pragma unroll
-            for (int off = 16; off > 0; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
-            if (c < C) {
-                if (lane < nbins) Q[((int64_t)b * nbins + lane) * C + c] = q0[c];
-                if (lane + 32 < nbins) Q[((int64_t)b * nbins + lane + 32) * C + c] = q1[c];
-                if (lane == 0) out[b * C + c] = v;
-            }
-        }
-    }
-}
-
 }  // namespace
 
 extern "C" int gnan_aggregate_blockdiag_graph_supported(int32_t nbins, int32_t Cr, int32_t C)
@@ -414,27 +322,6 @@ extern "C" int gnan_aggregate_blockdiag_graph_fwd(const uint8_t *hop, const int6
     if (C == 1) return vec ? launch(agg_bd_graph_fwd_kernel<1, true>) : launch(agg_bd_graph_fwd_kernel<1, false>);
     if (C == 2) return vec ? launch(agg_bd_graph_fwd_kernel<2, true>) : launch(agg_bd_graph_fwd_kernel<2, false>);
     return vec ? launch(agg_bd_graph_fwd_kernel<4, true>) : launch(agg_bd_graph_fwd_kernel<4, false>);
-}
-
-extern "C" int gnan_aggregate_blockdiag_graph_fwd_pairs(const float *pstat, const int32_t *pdepth, const int32_t *node_off, int32_t B,
-                                                        const float *T, int32_t nbins, int32_t Cr, const float *S, int32_t C, float *out,
-                                                        float *colw, float *Q, gnan_stream_t stream)
-{
-    GNAN_REQUIRE(B >= 0, "aggregate_blockdiag_graph_fwd_pairs: negative batch");
-    if (B == 0) return GNAN_OK;
-    if (!gnan_aggregate_blockdiag_graph_supported(nbins, Cr, C)) {
-        gnan_set_error("aggregate_blockdiag_graph_fwd_pairs: needs 2 <= nbins <= %d, C <= 4, Cr in {1,C} (nbins=%d Cr=%d C=%d)", BDG_MAX_NBINS,
-                       nbins, Cr, C);
-        return GNAN_ERR_UNSUPPORTED;
-    }
-    GNAN_REQUIRE(pstat && pdepth && node_off && T && S && out && colw && Q, "aggregate_blockdiag_graph_fwd_pairs: NULL pointer");
-    cudaStream_t st = (cudaStream_t)stream;
-    const int blocks = (int)std::min<int64_t>(ceil_div64(B, BDP_WARPS), 6 * (int64_t)gnan_sm_count());
-    if (C == 1) agg_bd_graph_pairs_fwd_kernel<1><<<blocks, BDP_WARPS * 32, 0, st>>>(pstat, pdepth, node_off, B, T, nbins, Cr, S, C, out, colw, Q);
-    else if (C == 2) agg_bd_graph_pairs_fwd_kernel<2><<<blocks, BDP_WARPS * 32, 0, st>>>(pstat, pdepth, node_off, B, T, nbins, Cr, S, C, out, colw, Q);
-    else agg_bd_graph_pairs_fwd_kernel<4><<<blocks, BDP_WARPS * 32, 0, st>>>(pstat, pdepth, node_off, B, T, nbins, Cr, S, C, out, colw, Q);
-    GNAN_LAUNCH_OK();
-    return GNAN_OK;
 }
 
 extern "C" size_t gnan_aggregate_blockdiag_graph_bwd_workspace_bytes(int32_t nbins, int32_t C)

@@ -6,9 +6,6 @@
 // matrices are node_distances = 1/(1+hop) and normalization_matrix = cnt[i, hop[i,j]] (gnan_hops_to_reference).
 #include <algorithm>
 #include <type_traits>
-#include <cub/block/block_scan.cuh>
-
-#include <cstdlib>
 #include "common.cuh"
 
 namespace {
@@ -108,272 +105,30 @@ apsp_batched_kernel(const int32_t *__restrict__ rowptr, const int32_t *__restric
     }
 }
 
-// ---- batched small graphs, v2: one warp per graph, bit-parallel over SOURCES, hop block assembled in shared memory -------
-// A lane owns vertices v = lane, lane+32, .. and keeps, per vertex, the bitmask of sources that reach it (W = ceil(n/32)
-// words). Level L is a pull over v's out-neighbours u: new[v] = (OR_u frontier[u]) & ~visited[v]; a new bit s means
-// dist(v -> s) = L, i.e. hop[v][s] = L, and popc(new[v]) is row v's level-L count (no atomics). The n x n hop block lives in
-// shared memory (byte stores there), padded so that it is congruent to its global address mod 16, and leaves as 16-byte
-// vector stores: the global hop bytes are written exactly once, unreachable pairs included (no memset). The level counts
-// (<= 127 per entry) are collected in a uint8 [n][nbins] shared-memory table and leave as one coalesced int32 block per
-// graph, zeros included: no memset of the level table and no scattered 4-byte global stores per (vertex, level), which
-// cost a 32-byte sector each and dominated the kernel.
-constexpr int BV2_W = 4;   // up to 128 nodes per graph
-__host__ __device__ inline size_t bv2_round16(size_t x) { return (x + 15) / 16 * 16; }
-
-// One graph on one warp, W = ceil(n/32) known at compile time (exact unrolling: a 20-node graph does 1/16 of the word work of
-// a 128-node one). Up to 8 neighbours of a vertex are cached as local-index bytes in two registers (no global load inside
-// the level loop; longer rows read the rest from the CSR), and the hop bytes of a level are scattered two bits per step
-// (lowest and highest new source).
-template <int W>
-__device__ __forceinline__ int bv2_graph(const int32_t *__restrict__ rowptr, const int32_t *__restrict__ col, int n0, int n, int lane,
-                                         uint8_t *hb, uint32_t *frs, uint8_t *cs, int nbins, bool levels, int32_t *overflow)
-{
-    uint32_t vis[W][W], nb_lo[W], nb_hi[W];
-    int dg[W], e8[W], e1[W];
-#pragma unroll
-    for (int k = 0; k < W; ++k) {
-        const int v = lane + 32 * k;
-        dg[k] = 0; e8[k] = e1[k] = 0;
-        nb_lo[k] = nb_hi[k] = 0xffffffffu;
-#pragma unroll
-        for (int ww = 0; ww < W; ++ww) vis[k][ww] = 0u;
-        if (v < n) {
-            const int eb = rowptr[n0 + v], ee = rowptr[n0 + v + 1];
-            int e = eb;
-            for (; e < ee && dg[k] < 8; ++e) {                      // neighbours outside the graph are ignored (as the CSR walk did)
-                const int u = __ldg(col + e) - n0;
-                if (u >= 0 && u < n) {
-                    const int sh = 8 * (dg[k] & 3);
-                    if (dg[k] < 4) nb_lo[k] = (nb_lo[k] & ~(0xffu << sh)) | ((uint32_t)u << sh);
-                    else nb_hi[k] = (nb_hi[k] & ~(0xffu << sh)) | ((uint32_t)u << sh);
-                    ++dg[k];
-                }
-            }
-            e8[k] = e; e1[k] = ee;
-#pragma unroll
-            for (int ww = 0; ww < W; ++ww) {
-                if (ww == k) vis[k][ww] = 1u << lane;
-                frs[v * W + ww] = ww == k ? 1u << lane : 0u;
-            }
-        }
-    }
-    __syncwarp();
-#pragma unroll
-    for (int k = 0; k < W; ++k) {
-        const int v = lane + 32 * k;
-        if (v < n) {
-            hb[v * n + v] = 0;
-            if (levels) cs[v * nbins] = 1;
-        }
-    }
-    int lvl_max = 0;
-    for (int level = 1; level <= n; ++level) {
-        const uint32_t *fc = frs + ((level - 1) & 1) * n * W;
-        uint32_t *fn = frs + (level & 1) * n * W;
-        const uint8_t lv = (uint8_t)min(level, 254);
-        bool any = false;
-#pragma unroll
-        for (int k = 0; k < W; ++k) {
-            const int v = lane + 32 * k;
-            if (v < n) {
-                uint32_t acc[W];
-#pragma unroll
-                for (int ww = 0; ww < W; ++ww) acc[ww] = 0u;
-#pragma unroll
-                for (int t = 0; t < 8; ++t) {
-                    if (t < dg[k]) {
-                        const uint32_t u = ((t < 4 ? nb_lo[k] : nb_hi[k]) >> (8 * (t & 3))) & 0xffu;
-#pragma unroll
-                        for (int ww = 0; ww < W; ++ww) acc[ww] |= fc[u * W + ww];
-                    }
-                }
-                for (int e = e8[k]; e < e1[k]; ++e) {               // rows with more than 8 neighbours
-                    const int u = __ldg(col + e) - n0;
-                    if (u >= 0 && u < n) {
-#pragma unroll
-                        for (int ww = 0; ww < W; ++ww) acc[ww] |= fc[u * W + ww];
-                    }
-                }
-                int newc = 0;
-#pragma unroll
-                for (int ww = 0; ww < W; ++ww) {
-                    const uint32_t nw = acc[ww] & ~vis[k][ww];
-                    vis[k][ww] |= nw;
-                    fn[v * W + ww] = nw;
-                    newc += __popc(nw);
-                    uint32_t m = nw;
-                    uint8_t *rowp = hb + v * n + ww * 32;
-                    while (m) {
-                        const int lo = __ffs(m) - 1, hi = 31 - __clz(m);
-                        rowp[lo] = lv;
-                        rowp[hi] = lv;
-                        m &= m - 1;
-                        m &= ~(1u << hi);
-                    }
-                }
-                if (newc) {
-                    any = true;
-                    if (level > 254 || level >= nbins - 1) atomicExch(overflow, 1);
-                    else if (levels) cs[v * nbins + level] = (uint8_t)newc;
-                }
-            }
-        }
-        __syncwarp();
-        if (!__any_sync(0xffffffffu, any)) break;
-        lvl_max = max(lvl_max, level);
-    }
-    if (levels) {
-#pragma unroll
-        for (int k = 0; k < W; ++k) {
-            const int v = lane + 32 * k;
-            if (v < n) {
-                int reached = 0;
-#pragma unroll
-                for (int ww = 0; ww < W; ++ww) reached += __popc(vis[k][ww]);
-                cs[v * nbins + nbins - 1] = (uint8_t)(n - reached);
-            }
-        }
-    }
-    return lvl_max;
-}
-
-// Graphs ordered by word count W = ceil(n/32), largest first (counting sort, one CTA): the warps of a CTA then run the
-// same instantiation of bv2_graph side by side (the four instantiations do not fit the instruction cache together: 25 % of the
-// stall samples were instruction fetches) and the expensive graphs start first.
-struct Cnt4 {
-    int c[4];
-    __host__ __device__ Cnt4 operator+(const Cnt4 &o) const { return Cnt4{{c[0] + o.c[0], c[1] + o.c[1], c[2] + o.c[2], c[3] + o.c[3]}}; }
-};
-
-__global__ void __launch_bounds__(1024)
-bv2_order_kernel(const int32_t *__restrict__ node_off, int B, int32_t *__restrict__ order)
-{
-    using Scan = cub::BlockScan<Cnt4, 1024>;
-    __shared__ typename Scan::TempStorage tmp;
-    const int t = threadIdx.x;
-    Cnt4 mine{{0, 0, 0, 0}};
-    for (int b = t; b < B; b += 1024) {                            // thread-strided: coalesced reads (the order inside a class is free)
-        const int n = node_off[b + 1] - node_off[b];
-        ++mine.c[3 - min(3, max(0, (n - 1) >> 5))];               // class 0 = the largest graphs
-    }
-    Cnt4 before, total;
-    Scan(tmp).ExclusiveScan(mine, before, Cnt4{{0, 0, 0, 0}}, cub::Sum(), total);
-    int off[4];
-    off[0] = before.c[0];
-    off[1] = total.c[0] + before.c[1];
-    off[2] = total.c[0] + total.c[1] + before.c[2];
-    off[3] = total.c[0] + total.c[1] + total.c[2] + before.c[3];
-    for (int b = t; b < B; b += 1024) {
-        const int n = node_off[b + 1] - node_off[b];
-        order[off[3 - min(3, max(0, (n - 1) >> 5))]++] = b;
-    }
-}
-
-__global__ void __launch_bounds__(512)
-apsp_batched_v2_kernel(const int32_t *__restrict__ rowptr, const int32_t *__restrict__ col, const int32_t *__restrict__ node_off,
-                       const int64_t *__restrict__ hop_off, int B, int max_n, int warps_per_cta, uint8_t *__restrict__ hop,
-                       int32_t *__restrict__ cnt, float *__restrict__ rscale, int nbins, int32_t *__restrict__ overflow,
-                       int32_t *__restrict__ max_level, const int32_t *__restrict__ order)
-{
-    extern __shared__ __align__(16) uint8_t sm2[];
-    __shared__ float rcp_tab[256];
-    const bool levels = cnt != nullptr || rscale != nullptr;      // level sizes wanted (as counts and / or as 1/count)
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    if (rscale) {
-        for (int t = threadIdx.x; t < 256; t += blockDim.x) rcp_tab[t] = t > 0 ? 1.0f / (float)t : 0.f;   // as level_rscale_kernel
-        __syncthreads();
-    }
-    if (w >= warps_per_cta) return;
-    const int Wmax = (max_n + 31) / 32;
-    const size_t hop_bytes = bv2_round16((size_t)max_n * max_n + 16);
-    const size_t fr_bytes = bv2_round16((size_t)2 * max_n * Wmax * 4);        // keeps every warp's slice 16-byte aligned
-    const size_t cnt_bytes = levels ? bv2_round16((size_t)max_n * nbins) : 0;
-    uint8_t *wbase = sm2 + (size_t)w * (hop_bytes + fr_bytes + cnt_bytes);
-    uint32_t *frs = reinterpret_cast<uint32_t *>(wbase + hop_bytes);          // [2][n][W]
-    uint8_t *cs = wbase + hop_bytes + fr_bytes;                               // [n][nbins] level counts
-    const int64_t warp = (int64_t)blockIdx.x * warps_per_cta + w;
-    const int64_t nwarps = (int64_t)gridDim.x * warps_per_cta;
-    const bool vec_tab = (nbins & 3) == 0;
-    int lvl_max = 0;
-    for (int64_t bi = warp; bi < B; bi += nwarps) {
-        const int64_t b = order ? order[bi] : bi;
-        const int n0 = node_off[b], n = node_off[b + 1] - n0;
-        uint8_t *gb = hop + hop_off[b];
-        const int pad = (int)(reinterpret_cast<uintptr_t>(gb) & 15);
-        uint8_t *hb = wbase + pad;                                             // hb + k  ==  gb + k  (mod 16)
-        const int total = n * n;
-        __syncwarp();
-        for (int t = lane * 16; t < total + 16; t += 512)
-            *reinterpret_cast<uint4 *>(wbase + t) = make_uint4(0xffffffffu, 0xffffffffu, 0xffffffffu, 0xffffffffu);
-        if (levels)
-            for (int t = lane * 16; t < n * nbins; t += 512) *reinterpret_cast<uint4 *>(cs + t) = make_uint4(0u, 0u, 0u, 0u);
-        __syncwarp();
-        int lm;
-        if (n <= 32) lm = bv2_graph<1>(rowptr, col, n0, n, lane, hb, frs, cs, nbins, levels, overflow);
-        else if (n <= 64) lm = bv2_graph<2>(rowptr, col, n0, n, lane, hb, frs, cs, nbins, levels, overflow);
-        else if (n <= 96) lm = bv2_graph<3>(rowptr, col, n0, n, lane, hb, frs, cs, nbins, levels, overflow);
-        else lm = bv2_graph<4>(rowptr, col, n0, n, lane, hb, frs, cs, nbins, levels, overflow);
-        lvl_max = max(lvl_max, lm);
-        __syncwarp();
-        if (levels) {
-            const int nt = n * nbins;                                         // the graph's [n][nbins] block is contiguous
-            if (cnt) {
-                int32_t *gc = cnt + (int64_t)n0 * nbins;
-                if (vec_tab) {
-                    for (int t = lane * 4; t < nt; t += 128) {
-                        const uint32_t c4 = *reinterpret_cast<const uint32_t *>(cs + t);
-                        *reinterpret_cast<int4 *>(gc + t) = make_int4(c4 & 0xff, (c4 >> 8) & 0xff, (c4 >> 16) & 0xff, c4 >> 24);
-                    }
-                } else {
-                    for (int t = lane; t < nt; t += 32) gc[t] = cs[t];
-                }
-            }
-            if (rscale) {                       // 1/count (0 for empty levels): gnan_level_rscale fused; the 256 possible quotients come from a table
-                float *gr = rscale + (int64_t)n0 * nbins;
-                if (vec_tab) {
-                    for (int t = lane * 4; t < nt; t += 128) {
-                        const uint32_t c4 = *reinterpret_cast<const uint32_t *>(cs + t);
-                        *reinterpret_cast<float4 *>(gr + t) = make_float4(rcp_tab[c4 & 0xff], rcp_tab[(c4 >> 8) & 0xff],
-                                                                          rcp_tab[(c4 >> 16) & 0xff], rcp_tab[c4 >> 24]);
-                    }
-                } else {
-                    for (int t = lane; t < nt; t += 32) gr[t] = rcp_tab[cs[t]];
-                }
-            }
-        }
-        // copy out: head bytes up to the first 16-byte boundary, vector body, tail bytes
-        const int head = min(total, (16 - pad) & 15);
-        if (lane < head) gb[lane] = hb[lane];
-        const int body = (total - head) / 16;
-        for (int t = lane; t < body; t += 32)
-            *reinterpret_cast<uint4 *>(gb + head + t * 16) = *reinterpret_cast<const uint4 *>(hb + head + t * 16);
-        const int tail0 = head + body * 16;
-        if (tail0 + lane < total) gb[tail0 + lane] = hb[tail0 + lane];
-    }
-    if (max_level) {
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) lvl_max = max(lvl_max, __shfl_xor_sync(0xffffffffu, lvl_max, o));
-        if (lane == 0 && lvl_max > 0) atomicMax(max_level, lvl_max);
-    }
-}
-
-// ---- batched small graphs, v3: a GROUP of 4 warps per graph slot -----------------------------------------------------------
-// v2 is bound by the latency of ONE warp's dependent instruction stream per graph (a lane walks up to 4 vertices one after the
-// other, 10-12 graphs in flight per SM). Here a lane owns ONE vertex and the warps of a group advance a level together
+// ---- batched small graphs, v3: a GROUP of 4 warps per graph slot, bit-parallel over SOURCES -----------------------------------
+// A lane owns ONE vertex v and keeps the bitmask of sources that reach it (W = ceil(n/32) words). Level L is a pull over v's
+// out-neighbours u: new[v] = (OR_u frontier[u]) & ~visited[v]; a new bit s means dist(v -> s) = L, i.e. hop[v][s] = L, and
+// popc(new[v]) is row v's level-L count (no atomics). One warp per graph would be bound by the latency of its dependent
+// instruction stream (a lane walking up to 4 vertices one after the other), so the warps of a group advance a level together
 // (named barrier with an OR reduction = "did anybody reach a new vertex"): graphs of 65..128 nodes take the 4 warps of a group,
 // graphs of 33..64 nodes run two at a time on warp pairs, graphs of up to 32 nodes four at a time on single warps, each in its
-// share of the group's shared-memory slice. Same data flow as v2 otherwise (hop block assembled in shared memory, written
-// once; level sizes through a uint8 table).
+// share of the group's shared-memory slice.
+// The n x n hop block is assembled in shared memory (byte stores there), padded so that it is congruent to its global address
+// mod 16, and leaves as 16-byte vector stores: the global hop bytes are written exactly once, unreachable pairs included (no
+// memset). The level counts (<= 127 per entry) are collected in a uint8 [n][nbins] shared-memory table and leave as one
+// coalesced int32 block per graph, zeros included: no memset of the level table and no scattered 4-byte global stores per
+// (vertex, level), which cost a 32-byte sector each.
+constexpr int BV3_MAX_W = 4;                               // up to 128 nodes per graph
 constexpr int BV3_GW = 4;                                  // warps per group
 constexpr int BV3_MAX_GROUPS = 5;                          // groups per CTA (3 named barriers each: ids 1..15)
 
-__host__ __device__ inline size_t bv3_hop_bytes(int cap) { return bv2_round16((size_t)cap * cap + 16); }
+__host__ __device__ inline size_t round16(size_t x) { return (x + 15) / 16 * 16; }
+__host__ __device__ inline size_t bv3_hop_bytes(int cap) { return round16((size_t)cap * cap + 16); }
 __host__ __device__ constexpr int bv3_ws(int W) { return W == 3 ? 4 : W; }         // frontier row stride in words: 16-byte rows for W = 3
 // two frontier buffers [n][WS] (+ the adjacency bit matrix [n][WS] when the kernel builds it from the edge segment itself)
-// with pair statistics: + two fp32 [n] buffers of 1/count of the current level (by level parity)
-__host__ __device__ inline size_t bv3_fr_bytes(int cap, int W, bool local = false, bool pst = false)
+__host__ __device__ inline size_t bv3_fr_bytes(int cap, int W, bool local = false)
 {
-    return bv2_round16((size_t)(local ? 3 : 2) * cap * bv3_ws(W) * 4 + (pst ? (size_t)2 * cap * 4 : 0));
+    return round16((size_t)(local ? 3 : 2) * cap * bv3_ws(W) * 4);
 }
 
 // frontier rows move as ONE shared-memory access (LDS.128 / LDS.64 instead of W scalar loads per neighbour)
@@ -398,9 +153,9 @@ __device__ __forceinline__ void bv3_store_row(uint32_t *row, const uint32_t (&w)
     else if (W == 2) *reinterpret_cast<uint2 *>(row) = make_uint2(w[0], w[1]);
     else row[0] = w[0];
 }
-__host__ __device__ inline size_t bv3_need(int cap, int W, int nbins, bool levels, bool local = false, bool pst = false)
+__host__ __device__ inline size_t bv3_need(int cap, int W, int nbins, bool levels, bool local = false)
 {
-    return bv3_hop_bytes(cap) + bv3_fr_bytes(cap, W, local, pst) + (levels ? bv2_round16((size_t)cap * nbins) : 0);
+    return bv3_hop_bytes(cap) + bv3_fr_bytes(cap, W, local) + (levels ? round16((size_t)cap * nbins) : 0);
 }
 
 // up to 8 out-neighbours of a vertex travel with it as bytes of two registers (lo, hi), dg of them
@@ -479,17 +234,11 @@ __device__ __forceinline__ bool bv3_any(int bar, bool p)
 
 // one graph on G warps, W = ceil(n/32) <= G words per vertex; thread ts = wsub * 32 + lane owns vertex ts.
 // LOCAL: the out-neighbours come from the adjacency bit matrix adj [n][WS] in shared memory (built by bv3_run from the graph's own
-// edge segment) instead of the CSR.
-// PST (undirected graphs only): also the pair statistics P[d,v] = sum_{i: hop(i,v) = d} 1/count(i,d) of the output-normalised graph
-// readout (models.py:366-384), written LEVEL-MAJOR into the graph's block `pgraph` [nbins][n] (rows 0..deepest level and the
-// last one, the unreachable bin; the rows in between are never written nor read). By symmetry the vertices at distance d from v are v's own new
-// sources at level d, and count(i,d) is vertex i's popcount at that level: every lane publishes 1/count of the level in shared
-// memory (rcl, by level parity) and, after the level's barrier, sums it over its new bits in the same loop that scatters the hop
-// bytes. The aggregation forward then never reads the hop bytes or a normaliser table.
-template <int W, int G, bool LOCAL, bool PST>
+// edge segment) instead of the CSR. The hop bytes of a level are scattered two bits per step (lowest and highest new source).
+template <int W, int G, bool LOCAL>
 __device__ __forceinline__ int bv3_graph(const int32_t *__restrict__ rowptr, const int32_t *__restrict__ col, int n0, int n, int ts,
                                          int bar, uint8_t *hb, uint32_t *frs, const uint32_t *adj, uint8_t *cs, int nbins, bool levels,
-                                         int32_t *overflow, float *rcl, float *pgraph)
+                                         int32_t *overflow)
 {
     constexpr int WS = bv3_ws(W);
     const int v = ts, lane = ts & 31, wsub = ts >> 5;
@@ -517,8 +266,6 @@ __device__ __forceinline__ int bv3_graph(const int32_t *__restrict__ rowptr, con
         if (levels) cs[v * nbins] = 1;
     }
     bv3_sync<G>(bar);
-    uint32_t nw[PST ? W : 1];                                     // PST: the new bits of the level, scattered after its barrier
-    if (PST && mine) pgraph[v] = 1.f;                             // level 0: v itself, count 1
     int lvl_max = 0;
     for (int level = 1; level <= n; ++level) {
         const uint32_t *fc = frs + ((level - 1) & 1) * n * WS;
@@ -546,23 +293,17 @@ __device__ __forceinline__ int bv3_graph(const int32_t *__restrict__ rowptr, con
                 newc += __popc(acc[ww]);
             }
             bv3_store_row<W>(fn + v * WS, acc);
-            if (!PST) {
 #pragma unroll
-                for (int ww = 0; ww < W; ++ww) {
-                    uint32_t m = acc[ww];
-                    uint8_t *rowp = hb + v * n + ww * 32;
-                    while (m) {
-                        const int lo = __ffs(m) - 1, hi = 31 - __clz(m);
-                        rowp[lo] = lv;
-                        rowp[hi] = lv;
-                        m &= m - 1;
-                        m &= ~(1u << hi);
-                    }
+            for (int ww = 0; ww < W; ++ww) {
+                uint32_t m = acc[ww];
+                uint8_t *rowp = hb + v * n + ww * 32;
+                while (m) {
+                    const int lo = __ffs(m) - 1, hi = 31 - __clz(m);
+                    rowp[lo] = lv;
+                    rowp[hi] = lv;
+                    m &= m - 1;
+                    m &= ~(1u << hi);
                 }
-            } else {
-                rcl[(level & 1) * n + v] = newc ? __frcp_rn((float)newc) : 0.f;
-#pragma unroll
-                for (int ww = 0; ww < W; ++ww) nw[ww] = acc[ww];
             }
             if (newc) {
                 any = true;
@@ -572,56 +313,18 @@ __device__ __forceinline__ int bv3_graph(const int32_t *__restrict__ rowptr, con
         }
         if (!bv3_any<G>(bar, any)) break;
         lvl_max = level;
-        if (PST && mine) {                                       // after the barrier: everybody's 1/count of this level is visible
-            const float *rc = rcl + (level & 1) * n;
-            float ps = 0.f, ps2 = 0.f;                            // two independent chains (lowest / highest new source)
-#pragma unroll
-            for (int ww = 0; ww < W; ++ww) {
-                uint32_t m = nw[ww];
-                uint8_t *rowp = hb + v * n + ww * 32;
-                const float *rcw = rc + ww * 32;
-                while (m) {
-                    const int lo = __ffs(m) - 1, hi = 31 - __clz(m);
-                    rowp[lo] = lv;
-                    rowp[hi] = lv;
-                    ps += rcw[lo];
-                    ps2 += hi != lo ? rcw[hi] : 0.f;
-                    m &= m - 1;
-                    m &= ~(1u << hi);
-                }
-            }
-            if (level < nbins - 1) pgraph[level * n + v] = ps + ps2;   // level-major: a warp writes 32 consecutive floats
-        }
     }
     int reached = 0;
 #pragma unroll
     for (int ww = 0; ww < W; ++ww) reached += __popc(vis[ww]);
     if (levels && mine) cs[v * nbins + nbins - 1] = (uint8_t)(n - reached);
-    if (PST) {
-        // unreachable bin: sum over the vertices outside v's component of 1/(their unreachable count); skipped for connected graphs
-        float U = 0.f;
-        if (bv3_any<G>(bar, mine && reached < n)) {
-            if (mine) rcl[v] = reached < n ? __frcp_rn((float)(n - reached)) : 0.f;
-            bv3_sync<G>(bar);
-            if (mine) {
-#pragma unroll
-                for (int ww = 0; ww < W; ++ww) {
-                    const int left = n - ww * 32;
-                    uint32_t m = ~vis[ww] & (left >= 32 ? 0xffffffffu : (left > 0 ? (1u << left) - 1u : 0u));
-                    while (m) {
-                        U += rcl[ww * 32 + __ffs(m) - 1];
-                        m &= m - 1;
-                    }
-                }
-            }
-        }
-        if (mine) pgraph[(nbins - 1) * n + v] = U;
-    }
     return lvl_max;
 }
 
 // graphs by word-count class (0 = 97..128 nodes ... 3 = up to 32), one thread per graph, warp-aggregated counters:
-// cls[0..4) = class sizes (zeroed by the caller), cls[4 + c * B ...) = the graphs of class c in arbitrary order
+// cls[0..4) = class sizes (zeroed by the caller), cls[4 + c * B ...) = the graphs of class c in arbitrary order.
+// The v3 kernel walks the classes largest first: the expensive graphs start first, and the groups of a CTA run the same
+// instantiation of bv3_graph side by side (the instantiations do not fit the instruction cache together).
 __global__ void bv3_classify_kernel(const int32_t *__restrict__ node_off, int B, int32_t *__restrict__ cls)
 {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
@@ -647,12 +350,10 @@ struct Bv3Out {
     const uint8_t *lsrc, *ldst;
     const int32_t *edge_off;
     int32_t *status;
-    float *pstat;        // PST: pair statistics, graph b's level-major block [nbins][n_b] at n0_b * nbins (status |= 4 when a graph's
-    int32_t *pdepth;     // adjacency is not symmetric); pdepth[b] = deepest level written
 };
 
 // graph b on the G warps of a sub-group: fill the slice, BFS, write the level table and the hop block out
-template <int W, int G, bool LOCAL, bool PST>
+template <int W, int G, bool LOCAL>
 __device__ __forceinline__ int bv3_run(const int32_t *__restrict__ rowptr, const int32_t *__restrict__ col,
                                        const int32_t *__restrict__ node_off, const int64_t *__restrict__ hop_off, int64_t b, int cap,
                                        int ts, int bar, uint8_t *slice, const Bv3Out &o, bool levels, int32_t *overflow)
@@ -665,8 +366,7 @@ __device__ __forceinline__ int bv3_run(const int32_t *__restrict__ rowptr, const
     constexpr int WS = bv3_ws(W);
     uint32_t *frs = reinterpret_cast<uint32_t *>(slice + bv3_hop_bytes(cap));  // [2][n][WS] (+ adjacency [n][WS])
     uint32_t *adj = frs + 2 * n * WS;
-    float *rcl = reinterpret_cast<float *>(adj + n * WS);                      // PST: [2][n] 1/count of the current level
-    uint8_t *cs = slice + bv3_hop_bytes(cap) + bv3_fr_bytes(cap, W, LOCAL, PST);   // [n][nbins]
+    uint8_t *cs = slice + bv3_hop_bytes(cap) + bv3_fr_bytes(cap, W, LOCAL);   // [n][nbins]
     const int total = n * n;
     for (int t = ts * 16; t < total + 16; t += T * 16)
         *reinterpret_cast<uint4 *>(slice + t) = make_uint4(0xffffffffu, 0xffffffffu, 0xffffffffu, 0xffffffffu);
@@ -686,19 +386,10 @@ __device__ __forceinline__ int bv3_run(const int32_t *__restrict__ rowptr, const
                 flags |= 1;
             }
         }
-        if (PST) {                                               // the pair statistics rely on hop(i,j) = hop(j,i)
-            bv3_sync<G>(bar);
-            for (int e = e0 + ts; e < e1; e += T) {
-                const uint32_t s = o.lsrc[e], d = o.ldst[e];
-                if (s < (uint32_t)n && d < (uint32_t)n && !((adj[d * WS + (s >> 5)] >> (s & 31)) & 1u)) flags |= 4;
-            }
-        }
         if (flags) atomicOr(o.status, flags);
     }
     bv3_sync<G>(bar);
-    const int lm = bv3_graph<W, G, LOCAL, PST>(rowptr, col, n0, n, ts, bar, hb, frs, adj, cs, nbins, levels, overflow, rcl,
-                                               PST ? o.pstat + (int64_t)n0 * nbins : nullptr);
-    if (PST && ts == 0) o.pdepth[b] = min(lm, nbins - 2);
+    const int lm = bv3_graph<W, G, LOCAL>(rowptr, col, n0, n, ts, bar, hb, frs, adj, cs, nbins, levels, overflow);
     bv3_sync<G>(bar);
     if (levels) {
         const int nt = n * nbins;                                               // the graph's [n][nbins] block is contiguous
@@ -757,7 +448,7 @@ struct Bv3Readout {
 // frontier rows [2][cap][WS], adjacency [cap][WS], 1/count [2][cap], per-warp Q [G][nbins][CC] + per-warp out [G][CC]
 __host__ __device__ inline size_t bv3_ro_need(int cap, int W, int G, int nbins, int CC)
 {
-    return bv2_round16((size_t)3 * cap * bv3_ws(W) * 4 + (size_t)2 * cap * 4 + (size_t)G * (nbins + 1) * CC * 4);
+    return round16((size_t)3 * cap * bv3_ws(W) * 4 + (size_t)2 * cap * 4 + (size_t)G * (nbins + 1) * CC * 4);
 }
 
 // lane's share of bin d: colw += T[d,:] p, the warp's Q slot [d,:] = sum over the warp's lanes of S[v,:] p (all 32 lanes call it)
@@ -939,13 +630,13 @@ __device__ __forceinline__ int bv3_readout_run(const int32_t *__restrict__ node_
 }
 
 // one work item of the v3 kernel: the BFS of bv3_run, or (CC > 0) the BFS fused with the graph readout
-template <int W, int G, bool LOCAL, bool PST, int CC>
+template <int W, int G, bool LOCAL, int CC>
 __device__ __forceinline__ int bv3_item(const int32_t *__restrict__ rowptr, const int32_t *__restrict__ col,
                                         const int32_t *__restrict__ node_off, const int64_t *__restrict__ hop_off, int64_t b, int cap,
                                         int ts, int bar, uint8_t *slice, const Bv3Out &o, const Bv3Readout &r, bool levels, int32_t *overflow)
 {
     if constexpr (CC > 0) return bv3_readout_run<W, G, CC>(node_off, b, ts, bar, slice, o, r, overflow);
-    else return bv3_run<W, G, LOCAL, PST>(rowptr, col, node_off, hop_off, b, cap, ts, bar, slice, o, levels, overflow);
+    else return bv3_run<W, G, LOCAL>(rowptr, col, node_off, hop_off, b, cap, ts, bar, slice, o, levels, overflow);
 }
 
 // the batch's edge list in its transfer form (LOCAL instantiation: no CSR; rowptr / col are NULL)
@@ -953,16 +644,13 @@ struct Bv3Edges {
     const uint8_t *src, *dst;
     const int32_t *edge_off;
     int32_t *status;
-    float *pstat;
-    int32_t *pdepth;
 };
 
 // order = the output of bv3_classify_kernel
-// (the pair-statistics and the multi-channel readout instantiations keep the level's new bits across the barrier: 4 groups per
-// CTA give them 64 registers)
-constexpr int bv3_max_groups(bool pst, int cc) { return pst || cc > 1 ? BV3_MAX_GROUPS - 1 : BV3_MAX_GROUPS; }
-template <bool LOCAL, bool PST, int CC = 0>
-__global__ void __launch_bounds__(32 * BV3_GW * bv3_max_groups(PST, CC), 2)
+// (the multi-channel readout instantiations keep the level's new bits across the barrier: 4 groups per CTA give them 64 registers)
+constexpr int bv3_max_groups(int cc) { return cc > 1 ? BV3_MAX_GROUPS - 1 : BV3_MAX_GROUPS; }
+template <bool LOCAL, int CC = 0>
+__global__ void __launch_bounds__(32 * BV3_GW * bv3_max_groups(CC), 2)
 apsp_batched_v3_kernel(const int32_t *__restrict__ rowptr, const int32_t *__restrict__ col, const int32_t *__restrict__ node_off,
                        const int64_t *__restrict__ hop_off, int B, int max_n, int groups_per_cta, int slice_bytes, uint8_t *__restrict__ hop,
                        int32_t *__restrict__ cnt, float *__restrict__ rscale, int nbins, int32_t *__restrict__ overflow,
@@ -978,7 +666,7 @@ apsp_batched_v3_kernel(const int32_t *__restrict__ rowptr, const int32_t *__rest
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, g = warp / BV3_GW, wq = warp % BV3_GW;
     uint8_t *gslice = sm3 + (size_t)g * slice_bytes;
     const int bar_group = 1 + 3 * g;
-    const Bv3Out out{hop, cnt, rscale, rcp_tab, nbins, le.src, le.dst, le.edge_off, le.status, le.pstat, le.pdepth};
+    const Bv3Out out{hop, cnt, rscale, rcp_tab, nbins, le.src, le.dst, le.edge_off, le.status};
     const int c0 = order[0], c_big = c0 + order[1], c2 = order[2], c3 = order[3];
     const int32_t *ord0 = order + 4, *ord1 = ord0 + B, *ord2 = ord1 + B, *ord3 = ord2 + B;
     const int items2 = (c2 + 1) / 2, items1 = (c3 + 3) / 4;
@@ -991,20 +679,20 @@ apsp_batched_v3_kernel(const int32_t *__restrict__ rowptr, const int32_t *__rest
             const int64_t b = t < c0 ? ord0[t] : ord1[t - c0];
             const int n = node_off[b + 1] - node_off[b];
             const int ts = wq * 32 + lane;
-            const int lm = n <= 96 ? bv3_item<3, 4, LOCAL, PST, CC>(rowptr, col, node_off, hop_off, b, max_n, ts, bar_group, gslice, out, ro, levels, overflow)
-                                   : bv3_item<4, 4, LOCAL, PST, CC>(rowptr, col, node_off, hop_off, b, max_n, ts, bar_group, gslice, out, ro, levels, overflow);
+            const int lm = n <= 96 ? bv3_item<3, 4, LOCAL, CC>(rowptr, col, node_off, hop_off, b, max_n, ts, bar_group, gslice, out, ro, levels, overflow)
+                                   : bv3_item<4, 4, LOCAL, CC>(rowptr, col, node_off, hop_off, b, max_n, ts, bar_group, gslice, out, ro, levels, overflow);
             lvl_max = max(lvl_max, lm);
         } else if (t < c_big + items2) {                             // 33..64 nodes: two graphs on the two warp pairs
             const int pr = wq >> 1;
             const int64_t idx = 2 * (t - c_big) + pr;
             if (idx < c2)
-                lvl_max = max(lvl_max, bv3_item<2, 2, LOCAL, PST, CC>(rowptr, col, node_off, hop_off, ord2[idx], cap2, (wq & 1) * 32 + lane,
-                                                          bar_group + 1 + pr, gslice + (size_t)pr * half, out, ro, levels, overflow));
+                lvl_max = max(lvl_max, bv3_item<2, 2, LOCAL, CC>(rowptr, col, node_off, hop_off, ord2[idx], cap2, (wq & 1) * 32 + lane,
+                                                     bar_group + 1 + pr, gslice + (size_t)pr * half, out, ro, levels, overflow));
         } else {                                                     // up to 32 nodes: four graphs, a warp each
             const int64_t idx = 4 * (t - c_big - items2) + wq;
             if (idx < c3)
-                lvl_max = max(lvl_max, bv3_item<1, 1, LOCAL, PST, CC>(rowptr, col, node_off, hop_off, ord3[idx], cap1, lane, 0,
-                                                          gslice + (size_t)wq * quarter, out, ro, levels, overflow));
+                lvl_max = max(lvl_max, bv3_item<1, 1, LOCAL, CC>(rowptr, col, node_off, hop_off, ord3[idx], cap1, lane, 0,
+                                                     gslice + (size_t)wq * quarter, out, ro, levels, overflow));
         }
         bv3_sync<BV3_GW>(bar_group);                                 // the slice is re-partitioned / refilled by the next item
     }
@@ -1311,22 +999,22 @@ extern "C" int gnan_apsp_msbfs(const int32_t *rowptr, const int32_t *col, int32_
 
 // v3 launch: groups of 4 warps; the group's slice holds one graph of 65..128 nodes, two of 33..64 or four of up to 32
 // CC > 0: the BFS fused with the graph readout (bv3_readout_run; ro holds its tensors, hop / cnt / rscale are NULL)
-template <bool LOCAL, bool PST, int CC = 0>
+template <bool LOCAL, int CC = 0>
 static int launch_bv3(const int32_t *rowptr, const int32_t *col, const int32_t *node_off, const int64_t *hop_off, int32_t B, int32_t max_n,
                       uint8_t *hop, int32_t *cnt, float *rscale, int nb, bool levels, int32_t *overflow_flag, int32_t *max_level,
                       int32_t *order_ws, Bv3Edges le, cudaStream_t st, Bv3Readout ro = Bv3Readout{})
 {
     const int Wmax = (max_n + 31) / 32;
     auto need = [&](int cap, int W, int G) {
-        return CC > 0 ? bv3_ro_need(cap, W, G, nb, CC) : bv3_need(cap, W, nb, levels, LOCAL, PST);
+        return CC > 0 ? bv3_ro_need(cap, W, G, nb, CC) : bv3_need(cap, W, nb, levels, LOCAL);
     };
     size_t slice = 4 * need(std::min(max_n, 32), 1, 1);
     if (Wmax >= 2) slice = std::max(slice, 2 * need(std::min(max_n, 64), 2, 2));
     if (Wmax >= 3) slice = std::max(slice, need(max_n, Wmax, 4));
-    const int gpc = (int)std::min<size_t>(bv3_max_groups(PST, CC), (112 * 1024) / slice);     // two CTAs per SM
+    const int gpc = (int)std::min<size_t>(bv3_max_groups(CC), (112 * 1024) / slice);     // two CTAs per SM
     if (gpc < 1) return GNAN_ERR_UNSUPPORTED;
     const size_t smem3 = slice * gpc;
-    auto kernel = apsp_batched_v3_kernel<LOCAL, PST, CC>;
+    auto kernel = apsp_batched_v3_kernel<LOCAL, CC>;
     static thread_local size_t cached_smem3 = 0;
     static thread_local int cached_gpc = 0, cached_per_sm3 = 0;
     if (cached_smem3 != smem3 || cached_gpc != gpc || cached_per_sm3 == 0) {
@@ -1344,73 +1032,11 @@ static int launch_bv3(const int32_t *rowptr, const int32_t *col, const int32_t *
     return GNAN_OK;
 }
 
-// max_n is needed to size shared memory; exported variant with it explicit (the header-declared entry derives it on the host side)
-extern "C" int gnan_apsp_bfs_batched_n(const int32_t *rowptr, const int32_t *col, const int32_t *node_off, const int64_t *hop_off,
-                                       int32_t B, int32_t max_n, int64_t total_nodes, int64_t total_hop_bytes, uint8_t *hop,
-                                       int32_t *cnt, int32_t nbins, int32_t *overflow_flag, int32_t *max_level, gnan_stream_t stream)
+// the lane-per-source kernel for graphs of up to 256 nodes (the caller has checked the arguments)
+static int launch_batched_lanes(const int32_t *rowptr, const int32_t *col, const int32_t *node_off, const int64_t *hop_off, int32_t B,
+                                int32_t max_n, int64_t total_nodes, int64_t total_hop_bytes, uint8_t *hop, int32_t *cnt, int32_t nbins,
+                                int32_t *overflow_flag, int32_t *max_level, cudaStream_t st)
 {
-    return gnan_apsp_bfs_batched_ex(rowptr, col, node_off, hop_off, B, max_n, total_nodes, total_hop_bytes, hop, cnt, nullptr, nbins,
-                                    overflow_flag, max_level, nullptr, stream);
-}
-
-// rscale (optional): 1/count per (node, level) as fp32, what gnan_level_rscale would compute from cnt; cnt may then be NULL
-extern "C" int gnan_apsp_bfs_batched_ex(const int32_t *rowptr, const int32_t *col, const int32_t *node_off, const int64_t *hop_off,
-                                        int32_t B, int32_t max_n, int64_t total_nodes, int64_t total_hop_bytes, uint8_t *hop,
-                                        int32_t *cnt, float *rscale, int32_t nbins, int32_t *overflow_flag, int32_t *max_level,
-                                        int32_t *order_ws, gnan_stream_t stream)
-{
-    GNAN_REQUIRE(B >= 0, "apsp_bfs_batched: negative batch");
-    if (B == 0) return GNAN_OK;
-    GNAN_REQUIRE(rowptr && node_off && hop_off && hop && overflow_flag, "apsp_bfs_batched: NULL pointer");
-    GNAN_REQUIRE(!(cnt || rscale) || (nbins >= 2 && nbins <= 256), "apsp_bfs_batched: nbins %d out of [2,256]", nbins);
-    if (rscale && !(max_n <= 32 * BV2_W && total_nodes > 0)) {
-        gnan_set_error("apsp_bfs_batched: the fused 1/count output needs graphs of at most %d nodes and the totals", 32 * BV2_W);
-        return GNAN_ERR_UNSUPPORTED;
-    }
-    if (max_n < 1 || max_n > 32 * BW_MAX) {
-        gnan_set_error("apsp_bfs_batched: graphs with %d nodes unsupported (1..%d); use gnan_apsp_bfs", max_n, 32 * BW_MAX);
-        return GNAN_ERR_UNSUPPORTED;
-    }
-    cudaStream_t st = (cudaStream_t)stream;
-    if (max_n <= 32 * BV2_W && total_nodes > 0) {
-        const bool levels = cnt || rscale;
-        const int nb = levels ? nbins : 256;
-        static const bool force_v2 = getenv("GNAN_BFS_V2") != nullptr;
-        if (order_ws && !force_v2) {
-            const int rc3 = launch_bv3<false, false>(rowptr, col, node_off, hop_off, B, max_n, hop, cnt, rscale, nb, levels, overflow_flag,
-                                                     max_level, order_ws, Bv3Edges{nullptr, nullptr, nullptr, nullptr, nullptr, nullptr}, st);
-            if (rc3 != GNAN_ERR_UNSUPPORTED) return rc3;
-        }
-        // v2: one warp per graph; hop blocks assembled in shared memory and written once (no memset of hop)
-        const int Wmax = (max_n + 31) / 32;
-        const size_t per_warp = bv2_round16((size_t)max_n * max_n + 16) + bv2_round16((size_t)2 * max_n * Wmax * 4) +
-                                ((cnt || rscale) ? bv2_round16((size_t)max_n * nbins) : 0);
-        int wpc = (int)std::min<size_t>(16, (216 * 1024) / per_warp);         // one CTA per SM holding as many graphs (warps) as fit
-        if (wpc > 8 && (wpc & 1)) --wpc;
-        if (wpc >= 8 && 2 * per_warp * (wpc / 2) + 4096 <= 216 * 1024) wpc /= 2;      // two CTAs per SM when the halves fit too
-        if (wpc < 1) wpc = 1;
-        const size_t smem = per_warp * wpc;
-        static thread_local size_t cached_smem = 0;       // attribute + occupancy once per configuration (host time)
-        static thread_local int cached_wpc = 0, cached_per_sm = 0;
-        if (cached_smem != smem || cached_wpc != wpc || cached_per_sm == 0) {
-            GNAN_CUDA(cudaFuncSetAttribute(apsp_batched_v2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            GNAN_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cached_per_sm, apsp_batched_v2_kernel, 32 * wpc, smem));
-            cached_smem = smem; cached_wpc = wpc;
-        }
-        const int per_sm = cached_per_sm;
-        // persistent: every resident warp walks its share of the graphs (their cost varies like n^2 x depth: many per warp average out)
-        const int blocks = (int)std::min<int64_t>(ceil_div64(B, wpc), (int64_t)std::max(per_sm, 1) * gnan_sm_count());
-        if (order_ws && max_n > 32) {                 // mixed word counts: group the graphs by instantiation
-            bv2_order_kernel<<<1, 1024, 0, st>>>(node_off, B, order_ws);
-            GNAN_LAUNCH_OK();
-        } else {
-            order_ws = nullptr;
-        }
-        apsp_batched_v2_kernel<<<blocks, 32 * wpc, smem, st>>>(rowptr, col, node_off, hop_off, B, max_n, wpc, hop, cnt, rscale,
-                                                              (cnt || rscale) ? nbins : 256, overflow_flag, max_level, order_ws);
-        GNAN_LAUNCH_OK();
-        return GNAN_OK;
-    }
     const size_t smem = sizeof(uint32_t) * 8 * (size_t)max_n * ((max_n + 31) / 32);
     GNAN_CUDA(cudaFuncSetAttribute(apsp_batched_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int blocks = (int)std::min<int64_t>(ceil_div64(B, 8), 16 * gnan_sm_count());
@@ -1426,11 +1052,43 @@ extern "C" int gnan_apsp_bfs_batched_ex(const int32_t *rowptr, const int32_t *co
     return GNAN_OK;
 }
 
+// graphs of at most 128 nodes with known totals: v3; anything else: the lane-per-source kernel.
+// rscale (optional): 1/count per (node, level) as fp32, what gnan_level_rscale would compute from cnt; cnt may then be NULL
+extern "C" int gnan_apsp_bfs_batched_ex(const int32_t *rowptr, const int32_t *col, const int32_t *node_off, const int64_t *hop_off,
+                                        int32_t B, int32_t max_n, int64_t total_nodes, int64_t total_hop_bytes, uint8_t *hop,
+                                        int32_t *cnt, float *rscale, int32_t nbins, int32_t *overflow_flag, int32_t *max_level,
+                                        int32_t *order_ws, gnan_stream_t stream)
+{
+    GNAN_REQUIRE(B >= 0, "apsp_bfs_batched: negative batch");
+    if (B == 0) return GNAN_OK;
+    GNAN_REQUIRE(rowptr && node_off && hop_off && hop && overflow_flag, "apsp_bfs_batched: NULL pointer");
+    GNAN_REQUIRE(order_ws, "apsp_bfs_batched: NULL order_ws");
+    GNAN_REQUIRE(!(cnt || rscale) || (nbins >= 2 && nbins <= 256), "apsp_bfs_batched: nbins %d out of [2,256]", nbins);
+    if (rscale && !(max_n <= 32 * BV3_MAX_W && total_nodes > 0)) {
+        gnan_set_error("apsp_bfs_batched: the fused 1/count output needs graphs of at most %d nodes and the totals", 32 * BV3_MAX_W);
+        return GNAN_ERR_UNSUPPORTED;
+    }
+    if (max_n < 1 || max_n > 32 * BW_MAX) {
+        gnan_set_error("apsp_bfs_batched: graphs with %d nodes unsupported (1..%d); use gnan_apsp_bfs", max_n, 32 * BW_MAX);
+        return GNAN_ERR_UNSUPPORTED;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    if (max_n <= 32 * BV3_MAX_W && total_nodes > 0) {
+        const bool levels = cnt || rscale;
+        const int rc = launch_bv3<false>(rowptr, col, node_off, hop_off, B, max_n, hop, cnt, rscale, levels ? nbins : 256, levels,
+                                         overflow_flag, max_level, order_ws, Bv3Edges{}, st);
+        if (rc == GNAN_ERR_UNSUPPORTED) gnan_set_error("apsp_bfs_batched: level table too wide for the shared-memory slice");
+        return rc;
+    }
+    return launch_batched_lanes(rowptr, col, node_off, hop_off, B, max_n, total_nodes, total_hop_bytes, hop, cnt, nbins, overflow_flag,
+                                max_level, st);
+}
+
 // The batched BFS straight from the batch's edge list in its transfer form (no CSR): see include/gnan_b200.h
 extern "C" int gnan_apsp_bfs_batched_local(const uint8_t *src, const uint8_t *dst, const int32_t *edge_off, const int32_t *node_off,
                                            const int64_t *hop_off, int32_t B, int32_t max_n, uint8_t *hop, int32_t *cnt, float *rscale,
-                                           float *pstat, int32_t *pdepth, int32_t nbins, int32_t *status, int32_t *overflow_flag,
-                                           int32_t *max_level, int32_t *order_ws, gnan_stream_t stream)
+                                           int32_t nbins, int32_t *status, int32_t *overflow_flag, int32_t *max_level, int32_t *order_ws,
+                                           gnan_stream_t stream)
 {
     GNAN_REQUIRE(B >= 0, "apsp_bfs_batched_local: negative batch");
     GNAN_REQUIRE(status != nullptr, "apsp_bfs_batched_local: NULL status");
@@ -1438,20 +1096,16 @@ extern "C" int gnan_apsp_bfs_batched_local(const uint8_t *src, const uint8_t *ds
     GNAN_CUDA(cudaMemsetAsync(status, 0, sizeof(int32_t), st));
     if (B == 0) return GNAN_OK;
     GNAN_REQUIRE(edge_off && node_off && hop_off && hop && overflow_flag && order_ws, "apsp_bfs_batched_local: NULL pointer");
-    GNAN_REQUIRE(!(cnt || rscale || pstat) || (nbins >= 2 && nbins <= 256), "apsp_bfs_batched_local: nbins %d out of [2,256]", nbins);
-    GNAN_REQUIRE(!pstat == !pdepth, "apsp_bfs_batched_local: pstat and pdepth go together");
-    if (max_n < 1 || max_n > 32 * BV2_W) {
+    GNAN_REQUIRE(!(cnt || rscale) || (nbins >= 2 && nbins <= 256), "apsp_bfs_batched_local: nbins %d out of [2,256]", nbins);
+    if (max_n < 1 || max_n > 32 * BV3_MAX_W) {
         gnan_set_error("apsp_bfs_batched_local: graphs with %d nodes unsupported (1..%d); expand the edges and use gnan_apsp_bfs_batched_ex",
-                       max_n, 32 * BV2_W);
+                       max_n, 32 * BV3_MAX_W);
         return GNAN_ERR_UNSUPPORTED;
     }
     const bool levels = cnt || rscale;
-    const int nb = (levels || pstat) ? nbins : 256;
-    const Bv3Edges le{src, dst, edge_off, status, pstat, pdepth};
-    const int rc = pstat ? launch_bv3<true, true>(nullptr, nullptr, node_off, hop_off, B, max_n, hop, cnt, rscale, nb, levels, overflow_flag,
-                                                  max_level, order_ws, le, st)
-                         : launch_bv3<true, false>(nullptr, nullptr, node_off, hop_off, B, max_n, hop, cnt, rscale, nb, levels, overflow_flag,
-                                                   max_level, order_ws, le, st);
+    const Bv3Edges le{src, dst, edge_off, status};
+    const int rc = launch_bv3<true>(nullptr, nullptr, node_off, hop_off, B, max_n, hop, cnt, rscale, levels ? nbins : 256, levels,
+                                    overflow_flag, max_level, order_ws, le, st);
     if (rc == GNAN_ERR_UNSUPPORTED) gnan_set_error("apsp_bfs_batched_local: level table too wide for the shared-memory slice");
     return rc;
 }
@@ -1473,15 +1127,15 @@ extern "C" int gnan_bfs_graph_readout_fwd(const uint8_t *src, const uint8_t *dst
     if (B == 0) return GNAN_OK;
     GNAN_REQUIRE(src && dst && edge_off && node_off && T && S && out && colw && Q && overflow_flag && order_ws,
                  "bfs_graph_readout_fwd: NULL pointer");
-    if (max_n < 1 || max_n > 32 * BV2_W) {
-        gnan_set_error("bfs_graph_readout_fwd: graphs with %d nodes unsupported (1..%d)", max_n, 32 * BV2_W);
+    if (max_n < 1 || max_n > 32 * BV3_MAX_W) {
+        gnan_set_error("bfs_graph_readout_fwd: graphs with %d nodes unsupported (1..%d)", max_n, 32 * BV3_MAX_W);
         return GNAN_ERR_UNSUPPORTED;
     }
-    const Bv3Edges le{src, dst, edge_off, status, nullptr, nullptr};
+    const Bv3Edges le{src, dst, edge_off, status};
     const Bv3Readout ro{T, S, Cr, C, out, colw, Q};
     auto launch = [&](auto cc) {
-        return launch_bv3<true, false, decltype(cc)::value>(nullptr, nullptr, node_off, nullptr, B, max_n, nullptr, nullptr, nullptr, nbins,
-                                                            false, overflow_flag, max_level, order_ws, le, st, ro);
+        return launch_bv3<true, decltype(cc)::value>(nullptr, nullptr, node_off, nullptr, B, max_n, nullptr, nullptr, nullptr, nbins, false,
+                                                     overflow_flag, max_level, order_ws, le, st, ro);
     };
     const int rc = C == 1 ? launch(std::integral_constant<int, 1>{}) : C == 2 ? launch(std::integral_constant<int, 2>{})
                                                                              : launch(std::integral_constant<int, 4>{});
@@ -1493,8 +1147,13 @@ extern "C" int gnan_apsp_bfs_batched(const int32_t *rowptr, const int32_t *col, 
                                      int32_t B, uint8_t *hop, int32_t *cnt, int32_t nbins, int32_t *overflow_flag,
                                      gnan_stream_t stream)
 {
+    GNAN_REQUIRE(B >= 0, "apsp_bfs_batched: negative batch");
+    if (B == 0) return GNAN_OK;
+    GNAN_REQUIRE(rowptr && node_off && hop_off && hop && overflow_flag, "apsp_bfs_batched: NULL pointer");
+    GNAN_REQUIRE(!cnt || (nbins >= 2 && nbins <= 256), "apsp_bfs_batched: nbins %d out of [2,256]", nbins);
     // without a host-side size hint assume the largest supported graph
-    return gnan_apsp_bfs_batched_n(rowptr, col, node_off, hop_off, B, 32 * BW_MAX, 0, 0, hop, cnt, nbins, overflow_flag, nullptr, stream);
+    return launch_batched_lanes(rowptr, col, node_off, hop_off, B, 32 * BW_MAX, 0, 0, hop, cnt, nbins, overflow_flag, nullptr,
+                                (cudaStream_t)stream);
 }
 
 extern "C" int gnan_hops_to_reference(const uint8_t *hop, int64_t R, int64_t N, int64_t ld_hop, const int32_t *cnt,

@@ -103,12 +103,6 @@ class TensorGNAN(_Base):
             # kernel, neither the hop bytes nor the normaliser table are ever written (models.py:366-384)
             out = ops.bfs_graph_readout(pk.edges, pk.node_off, pk.max_nodes, T, S, pk.status)
             return self.readout_nam(out) if self._readout else out
-        if getattr(pk, "pair_stats", None) is not None and self.normalize_rho and self.is_graph_task and T.dim() == 2:
-            # the batched BFS accumulated the pair statistics of this readout itself: no pass over the hop bytes (models.py:366-384)
-            out = ops.aggregate_blockdiag_pairs(pk.pair_stats, pk.pair_depth, pk.node_off, T, S)
-            return self.readout_nam(out) if self._readout else out
-        if pk.level_counts is None and getattr(pk, "level_rscale", None) is None:
-            raise ValueError("this batch carries pair statistics only (output-normalised graph readout with a global table)")
         rs = None
         if self.normalize_rho:       # models.py:368-370; a batch straight from apsp_batched(..., rscale=True) carries it already
             rs = pk.level_rscale if getattr(pk, "level_rscale", None) is not None else ops.level_rscale(pk.level_counts)

@@ -10,7 +10,7 @@ from torch import Tensor
 from . import _lib
 from ._lib import MlpGrads, MlpParams, check, load, ptr, stream_handle
 
-__all__ = ["mlp", "aggregate_rows", "aggregate_blockdiag", "aggregate_blockdiag_pairs", "rho_table_inputs", "level_rscale", "alloc_hop", "hop_ld",
+__all__ = ["mlp", "aggregate_rows", "aggregate_blockdiag", "rho_table_inputs", "level_rscale", "alloc_hop", "hop_ld",
            "cross_entropy_rows", "bce_with_logits"]
 
 
@@ -496,54 +496,6 @@ def _bdg_backward(ctx, g, _g_colw, _g_q):
 
 
 agg_bd_graph_fwd.register_autograd(_bdg_backward, setup_context=_bdg_setup)
-
-@torch.library.custom_op("gnan_b200::agg_bd_graph_pairs_fwd", mutates_args=())
-def agg_bd_graph_pairs_fwd(pstat: Tensor, pdepth: Tensor, node_off: Tensor, T: Tensor, S: Tensor) -> Tuple[Tensor, Tensor, Tensor]:
-    """Graph readout from the pair statistics the batched BFS accumulated itself (preprocess.apsp_batched(..., pair_stats=True)):
-    same outputs as agg_bd_graph_fwd without a pass over the hop bytes (models.py:366-384)."""
-    lib = load()
-    T, S, pstat = _f32(T, "T"), _f32(S, "S"), _f32(pstat, "pstat")
-    if node_off.dtype != torch.int32 or pdepth.dtype != torch.int32:
-        raise TypeError("node_off / pdepth int32 expected")
-    B = node_off.numel() - 1
-    N, C = S.shape
-    nbins, Cr = T.shape
-    if pstat.numel() != N * nbins or pdepth.numel() != B:
-        raise ValueError(f"pair statistics must hold {N}*{nbins} floats and {B} depths, got {pstat.numel()} / {pdepth.numel()}")
-    out = torch.empty(B, C, dtype=torch.float32, device=S.device)
-    colw = torch.empty(N, Cr, dtype=torch.float32, device=S.device)
-    Q = torch.empty(B, nbins, C, dtype=torch.float32, device=S.device)
-    with _timed("aggregate_blockdiag_fwd"):
-        check(lib.gnan_aggregate_blockdiag_graph_fwd_pairs(ptr(pstat), ptr(pdepth.contiguous()), ptr(node_off), B, ptr(T), nbins, Cr, ptr(S), C,
-                                                           ptr(out), ptr(colw), ptr(Q), stream_handle()),
-              "gnan_aggregate_blockdiag_graph_fwd_pairs")
-    return out, colw, Q
-
-
-@agg_bd_graph_pairs_fwd.register_fake
-def _(pstat, pdepth, node_off, T, S):
-    B = node_off.numel() - 1
-    return S.new_empty(B, S.shape[1]), S.new_empty(S.shape[0], T.shape[1]), S.new_empty(B, T.shape[0], S.shape[1])
-
-
-def _bdgp_setup(ctx, inputs, output):
-    ctx.save_for_backward(inputs[2], output[1], output[2])
-
-
-def _bdgp_backward(ctx, g, _g_colw, _g_q):
-    node_off, colw, Q = ctx.saved_tensors
-    dS, dT = agg_bd_graph_bwd(node_off, g.contiguous(), colw, Q)
-    return None, None, None, dT, dS
-
-
-agg_bd_graph_pairs_fwd.register_autograd(_bdgp_backward, setup_context=_bdgp_setup)
-
-
-def aggregate_blockdiag_pairs(pstat, pdepth, node_off, T, S):
-    """[B,C] graph readout from pair statistics; raises for shapes the kernel does not cover (use the hop-byte path then)"""
-    if T.dim() != 2 or not load().gnan_aggregate_blockdiag_graph_supported(T.shape[0], T.shape[1], S.shape[1]):
-        raise NotImplementedError("pair statistics cover a global table with nbins <= 64 and C <= 4: build the batch with rscale=True instead")
-    return agg_bd_graph_pairs_fwd(pstat, pdepth, node_off, T, S)[0]
 
 
 def bfs_graph_readout_fwd(edges, node_off: Tensor, max_n: int, T: Tensor, S: Tensor, status: Tensor) -> Tuple[Tensor, Tensor, Tensor]:

@@ -249,18 +249,12 @@ class PackedBatch:
     hop_off int64 [B+1], level_counts int32 [sumN,nbins], batch_vector int64 [sumN] (kept for API parity), y.
     """
 
-    def __init__(self, x, hop, hop_off, node_off, level_counts, y=None, max_nodes=None, level_rscale=None, pair_stats=None,
-                 pair_depth=None):
+    def __init__(self, x, hop, hop_off, node_off, level_counts, y=None, max_nodes=None, level_rscale=None):
         self.x, self.hop, self.hop_off, self.node_off, self.level_counts, self.y = x, hop, hop_off, node_off, level_counts, y
         self.max_nodes = max_nodes
         # optional fp32 [sumN,nbins] 1/level_counts (0 for empty levels), written by the batched BFS itself
         # (apsp_batched(..., rscale=True)); level_counts may then be None
         self.level_rscale = level_rscale
-        # optional pair statistics P_b[d,j] = sum_{i: hop(i,j)=d} 1/level_counts[i,d], accumulated by the batched BFS
-        # (apsp_batched(..., pair_stats=True), undirected graphs): fp32 [sumN,nbins] storage holding graph b's LEVEL-MAJOR block
-        # [nbins][n_b] at row node_off[b] (rows 0..pair_depth[b] and the last one are defined), pair_depth int32 [B]. The
-        # output-normalised graph readout needs nothing else.
-        self.pair_stats, self.pair_depth = pair_stats, pair_depth
 
     deferred = False    # see _DeferredBatch
 
@@ -270,7 +264,7 @@ class PackedBatch:
 
     @property
     def nbins(self):
-        for t in (self.level_counts, self.level_rscale, self.pair_stats):
+        for t in (self.level_counts, self.level_rscale):
             if t is not None:
                 return t.shape[1]
         raise ValueError("PackedBatch without a level table")
@@ -283,12 +277,12 @@ class PackedBatch:
     def to(self, device):
         mv = lambda t: None if t is None else t.to(device, non_blocking=True)
         return PackedBatch(mv(self.x), mv(self.hop), mv(self.hop_off), mv(self.node_off), mv(self.level_counts), mv(self.y),
-                           self.max_nodes, mv(self.level_rscale), mv(self.pair_stats), mv(self.pair_depth))
+                           self.max_nodes, mv(self.level_rscale))
 
     def pin_memory(self):
         pm = lambda t: None if t is None else t.pin_memory()
         return PackedBatch(pm(self.x), pm(self.hop), pm(self.hop_off), pm(self.node_off), pm(self.level_counts), pm(self.y),
-                           self.max_nodes, pm(self.level_rscale), pm(self.pair_stats), pm(self.pair_depth))
+                           self.max_nodes, pm(self.level_rscale))
 
 
 class _DeferredBatch(PackedBatch):
@@ -406,8 +400,6 @@ def check_batched_status(status):
         raise ValueError("duplicate edges in the batch: call apsp_batched without nbins (multi-edge emulation path)")
     if over:
         raise ValueError("a hop distance does not fit the fixed-width level table: pass a larger nbins")
-    if st & 4:
-        raise ValueError("pair statistics were requested for a batch with a directed (non-symmetric) graph: use rscale=True")
 
 
 def apsp_batched(edge_index, node_off, device="cuda", x=None, y=None, node_off_device=None, _level_table_width=48, nbins=None,
@@ -426,16 +418,13 @@ def apsp_batched(edge_index, node_off, device="cuda", x=None, y=None, node_off_d
     rscale=True (fixed-width mode, graphs of at most 128 nodes): the BFS writes the output normaliser 1/level_counts
     (`PackedBatch.level_rscale`, fp32) INSTEAD of the int32 level counts, which the output-normalised models
     (models.TensorGNAN, normalize_rho=True) consume directly: one table written, none converted.
-    With a `LocalEdges` input (and pair_stats=False) the distances are DEFERRED: the call launches nothing and returns a batch
+    With a `LocalEdges` input the distances are DEFERRED: the call launches nothing and returns a batch
     that holds the edge segments (`deferred` is True). models.TensorGNAN's output-normalised graph readout then runs the BFS and
     the readout as one kernel (ops.bfs_graph_readout) and never materialises hop bytes or the normaliser table; the first read of
     `hop` or `level_rscale` runs this BFS once and caches both. `status` is the same device word either way, filled by the
     first kernel that consumes the edges (check it after the forward).
-
-    pair_stats=True (fixed-width mode, `LocalEdges` input, UNDIRECTED graphs of at most 128 nodes): the BFS
-    also accumulates the pair statistics of the output-normalised graph readout (`PackedBatch.pair_stats`; see PackedBatch), so
-    that models.TensorGNAN.forward_packed never reads the hop bytes or a normaliser table; status bit 4 = a graph was not
-    symmetric. Without rscale=True no level table is written at all.
+    pair_stats=True (`LocalEdges` input only) returns the same deferred batch as rscale=True: the pair statistics of the graph
+    readout are formed only inside the fused BFS + readout kernel.
 
     Pass node_off as a HOST tensor / array (what a data loader has): block sizes and offsets are then computed on the host
     and the call synchronises exactly once, at the end (overflow flag + largest hop, which sizes the level table).
@@ -472,11 +461,11 @@ def apsp_batched(edge_index, node_off, device="cuda", x=None, y=None, node_off_d
     if local is None:
         rowptr, col, _ = build_csr(edge_index, sumN, device, status=st[0:1])
 
-    def bfs(hop, cnt_t, rs_t, order_ws, ps_t=None, pd_t=None):
+    def bfs(hop, cnt_t, rs_t, order_ws):
         if local is not None:
             check(lib.gnan_apsp_bfs_batched_local(ptr(local.src), ptr(local.dst), ptr(local.edge_off), ptr(node_off_d), ptr(hop_off), B, max_n,
-                                                  ptr(hop), ptr(cnt_t), ptr(rs_t), ptr(ps_t), ptr(pd_t), nb, st.data_ptr(), st.data_ptr() + 4,
-                                                  st.data_ptr() + 8, ptr(order_ws), stream_handle()), "gnan_apsp_bfs_batched_local")
+                                                  ptr(hop), ptr(cnt_t), ptr(rs_t), nb, st.data_ptr(), st.data_ptr() + 4, st.data_ptr() + 8,
+                                                  ptr(order_ws), stream_handle()), "gnan_apsp_bfs_batched_local")
         else:
             check(lib.gnan_apsp_bfs_batched_ex(ptr(rowptr), ptr(col), ptr(node_off_d), ptr(hop_off), B, max_n, sumN, total, ptr(hop), ptr(cnt_t),
                                                ptr(rs_t), nb, st.data_ptr() + 4, st.data_ptr() + 8, ptr(order_ws), stream_handle()),
@@ -490,7 +479,7 @@ def apsp_batched(edge_index, node_off, device="cuda", x=None, y=None, node_off_d
     if rscale or pair_stats:
         if nbins is None or max_n > 128 or sumN == 0:
             raise ValueError("rscale=True needs the fixed-width mode (nbins=...) and graphs of at most 128 nodes")
-        if local is not None and not pair_stats:
+        if local is not None:
             def materialise():
                 hop = torch.empty(max(total, 1), dtype=torch.uint8, device=device)
                 rs = torch.empty(sumN, nb, dtype=torch.float32, device=device)
@@ -502,13 +491,11 @@ def apsp_batched(edge_index, node_off, device="cuda", x=None, y=None, node_off_d
             pk.status = st
             return pk
         hop = torch.empty(max(total, 1), dtype=torch.uint8, device=device)
-        rs = torch.empty(sumN, nb, dtype=torch.float32, device=device) if rscale else None
-        ps = torch.empty(sumN, nb, dtype=torch.float32, device=device) if pair_stats else None
-        pd = torch.empty(B, dtype=torch.int32, device=device) if pair_stats else None
+        rs = torch.empty(sumN, nb, dtype=torch.float32, device=device)
         order_ws = torch.empty(4 * B + 4, dtype=torch.int32, device=device)
         with _timed("apsp_bfs_batched"):
-            bfs(hop, None, rs, order_ws, ps, pd)
-        pk = PackedBatch(x, hop, hop_off, node_off_d, None, y, max_n, level_rscale=rs, pair_stats=ps, pair_depth=pd)
+            bfs(hop, None, rs, order_ws)
+        pk = PackedBatch(x, hop, hop_off, node_off_d, None, y, max_n, level_rscale=rs)
         pk.status = st
         return pk
     hop = torch.empty(max(total, 1), dtype=torch.uint8, device=device)

@@ -251,12 +251,6 @@ int gnan_aggregate_blockdiag_graph_fwd(const uint8_t *hop, const int64_t *hop_of
                                        const float *T /* [nbins,Cr] */, int32_t nbins, int32_t Cr,
                                        const float *rscale /* [sumN,nbins] or NULL */, const float *S, int32_t C,
                                        float *out /* [B,C] */, float *colw, float *Q, int32_t *work_counter, gnan_stream_t stream);
-/* The same forward from the pair statistics (pstat, pdepth) that gnan_apsp_bfs_batched_local accumulated inside the BFS
- * (output-normalised readout of undirected graphs): no pass over the hop bytes at all; same out / colw / Q, same backward. */
-int gnan_aggregate_blockdiag_graph_fwd_pairs(const float *pstat, const int32_t *pdepth, const int32_t *node_off, int32_t B,
-                                             const float *T, int32_t nbins,
-                                             int32_t Cr, const float *S, int32_t C, float *out, float *colw, float *Q,
-                                             gnan_stream_t stream);
 size_t gnan_aggregate_blockdiag_graph_bwd_workspace_bytes(int32_t nbins, int32_t C);
 int gnan_aggregate_blockdiag_graph_bwd(const int32_t *node_off, int32_t B, int32_t nbins, int32_t Cr, int32_t C,
                                        const float *g /* [B,C] */, const float *colw, const float *Q, float *dS, float *dT,
@@ -329,40 +323,29 @@ int gnan_apsp_bfs_batched(const int32_t *rowptr /* [sumN+1] */, const int32_t *c
                           int32_t nbins, int32_t *overflow_flag, gnan_stream_t stream);
 
 /* same with host-side size hints: max_n = the largest graph (sizes shared memory; graphs of up to 256 nodes); total_nodes =
- * node_off[B] and total_hop_bytes = hop_off[B] (both > 0: the unreachable / zero background of hop and cnt is written by two
- * memsets at HBM speed instead of per-source store loops; 0 = unknown); max_level (optional, zero-initialised by the caller)
- * receives the largest finite hop of the batch (atomicMax), which sizes the trimmed level table */
-int gnan_apsp_bfs_batched_n(const int32_t *rowptr, const int32_t *col, const int32_t *node_off, const int64_t *hop_off,
-                            int32_t B, int32_t max_n, int64_t total_nodes, int64_t total_hop_bytes, uint8_t *hop, int32_t *cnt,
-                            int32_t nbins, int32_t *overflow_flag, int32_t *max_level, gnan_stream_t stream);
-
-/* same, with an optional fused normaliser output: rscale [sumN,nbins] fp32 = 1/count (0 for an empty level), i.e. what
- * gnan_level_rscale computes from cnt (models.py:368-370 divides by the level size); cnt may then be NULL. Needs the totals
- * and graphs of at most 128 nodes. */
+ * node_off[B] and total_hop_bytes = hop_off[B] (0 = unknown); max_level (optional, zero-initialised by the caller) receives the
+ * largest finite hop of the batch (atomicMax), which sizes the trimmed level table. order_ws [4*B+4] is required scratch.
+ * Graphs of at most 128 nodes with the totals known are grouped by size class, and a GROUP OF 4 WARPS works on one graph of
+ * 65..128 nodes, two of 33..64 or four of up to 32 nodes at a time (one vertex per lane, a named barrier with an OR reduction per
+ * BFS level). Otherwise one lane per source (graphs of up to 256 nodes); with both totals > 0 the unreachable / zero background
+ * of hop and cnt is then written by two memsets at HBM speed instead of per-source store loops.
+ * rscale (optional) [sumN,nbins] fp32 = 1/count (0 for an empty level), i.e. what gnan_level_rscale computes from cnt
+ * (models.py:368-370 divides by the level size); cnt may then be NULL. Needs the totals and graphs of at most 128 nodes. */
 int gnan_apsp_bfs_batched_ex(const int32_t *rowptr, const int32_t *col, const int32_t *node_off, const int64_t *hop_off,
                              int32_t B, int32_t max_n, int64_t total_nodes, int64_t total_hop_bytes, uint8_t *hop, int32_t *cnt,
                              float *rscale, int32_t nbins, int32_t *overflow_flag, int32_t *max_level,
-                             int32_t *order_ws /* [4*B+4] scratch or NULL, see below */, gnan_stream_t stream);
-/* order_ws: with it the graphs are grouped by size class and a GROUP OF 4 WARPS works on one graph of 65..128 nodes, two of 33..64
- * or four of up to 32 nodes at a time (one vertex per lane, a named barrier with an OR reduction per BFS level); NULL = the
- * older kernel, one warp per graph. */
+                             int32_t *order_ws /* [4*B+4] scratch */, gnan_stream_t stream);
 
 /* gnan_apsp_bfs_batched_ex WITHOUT a CSR: the batch's edges in their transfer form (gnan_edges_from_local: src / dst uint8 indices
  * inside the graph, edge_off [B+1], edges grouped by graph). Every 4-warp group builds its graph's adjacency bit matrix in shared
  * memory from the graph's own edge segment; gnan_build_csr (and its ~0.1 ms per 4 M edges) drops out of a training step that
  * preprocesses its batch. Graphs of at most 128 nodes; order_ws [4*B+4] is required. *status (device int32, zeroed here) gets
  * gnan_build_csr's bits: 1 = an endpoint >= the graph's node count (edge dropped), 2 = a repeated (src,dst) pair (the reference
- * sums those into weight-2 edges: the caller must take the multi-edge path). pre_process_datasets.py:106-122 per graph.
- * pstat + pdepth (optional, UNDIRECTED graphs): the pair statistics of the output-normalised graph readout,
- * P_b[d,j] = sum_{i: hop(i,j) = d} 1/cnt[i,d], accumulated inside the BFS level loop. pstat: sumN*nbins floats, graph b's block at
- * node_off[b]*nbins, LEVEL-MAJOR [nbins][n_b]: rows 0..pdepth[b] (the graph's deepest level) and row nbins-1 (the unreachable bin)
- * are written, the rows in between are left untouched and must not be read; pdepth: int32 [B].
- * gnan_aggregate_blockdiag_graph_fwd_pairs consumes them instead of the hop bytes + the normaliser table. A graph whose edge
- * list is not symmetric sets status bit 4 (its block of pstat is then meaningless). */
+ * sums those into weight-2 edges: the caller must take the multi-edge path). pre_process_datasets.py:106-122 per graph. */
 int gnan_apsp_bfs_batched_local(const uint8_t *src, const uint8_t *dst, const int32_t *edge_off, const int32_t *node_off,
                                 const int64_t *hop_off, int32_t B, int32_t max_n, uint8_t *hop, int32_t *cnt, float *rscale,
-                                float *pstat, int32_t *pdepth, int32_t nbins, int32_t *status, int32_t *overflow_flag,
-                                int32_t *max_level, int32_t *order_ws, gnan_stream_t stream);
+                                int32_t nbins, int32_t *status, int32_t *overflow_flag, int32_t *max_level, int32_t *order_ws,
+                                gnan_stream_t stream);
 
 /* gnan_apsp_bfs_batched_local fused with gnan_aggregate_blockdiag_graph_fwd on the output-normaliser table (models.py:366-384 with
  * normalize_rho, a global table T [nbins,Cr]): the same out [B,C], colw [sumN,Cr] and Q [B,nbins,C] (gnan_aggregate_blockdiag_graph_bwd

@@ -48,6 +48,10 @@ def test_argument_validation_without_gpu(lib_path):
     assert rc == 1 and b"wo" in lib.gnan_last_error()
     rc = lib.gnan_aggregate_rows_fwd(None, 4, 4, 16, None, 0, 5, 1, None, None, 1, None, None)
     assert rc == 1
+    arr = (ctypes.c_int64 * 8)()
+    buf = ctypes.addressof(arr)
+    rc =lib.gnan_apsp_bfs_batched_ex(buf, buf, buf, buf, 1, 4, 4, 16, buf, None, None, 0, buf, None, None, None)   # order_ws NULL
+    assert rc == 1 and b"order_ws" in lib.gnan_last_error()
     assert lib.gnan_mlp_workspace_bytes(0, ctypes.byref(p), 0, 0) == 0
 
 

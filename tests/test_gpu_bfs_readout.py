@@ -37,20 +37,30 @@ def _fused_vs_materialised(directed, C, rho_per_feature, seed):
     sizes = SIZES + [int(v) for v in rng.integers(1, 129, size=120)]
     ei, node_off = _edges(rng, sizes, directed)
     x = torch.tensor(rng.normal(size=(node_off[-1], 5))).float().to(DEV)
-    pk = apsp_batched(LocalEdges.from_edge_index(ei, node_off), node_off, device=DEV, x=x, nbins=48, rscale=True)
-    assert pk.deferred and pk.nbins == 48
+    le = LocalEdges.from_edge_index(ei, node_off)
+    pk = apsp_batched(le, node_off, device=DEV, x=x, nbins=48, rscale=True)
+    alias = apsp_batched(le, node_off, device=DEV, x=x, nbins=48, pair_stats=True)     # the same deferred batch
+    assert pk.deferred and alias.deferred and pk.nbins == alias.nbins == 48
     m = _model(5, C, rho_per_feature)
     w = torch.tensor(rng.normal(size=(len(sizes), C))).float().to(DEV)
-    res = []
-    for _ in range(2):                               # fused (distances never materialised), then the hop-byte path on the same batch
+
+    def step(batch):
         m.zero_grad(set_to_none=True)
-        out = m(pk)
+        out = m(batch)
         (out * w).sum().backward()
-        res.append((out.detach().clone(), [p.grad.clone() for p in m.parameters() if p.grad is not None]))
-        if pk.deferred:
-            check_batched_status(pk.status)
-            pk.hop                                   # materialise: the next forward reads the hop bytes + normaliser table
-            assert not pk.deferred and pk.level_rscale is not None
+        return out.detach().clone(), [p.grad.clone() for p in m.parameters() if p.grad is not None]
+
+    res = [step(pk)]                                 # fused (distances never materialised)
+    via_alias = step(alias)
+    for b in (pk, alias):
+        assert b.deferred
+        check_batched_status(b.status)
+    assert torch.equal(via_alias[0], res[0][0]) and len(via_alias[1]) == len(res[0][1])
+    for a, b in zip(via_alias[1], res[0][1]):
+        assert G.rel_err(a.cpu().numpy(), b.cpu().numpy()) < TOL
+    pk.hop                                           # materialise: the next forward reads the hop bytes + normaliser table
+    assert not pk.deferred and pk.level_rscale is not None
+    res.append(step(pk))                             # the hop-byte path on the same batch
     assert len(res[0][1]) == len(res[1][1]) > 0
     assert G.rel_err(res[0][0].cpu().numpy(), res[1][0].cpu().numpy()) < TOL
     for a, b in zip(res[0][1], res[1][1]):

@@ -144,79 +144,6 @@ def test_molecule_step_with_fused_normaliser_matches_the_counts_path():
         assert float((a - b).norm()) <= 1e-6 * float(b.norm()) + 1e-12
 
 
-def test_batched_bfs_pair_statistics_vs_float64():
-    """apsp_batched(LocalEdges, pair_stats=True): P_b[d,j] = sum_{i: hop(i,j)=d} 1/count(i,d) accumulated inside the BFS level loop
-    (undirected graphs; level-major block per graph, unreachable pairs in the last row, the graph's deepest level in pair_depth)
-    against a float64 evaluation from the hop blocks and level counts."""
-    from gnan_b200.preprocess import LocalEdges, apsp_batched, check_batched_status
-    rng = np.random.default_rng(21)
-    sizes = [int(v) for v in rng.integers(1, 129, size=150)] + [128, 97, 65, 64, 33, 32, 1, 2]
-    node_off = np.concatenate([[0], np.cumsum(sizes)])
-    eis = [random_graph(rng, n, 2.0 if i % 3 else 1.2, False, n_isolated=2 if n > 8 and i % 2 else 0) for i, n in enumerate(sizes)]
-    ei = torch.tensor(np.concatenate([e + node_off[i] for i, e in enumerate(eis)], axis=1))
-    le = LocalEdges.from_edge_index(ei, node_off)
-    nb = 132
-    ref = apsp_batched(ei, node_off, device=DEV, nbins=nb)
-    pk = apsp_batched(le, node_off, device=DEV, nbins=nb, pair_stats=True)
-    both = apsp_batched(le, node_off, device=DEV, nbins=nb, pair_stats=True, rscale=True)
-    check_batched_status(pk.status); check_batched_status(both.status)
-    assert pk.level_counts is None and pk.level_rscale is None and pk.nbins == nb
-    assert torch.equal(pk.hop, ref.hop) and torch.equal(both.pair_depth, pk.pair_depth) and torch.equal(both.level_rscale, apsp_batched(
-        ei, node_off, device=DEV, nbins=nb, rscale=True).level_rscale)
-    hop, cnt, ho = ref.hop.cpu().numpy(), ref.level_counts.cpu().numpy().astype(np.float64), ref.hop_off.cpu().numpy()
-    P, depth = pk.pair_stats.cpu().numpy().reshape(-1), pk.pair_depth.cpu().numpy()
-    for b, n in enumerate(sizes):
-        h = hop[ho[b]:ho[b + 1]].reshape(n, n).astype(np.int64)
-        d = np.minimum(h, nb - 1)
-        c = cnt[node_off[b]:node_off[b + 1]]
-        r = np.where(c > 0, 1.0 / np.maximum(c, 1), 0.0)
-        want = np.zeros((n, nb))
-        ii, jj = np.meshgrid(np.arange(n), np.arange(n), indexing="ij")
-        np.add.at(want, (jj.ravel(), d.ravel()), r[ii.ravel(), d.ravel()])
-        got = P[node_off[b] * nb:node_off[b + 1] * nb].reshape(nb, n)        # the graph's level-major block
-        finite = h[h < 255]
-        assert depth[b] == (int(finite.max()) if finite.size else 0), b
-        rows = list(range(depth[b] + 1)) + [nb - 1]                          # the rows in between are not written
-        assert np.abs(got[rows] - want.T[rows]).max() <= 2e-6 * max(1.0, np.abs(want).max()), b
-        assert np.abs(want.T[depth[b] + 1:nb - 1]).max(initial=0.0) == 0.0
-    directed = [random_graph(rng, n, 2.0, True) for n in sizes[:20]]
-    no2 = np.concatenate([[0], np.cumsum(sizes[:20])])
-    eid = torch.tensor(np.concatenate([e + no2[i] for i, e in enumerate(directed)], axis=1))
-    bad = apsp_batched(LocalEdges.from_edge_index(eid, no2), no2, device=DEV, nbins=nb, pair_stats=True)
-    assert int(bad.status[0]) & 4
-    with pytest.raises(ValueError):
-        check_batched_status(bad.status)
-
-
-@pytest.mark.parametrize("C", [1, 3, 4])
-def test_graph_readout_from_pair_statistics_matches_the_hop_byte_path(C):
-    """models.TensorGNAN on a batch that carries pair statistics only == the same model on the batch with hop bytes + normaliser
-    (outputs and every parameter gradient; the two forwards sum in different orders: 2e-6)."""
-    from gnan_b200.models import TensorGNAN
-    from gnan_b200.preprocess import LocalEdges, apsp_batched
-    rng = np.random.default_rng(C * 7)
-    sizes = [int(v) for v in rng.integers(5, 101, size=80)]
-    node_off = np.concatenate([[0], np.cumsum(sizes)])
-    eis = [random_graph(rng, n, 2.2, False, n_isolated=1 if i % 4 == 0 else 0) for i, n in enumerate(sizes)]
-    ei = torch.tensor(np.concatenate([e + node_off[i] for i, e in enumerate(eis)], axis=1))
-    le = LocalEdges.from_edge_index(ei, node_off)
-    x = torch.tensor(rng.normal(size=(node_off[-1], 5))).float().to(DEV)
-    torch.manual_seed(0)
-    m = TensorGNAN(5, C, 3, 64, normalize_rho=True, is_graph_task=True, readout_n_layers=0, device=DEV).to(DEV)
-    m.fs.xavier_normal_(1.0); m.rho.xavier_normal_(1.0)
-    w = torch.tensor(rng.normal(size=(len(sizes), C))).float().to(DEV)
-    res = []
-    for kw in (dict(rscale=True), dict(pair_stats=True)):
-        pk = apsp_batched(le, node_off, device=DEV, x=x, nbins=48, **kw)
-        m.zero_grad(set_to_none=True)
-        out = m(pk)
-        (out.reshape(len(sizes), -1) * w[:, :out.reshape(len(sizes), -1).shape[1]]).sum().backward()
-        res.append((out.detach().clone(), [p.grad.clone() for p in m.parameters() if p.grad is not None]))
-    assert float((res[0][0] - res[1][0]).norm()) <= 2e-6 * float(res[0][0].norm())
-    for a, b in zip(res[0][1], res[1][1]):
-        assert float((a - b).norm()) <= 2e-6 * float(b.norm()) + 1e-12
-
-
 def test_gather_segment_sum_few_long_segments():
     """the block-per-segment variant (a handful of segments with ~1e5 rows each: one-hot columns) against float64"""
     from gnan_b200 import ops
