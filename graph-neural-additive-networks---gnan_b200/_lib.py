@@ -13,6 +13,7 @@ c_void_p, c_int, c_int32, c_int64, c_size_t, c_float, c_uint64 = (
 PREC_FP32, PREC_TF32X3, PREC_TF32 = 0, 1, 2
 PRECISIONS = {"fp32": PREC_FP32, "tf32x3": PREC_TF32X3, "tf32": PREC_TF32}
 HOP_UNREACHABLE = 255
+APSP_BATCHED_MAX_NODES = 1024    # GNAN_APSP_BATCHED_MAX_NODES: largest graph of the batched BFS (gnan_apsp_bfs_batched_ex)
 AGG_AUTO, AGG_CUDA_CORES, AGG_TENSOR_CORES = 0, 1, 2
 AGG_ALGOS = {"auto": AGG_AUTO, "cuda": AGG_CUDA_CORES, "tc": AGG_TENSOR_CORES}
 

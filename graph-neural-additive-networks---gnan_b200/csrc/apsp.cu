@@ -323,20 +323,32 @@ __device__ __forceinline__ int bv3_graph(const int32_t *__restrict__ rowptr, con
 
 // graphs by word-count class (0 = 97..128 nodes ... 3 = up to 32), one thread per graph, warp-aggregated counters:
 // cls[0..4) = class sizes (zeroed by the caller), cls[4 + c * B ...) = the graphs of class c in arbitrary order.
+// LARGE (batches with graphs of more than 128 nodes, order_ws [5 * B + 5]; the first 4 * B + 4 words keep their layout): class 4 =
+// more than 128 nodes (apsp_batched_large_kernel), its size at cls[4 * B + 4] (zeroed by the caller), its graphs from cls[4 * B + 5] on.
 // The v3 kernel walks the classes largest first: the expensive graphs start first, and the groups of a CTA run the same
 // instantiation of bv3_graph side by side (the instantiations do not fit the instruction cache together).
+template <bool LARGE>
 __global__ void bv3_classify_kernel(const int32_t *__restrict__ node_off, int B, int32_t *__restrict__ cls)
 {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     const bool ok = b < B;
-    int c = 4;
-    if (ok) c = 3 - min(3, max(0, (node_off[b + 1] - node_off[b] - 1) >> 5));
+    int c = LARGE ? 5 : 4;                                                // (no graph: a value of no class)
+    if (ok) {
+        const int n = node_off[b + 1] - node_off[b];
+        c = LARGE && n > 32 * BV3_MAX_W ? 4 : 3 - min(3, max(0, (n - 1) >> 5));
+    }
     const uint32_t peers = __match_any_sync(0xffffffffu, c);
     const int lane = threadIdx.x & 31, leader = __ffs(peers) - 1;
     int base = 0;
-    if (ok && lane == leader) base = atomicAdd(cls + c, __popc(peers));
-    base = __shfl_sync(0xffffffffu, base, leader);
-    if (ok) cls[4 + (size_t)c * B + base + __popc(peers & ((1u << lane) - 1))] = b;
+    if constexpr (LARGE) {
+        if (ok && lane == leader) base = atomicAdd(cls + (c < 4 ? c : 4 + 4 * B), __popc(peers));
+        base = __shfl_sync(0xffffffffu, base, leader);
+        if (ok) cls[4 + (size_t)c * B + (c >> 2) + base + __popc(peers & ((1u << lane) - 1))] = b;   // class 4: after its size word
+    } else {
+        if (ok && lane == leader) base = atomicAdd(cls + c, __popc(peers));
+        base = __shfl_sync(0xffffffffu, base, leader);
+        if (ok) cls[4 + (size_t)c * B + base + __popc(peers & ((1u << lane) - 1))] = b;
+    }
 }
 
 struct Bv3Out {
@@ -703,6 +715,118 @@ apsp_batched_v3_kernel(const int32_t *__restrict__ rowptr, const int32_t *__rest
     }
 }
 
+// ---- batched graphs of 129..GNAN_APSP_BATCHED_MAX_NODES nodes: one CTA per graph, bit-parallel over 128 sources at a time -------
+// The v3 pull on a whole CTA: thread t owns vertices t and t + BL_THREADS and keeps, per vertex, the bits of the chunk's sources
+// s0..s0+127 that reach it (BL_W words). Level L: new[v] = (OR_{u in out(v)} frontier[u]) & ~visited[v]; a new bit s means
+// hop[v][s0+s] = L and popc(new[v]) adds to row v's level-L count. A thread owns rows v of hop and cnt: no atomics. One
+// __syncthreads_or per level ends the level loop of a chunk. The CTA first writes its graph's 255 / 0 background (coalesced
+// 16-byte stores), then scatters the reached bytes and adds each chunk's counts into the rows. Neighbours come from the CSR.
+constexpr int BL_THREADS = 512;
+constexpr int BL_VPT = GNAN_APSP_BATCHED_MAX_NODES / BL_THREADS;   // vertices per thread
+constexpr int BL_W = 4;                                              // source words per vertex: 128 sources per chunk
+
+__global__ void __launch_bounds__(BL_THREADS, 2)
+apsp_batched_large_kernel(const int32_t *__restrict__ rowptr, const int32_t *__restrict__ col, const int32_t *__restrict__ node_off,
+                          const int64_t *__restrict__ hop_off, int B, uint8_t *__restrict__ hop, int32_t *__restrict__ cnt, int nbins,
+                          int32_t *__restrict__ overflow, int32_t *__restrict__ max_level, const int32_t *__restrict__ order)
+{
+    __shared__ __align__(16) uint32_t fr[2][GNAN_APSP_BATCHED_MAX_NODES * BL_W];   // frontier rows [n][BL_W], by level parity
+    const int tid = threadIdx.x;
+    const int n_large = order[4 + 4 * (size_t)B];
+    const int32_t *list = order + 5 + 4 * (size_t)B;
+    int lvl_max = 0;
+    for (int t = blockIdx.x; t < n_large; t += gridDim.x) {
+        const int64_t b = list[t];
+        const int n0 = node_off[b], n = node_off[b + 1] - n0;
+        uint8_t *gb = hop + hop_off[b];
+        int32_t *gc = cnt ? cnt + (int64_t)n0 * nbins : nullptr;
+        // background: head bytes up to the first 16-byte boundary, vector body, tail bytes
+        const int total = n * n;
+        const int head = min(total, (int)((16 - (reinterpret_cast<uintptr_t>(gb) & 15)) & 15));
+        if (tid < head) gb[tid] = GNAN_HOP_UNREACHABLE;
+        const int body = (total - head) / 16;
+        for (int i = tid; i < body; i += BL_THREADS)
+            *reinterpret_cast<uint4 *>(gb + head + (size_t)i * 16) = make_uint4(0xffffffffu, 0xffffffffu, 0xffffffffu, 0xffffffffu);
+        const int tail0 = head + body * 16;
+        if (tid < 16 && tail0 + tid < total) gb[tail0 + tid] = GNAN_HOP_UNREACHABLE;
+        if (gc)
+            for (int i = tid; i < n * nbins; i += BL_THREADS) gc[i] = 0;
+        __syncthreads();
+        int reached[BL_VPT];
+#pragma unroll
+        for (int k = 0; k < BL_VPT; ++k) {
+            const int v = tid + k * BL_THREADS;
+            reached[k] = 1;
+            if (v < n) {
+                gb[(size_t)v * n + v] = 0;
+                if (gc) gc[(int64_t)v * nbins] = 1;
+            }
+        }
+        for (int s0 = 0; s0 < n; s0 += 32 * BL_W) {
+            uint32_t vis[BL_VPT][BL_W];
+#pragma unroll
+            for (int k = 0; k < BL_VPT; ++k) {
+                const int v = tid + k * BL_THREADS, rel = v - s0;
+#pragma unroll
+                for (int ww = 0; ww < BL_W; ++ww) vis[k][ww] = (rel >= 0 && (rel >> 5) == ww) ? 1u << (rel & 31) : 0u;
+                if (v < n) bv3_store_row<BL_W>(fr[0] + v * BL_W, vis[k]);
+            }
+            __syncthreads();
+            for (int level = 1; level <= n; ++level) {
+                const uint32_t *fc = fr[(level - 1) & 1];
+                uint32_t *fn = fr[level & 1];
+                const uint8_t lv = (uint8_t)min(level, 254);
+                bool any = false;
+#pragma unroll
+                for (int k = 0; k < BL_VPT; ++k) {
+                    const int v = tid + k * BL_THREADS;
+                    if (v < n) {
+                        uint32_t acc[BL_W] = {0u, 0u, 0u, 0u};
+                        const int e1 = rowptr[n0 + v + 1];
+                        for (int e = rowptr[n0 + v]; e < e1; ++e) {          // neighbours outside the graph are ignored
+                            const int u = __ldg(col + e) - n0;
+                            if (u >= 0 && u < n) bv3_or_row<BL_W>(fc + u * BL_W, acc);
+                        }
+                        int newc = 0;
+#pragma unroll
+                        for (int ww = 0; ww < BL_W; ++ww) {
+                            acc[ww] &= ~vis[k][ww];
+                            vis[k][ww] |= acc[ww];
+                            newc += __popc(acc[ww]);
+                        }
+                        bv3_store_row<BL_W>(fn + v * BL_W, acc);
+                        if (newc) {
+                            any = true;
+                            uint8_t *rowp = gb + (size_t)v * n + s0;
+#pragma unroll
+                            for (int ww = 0; ww < BL_W; ++ww) {
+                                uint32_t m = acc[ww];
+                                while (m) {
+                                    rowp[ww * 32 + __ffs(m) - 1] = lv;
+                                    m &= m - 1;
+                                }
+                            }
+                            if (level > 254 || level >= nbins - 1) atomicExch(overflow, 1);
+                            else if (gc) gc[(int64_t)v * nbins + level] += newc;
+                            reached[k] += newc;
+                        }
+                    }
+                }
+                if (!__syncthreads_or(any)) break;
+                lvl_max = max(lvl_max, level);
+            }
+        }
+        if (gc) {
+#pragma unroll
+            for (int k = 0; k < BL_VPT; ++k) {
+                const int v = tid + k * BL_THREADS;
+                if (v < n) gc[(int64_t)v * nbins + nbins - 1] = n - reached[k];
+            }
+        }
+    }
+    if (max_level && tid == 0 && lvl_max > 0) atomicMax(max_level, lvl_max);   // lvl_max is uniform over the CTA
+}
+
 // ---- one large graph: one warp per source, queue + bitmap in the workspace -----------------------------------------
 __global__ void __launch_bounds__(256)
 apsp_bfs_kernel(const int32_t *__restrict__ rowptr, const int32_t *__restrict__ col, int N, int src_begin, int src_end,
@@ -999,10 +1123,11 @@ extern "C" int gnan_apsp_msbfs(const int32_t *rowptr, const int32_t *col, int32_
 
 // v3 launch: groups of 4 warps; the group's slice holds one graph of 65..128 nodes, two of 33..64 or four of up to 32
 // CC > 0: the BFS fused with the graph readout (bv3_readout_run; ro holds its tensors, hop / cnt / rscale are NULL)
+// large: the batch also has graphs of more than 128 nodes (order_ws [5*B+5]; max_n = 128 sizes the slices of the others)
 template <bool LOCAL, int CC = 0>
 static int launch_bv3(const int32_t *rowptr, const int32_t *col, const int32_t *node_off, const int64_t *hop_off, int32_t B, int32_t max_n,
                       uint8_t *hop, int32_t *cnt, float *rscale, int nb, bool levels, int32_t *overflow_flag, int32_t *max_level,
-                      int32_t *order_ws, Bv3Edges le, cudaStream_t st, Bv3Readout ro = Bv3Readout{})
+                      int32_t *order_ws, Bv3Edges le, cudaStream_t st, Bv3Readout ro = Bv3Readout{}, bool large = false)
 {
     const int Wmax = (max_n + 31) / 32;
     auto need = [&](int cap, int W, int G) {
@@ -1024,7 +1149,12 @@ static int launch_bv3(const int32_t *rowptr, const int32_t *col, const int32_t *
     }
     const int blocks3 = (int)std::min<int64_t>(ceil_div64(B, gpc), (int64_t)std::max(cached_per_sm3, 1) * gnan_sm_count());
     GNAN_CUDA(cudaMemsetAsync(order_ws, 0, 4 * sizeof(int32_t), st));
-    bv3_classify_kernel<<<(unsigned)ceil_div64(B, 256), 256, 0, st>>>(node_off, B, order_ws);
+    if (large) {
+        GNAN_CUDA(cudaMemsetAsync(order_ws + 4 * (size_t)B + 4, 0, sizeof(int32_t), st));
+        bv3_classify_kernel<true><<<(unsigned)ceil_div64(B, 256), 256, 0, st>>>(node_off, B, order_ws);
+    } else {
+        bv3_classify_kernel<false><<<(unsigned)ceil_div64(B, 256), 256, 0, st>>>(node_off, B, order_ws);
+    }
     GNAN_LAUNCH_OK();
     kernel<<<blocks3, 32 * BV3_GW * gpc, smem3, st>>>(rowptr, col, node_off, hop_off, B, max_n, gpc, (int)slice, hop, cnt, rscale, nb,
                                                       overflow_flag, max_level, order_ws, le, ro);
@@ -1052,7 +1182,23 @@ static int launch_batched_lanes(const int32_t *rowptr, const int32_t *col, const
     return GNAN_OK;
 }
 
-// graphs of at most 128 nodes with known totals: v3; anything else: the lane-per-source kernel.
+// graphs of more than 128 nodes in the batch: class 4 of bv3_classify_kernel (the caller has run it into order_ws [5*B+5]).
+// B bounds the number of such graphs; CTAs past the end of the class exit at once.
+static int launch_batched_large(const int32_t *rowptr, const int32_t *col, const int32_t *node_off, const int64_t *hop_off, int32_t B,
+                                uint8_t *hop, int32_t *cnt, int nb, int32_t *overflow_flag, int32_t *max_level, const int32_t *order_ws,
+                                cudaStream_t st)
+{
+    static thread_local int per_sm = 0;
+    if (per_sm == 0) GNAN_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, apsp_batched_large_kernel, BL_THREADS, 0));
+    const int blocks = (int)std::min<int64_t>(B, (int64_t)std::max(per_sm, 1) * gnan_sm_count());
+    apsp_batched_large_kernel<<<blocks, BL_THREADS, 0, st>>>(rowptr, col, node_off, hop_off, B, hop, cnt, nb, overflow_flag, max_level,
+                                                             order_ws);
+    GNAN_LAUNCH_OK();
+    return GNAN_OK;
+}
+
+// graphs of at most 128 nodes with known totals: v3; at most 256 nodes otherwise: the lane-per-source kernel; larger graphs (up to
+// GNAN_APSP_BATCHED_MAX_NODES, totals known): v3 for the graphs of at most 128 nodes and apsp_batched_large_kernel for the others.
 // rscale (optional): 1/count per (node, level) as fp32, what gnan_level_rscale would compute from cnt; cnt may then be NULL
 extern "C" int gnan_apsp_bfs_batched_ex(const int32_t *rowptr, const int32_t *col, const int32_t *node_off, const int64_t *hop_off,
                                         int32_t B, int32_t max_n, int64_t total_nodes, int64_t total_hop_bytes, uint8_t *hop,
@@ -1068,8 +1214,14 @@ extern "C" int gnan_apsp_bfs_batched_ex(const int32_t *rowptr, const int32_t *co
         gnan_set_error("apsp_bfs_batched: the fused 1/count output needs graphs of at most %d nodes and the totals", 32 * BV3_MAX_W);
         return GNAN_ERR_UNSUPPORTED;
     }
-    if (max_n < 1 || max_n > 32 * BW_MAX) {
-        gnan_set_error("apsp_bfs_batched: graphs with %d nodes unsupported (1..%d); use gnan_apsp_bfs", max_n, 32 * BW_MAX);
+    if (max_n < 1 || max_n > GNAN_APSP_BATCHED_MAX_NODES) {
+        gnan_set_error("apsp_bfs_batched: graphs with %d nodes unsupported (1..%d = GNAN_APSP_BATCHED_MAX_NODES); use gnan_apsp_bfs",
+                       max_n, GNAN_APSP_BATCHED_MAX_NODES);
+        return GNAN_ERR_UNSUPPORTED;
+    }
+    if (max_n > 32 * BW_MAX && total_nodes <= 0) {
+        gnan_set_error("apsp_bfs_batched: graphs of %d..%d (GNAN_APSP_BATCHED_MAX_NODES) nodes need the totals (total_nodes > 0)",
+                       32 * BW_MAX + 1, GNAN_APSP_BATCHED_MAX_NODES);
         return GNAN_ERR_UNSUPPORTED;
     }
     cudaStream_t st = (cudaStream_t)stream;
@@ -1079,6 +1231,17 @@ extern "C" int gnan_apsp_bfs_batched_ex(const int32_t *rowptr, const int32_t *co
                                          overflow_flag, max_level, order_ws, Bv3Edges{}, st);
         if (rc == GNAN_ERR_UNSUPPORTED) gnan_set_error("apsp_bfs_batched: level table too wide for the shared-memory slice");
         return rc;
+    }
+    if (max_n > 32 * BW_MAX) {
+        const int nb = cnt ? nbins : 256;
+        const int rc = launch_bv3<false>(rowptr, col, node_off, hop_off, B, 32 * BV3_MAX_W, hop, cnt, nullptr, nb, cnt != nullptr,
+                                         overflow_flag, max_level, order_ws, Bv3Edges{}, st, Bv3Readout{}, true);
+        if (rc == GNAN_ERR_UNSUPPORTED) {
+            gnan_set_error("apsp_bfs_batched: level table too wide for the shared-memory slice");
+            return rc;
+        }
+        if (rc != GNAN_OK) return rc;
+        return launch_batched_large(rowptr, col, node_off, hop_off, B, hop, cnt, nb, overflow_flag, max_level, order_ws, st);
     }
     return launch_batched_lanes(rowptr, col, node_off, hop_off, B, max_n, total_nodes, total_hop_bytes, hop, cnt, nbins, overflow_flag,
                                 max_level, st);

@@ -79,7 +79,9 @@ class PackedDataset:
     @classmethod
     def from_graphs(cls, graphs: Sequence, device="cuda", add_constant_column=True):
         """Graphs with `.x [n,K]`, `.edge_index [2,E]` (local ids) and optionally `.y`: ONE batched GPU BFS for the whole
-        dataset (pre_process_datasets.py:106-122 without the per-graph Python loop). Graphs of at most 256 nodes."""
+        dataset (pre_process_datasets.py:106-122 without the per-graph Python loop) for graphs of up to
+        preprocess._lib.APSP_BATCHED_MAX_NODES (1024) nodes, which covers the TU graph-classification sets (Mutagenicity, PROTEINS).
+        A dataset with a larger graph, or with duplicate edges, is preprocessed graph by graph instead (same result, slower)."""
         sizes = torch.tensor([int(g.x.shape[0]) for g in graphs], dtype=torch.int64)
         node_off = torch.zeros(len(graphs) + 1, dtype=torch.int64)
         node_off[1:] = torch.cumsum(sizes, 0)

@@ -404,8 +404,11 @@ def check_batched_status(status):
 
 def apsp_batched(edge_index, node_off, device="cuda", x=None, y=None, node_off_device=None, _level_table_width=48, nbins=None,
                  hop_off_device=None, rscale=False, pair_stats=False):
-    """Hop blocks of B small graphs (<= 256 nodes each) in one launch. edge_index uses GLOBAL node ids of the
-    concatenated node set; node_off [B+1] are the graph boundaries. edge_index may also be a `LocalEdges` (the batch's edge list
+    """Hop blocks of B graphs in one launch. edge_index uses GLOBAL node ids of the
+    concatenated node set; node_off [B+1] are the graph boundaries. Graphs of up to _lib.APSP_BATCHED_MAX_NODES (1024) nodes run
+    in the batched BFS (graphs of more than 128 nodes on one CTA each). A batch with a larger graph goes through per-graph `apsp`
+    calls in the free mode (slow, one synchronisation per graph) and raises ValueError in the fixed-width mode (nbins=...), before
+    any launch. edge_index may also be a `LocalEdges` (the batch's edge list
     in its transfer form): batches of graphs with at most 128 nodes then skip the CSR builder altogether — every 4-warp group of
     the BFS kernel builds its graph's adjacency bit matrix in shared memory from the graph's own edge segment
     (gnan_apsp_bfs_batched_local); other batches expand it to the int64 list first.
@@ -445,6 +448,11 @@ def apsp_batched(edge_index, node_off, device="cuda", x=None, y=None, node_off_d
     hop_off_h = np.zeros(B + 1, dtype=np.int64)
     np.cumsum(sizes * sizes, out=hop_off_h[1:])
     total = int(hop_off_h[-1])
+    if max_n > _lib.APSP_BATCHED_MAX_NODES:
+        if nbins is not None:
+            raise ValueError(f"apsp_batched: a graph of {max_n} nodes; the fixed-width mode (nbins=...) takes graphs of at most "
+                             f"{_lib.APSP_BATCHED_MAX_NODES} nodes (call it without nbins: per-graph path)")
+        return _apsp_batched_per_graph(edge_index, no_h, device, x, y)       # (a LocalEdges list cannot address such a graph)
     if node_off_device is None:
         node_off_device = torch.from_numpy(no_h.astype(np.int32)).to(device, non_blocking=True)
     node_off_d = node_off_device
@@ -470,6 +478,8 @@ def apsp_batched(edge_index, node_off, device="cuda", x=None, y=None, node_off_d
             check(lib.gnan_apsp_bfs_batched_ex(ptr(rowptr), ptr(col), ptr(node_off_d), ptr(hop_off), B, max_n, sumN, total, ptr(hop), ptr(cnt_t),
                                                ptr(rs_t), nb, st.data_ptr() + 4, st.data_ptr() + 8, ptr(order_ws), stream_handle()),
                   "gnan_apsp_bfs_batched_ex")
+    def order_ws():                              # graphs are processed grouped by size class (a fifth class above 256 nodes)
+        return torch.empty(5 * B + 5 if max_n > 256 else 4 * B + 4, dtype=torch.int32, device=device)
     nb_full = min(256, max_n + 1)                # a finite hop inside a graph is at most max_n - 1; last column = unreachable
     nb = min(nb_full, _level_table_width) if _level_table_width else nb_full
     if nbins is not None:
@@ -500,9 +510,8 @@ def apsp_batched(edge_index, node_off, device="cuda", x=None, y=None, node_off_d
         return pk
     hop = torch.empty(max(total, 1), dtype=torch.uint8, device=device)
     cnt = torch.empty(sumN, nb, dtype=torch.int32, device=device)
-    order_ws = torch.empty(4 * B + 4, dtype=torch.int32, device=device)     # graphs are processed grouped by size class
     with _timed("apsp_bfs_batched"):
-        bfs(hop, cnt, None, order_ws)
+        bfs(hop, cnt, None, order_ws())
     if nbins is not None:
         pk = PackedBatch(x, hop, hop_off, node_off_d, cnt, y, max_n)
         pk.status = st
@@ -512,7 +521,7 @@ def apsp_batched(edge_index, node_off, device="cuda", x=None, y=None, node_off_d
     if status & 2:
         if isinstance(edge_index, LocalEdges):
             edge_index = edge_index.expand(node_off_d)
-        return _apsp_batched_multi_edges(edge_index, no_h, device, x, y)
+        return _apsp_batched_per_graph(edge_index, no_h, device, x, y)
     if over and nb < nb_full:                    # deeper than the narrow level table: once more with the full width
         return apsp_batched(edge_index, node_off, device, x, y, node_off_device, _level_table_width=0, hop_off_device=hop_off_device)
     if over:
@@ -523,9 +532,10 @@ def apsp_batched(edge_index, node_off, device="cuda", x=None, y=None, node_off_d
     return PackedBatch(x, hop, hop_off, node_off_d, lc, y, max_n)
 
 
-def _apsp_batched_multi_edges(edge_index, no_h, device, x, y):
-    """Slow path of apsp_batched for batches with duplicate edges: per-graph `apsp` (which emulates the reference's summed
-    weights), assembled into the packed form."""
+def _apsp_batched_per_graph(edge_index, no_h, device, x, y):
+    """Slow path of apsp_batched for batches with duplicate edges (per-graph `apsp` emulates the reference's summed weights) or
+    with a graph of more than _lib.APSP_BATCHED_MAX_NODES nodes: one `apsp` call per graph (any size), assembled into the
+    packed form."""
     import numpy as np
     ei = torch.as_tensor(edge_index).to(device=device, dtype=torch.int64)
     B = no_h.shape[0] - 1
@@ -534,6 +544,8 @@ def _apsp_batched_multi_edges(edge_index, no_h, device, x, y):
         lo, hi = int(no_h[b]), int(no_h[b + 1])
         sel = (ei[0] >= lo) & (ei[0] < hi)
         hd = apsp(ei[:, sel] - lo, hi - lo, device=device, method="warp")
+        if hd.wide:
+            raise NotImplementedError("a hop distance > 254 does not fit the uint8 hop matrix")
         hops.append(hd.hop[:, :hi - lo].reshape(-1))
         cnts.append(hd.level_counts)
         D = max(D, hd.nbins - 2)
@@ -555,7 +567,8 @@ def pre_process(data, is_graph_task, data_name=None, processed_data_dir=None, de
     Graph task: `data` is a list of graphs; node task: one graph (num_nodes inferred from edge_index like :128).
     With `processed_data_dir` (and `data_name`) the result is written once, like :144-148, but in the packed format of
     gnan_b200.packed ({dir}/{name}.gnan_b200.pt: 1 byte per node pair instead of 8); read it back with
-    packed.PackedDataset.load (graph task) or packed.load_node (node task).
+    packed.PackedDataset.load (graph task) or packed.load_node (node task). The graph-task file is built by one batched BFS
+    (packed.PackedDataset.from_graphs) for graphs of up to _lib.APSP_BATCHED_MAX_NODES (1024) nodes, per graph beyond.
     """
     import os
     graphs = list(data) if is_graph_task else [data]
