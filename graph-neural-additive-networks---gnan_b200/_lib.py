@@ -94,10 +94,8 @@ SIGNATURES = {
     "gnan_apsp_msbfs_workspace_bytes": (c_size_t, [c_int32]),
     "gnan_apsp_msbfs": (c_int, [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p, c_int64, c_void_p, c_int32, c_void_p,
                                 c_void_p, c_size_t, c_void_p]),
-    "gnan_apsp_bfs_batched": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_int32, c_void_p,
-                                      c_void_p]),
-    "gnan_apsp_bfs_batched_ex": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int64, c_int64, c_void_p, c_void_p,
-                                         c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "gnan_apsp_bfs_batched_ex": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_int32,
+                                         c_void_p, c_void_p, c_void_p, c_void_p]),
     "gnan_loss_workspace_bytes": (c_size_t, []),
     "gnan_cross_entropy_rows": (c_int, [c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_int64, c_float, c_void_p, c_void_p, c_void_p,
                                         c_void_p, c_size_t, c_void_p]),

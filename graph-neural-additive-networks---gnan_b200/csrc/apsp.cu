@@ -10,101 +10,6 @@
 
 namespace {
 
-// ---- batched small graphs: one warp per graph, one lane per source, bitmask frontiers in registers ------------------
-constexpr int BW_MAX = 8;  // up to 256 nodes per graph
-
-__global__ void __launch_bounds__(256)
-apsp_batched_kernel(const int32_t *__restrict__ rowptr, const int32_t *__restrict__ col, const int32_t *__restrict__ node_off,
-                    const int64_t *__restrict__ hop_off, int B, int max_n, uint8_t *__restrict__ hop, int32_t *__restrict__ cnt,
-                    int nbins, int32_t *__restrict__ overflow, int prefilled, int32_t *__restrict__ max_level)
-{
-    extern __shared__ uint32_t sadj[];  // [8 warps][max_n][Wmax]
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    const int Wmax = (max_n + 31) / 32;
-    uint32_t *adj = sadj + (size_t)w * max_n * Wmax;
-    const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
-    int lvl_max = 0;                                       // largest finite hop seen by this lane
-    for (int64_t b = warp; b < B; b += nwarps) {
-        const int n0 = node_off[b], n = node_off[b + 1] - n0;
-        const int W = (n + 31) / 32;
-        uint8_t *hb = hop + hop_off[b];
-        __syncwarp();
-        for (int v = lane; v < n; v += 32) {
-            for (int ww = 0; ww < W; ++ww) adj[v * W + ww] = 0u;
-            for (int e = rowptr[n0 + v]; e < rowptr[n0 + v + 1]; ++e) {
-                const int t = col[e] - n0;
-                if (t >= 0 && t < n) adj[v * W + (t >> 5)] |= 1u << (t & 31);
-            }
-        }
-        __syncwarp();
-        for (int s = lane; s < n; s += 32) {
-            uint32_t vis[BW_MAX], fr[BW_MAX], nx[BW_MAX];
-#pragma unroll
-            for (int ww = 0; ww < BW_MAX; ++ww) { vis[ww] = 0u; fr[ww] = 0u; }
-#pragma unroll
-            for (int ww = 0; ww < BW_MAX; ++ww)
-                if (ww == (s >> 5)) { vis[ww] = 1u << (s & 31); fr[ww] = vis[ww]; }
-            uint8_t *row = hb + (size_t)s * n;
-            if (!prefilled)                                  // (the host wrapper memsets hop / cnt when it knows their sizes)
-                for (int v = 0; v < n; ++v) row[v] = GNAN_HOP_UNREACHABLE;
-            row[s] = 0;
-            int32_t *crow = cnt ? cnt + (int64_t)(n0 + s) * nbins : nullptr;
-            if (crow) {
-                if (!prefilled)
-                    for (int d = 0; d < nbins; ++d) crow[d] = 0;
-                crow[0] = 1;
-            }
-            int reached = 1;
-            for (int level = 1; level <= n; ++level) {
-#pragma unroll
-                for (int ww = 0; ww < BW_MAX; ++ww) nx[ww] = 0u;
-#pragma unroll
-                for (int fw = 0; fw < BW_MAX; ++fw) {
-                    if (fw < W) {
-                        uint32_t m = fr[fw];
-                        while (m) {
-                            const int v = fw * 32 + __ffs(m) - 1;
-                            m &= m - 1;
-#pragma unroll
-                            for (int ww = 0; ww < BW_MAX; ++ww)
-                                if (ww < W) nx[ww] |= adj[v * W + ww];
-                        }
-                    }
-                }
-                int newc = 0;
-#pragma unroll
-                for (int ww = 0; ww < BW_MAX; ++ww) {
-                    nx[ww] &= ~vis[ww];
-                    vis[ww] |= nx[ww];
-                    newc += __popc(nx[ww]);
-                }
-                if (newc == 0) break;
-                if (level > 254 || level >= nbins - 1) { atomicExch(overflow, 1); }
-                const uint8_t lv = (uint8_t)min(level, 254);
-#pragma unroll
-                for (int ww = 0; ww < BW_MAX; ++ww) {
-                    uint32_t m = nx[ww];
-                    while (m) {
-                        row[ww * 32 + __ffs(m) - 1] = lv;
-                        m &= m - 1;
-                    }
-                    fr[ww] = nx[ww];
-                }
-                if (crow && level < nbins - 1) crow[level] = newc;
-                reached += newc;
-                lvl_max = max(lvl_max, level);
-            }
-            if (crow) crow[nbins - 1] = n - reached;
-        }
-    }
-    if (max_level) {
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) lvl_max = max(lvl_max, __shfl_xor_sync(0xffffffffu, lvl_max, o));
-        if (lane == 0 && lvl_max > 0) atomicMax(max_level, lvl_max);
-    }
-}
-
 // ---- batched small graphs, v3: a GROUP of 4 warps per graph slot, bit-parallel over SOURCES -----------------------------------
 // A lane owns ONE vertex v and keeps the bitmask of sources that reach it (W = ceil(n/32) words). Level L is a pull over v's
 // out-neighbours u: new[v] = (OR_u frontier[u]) & ~visited[v]; a new bit s means dist(v -> s) = L, i.e. hop[v][s] = L, and
@@ -321,34 +226,28 @@ __device__ __forceinline__ int bv3_graph(const int32_t *__restrict__ rowptr, con
     return lvl_max;
 }
 
-// graphs by word-count class (0 = 97..128 nodes ... 3 = up to 32), one thread per graph, warp-aggregated counters:
-// cls[0..4) = class sizes (zeroed by the caller), cls[4 + c * B ...) = the graphs of class c in arbitrary order.
-// LARGE (batches with graphs of more than 128 nodes, order_ws [5 * B + 5]; the first 4 * B + 4 words keep their layout): class 4 =
-// more than 128 nodes (apsp_batched_large_kernel), its size at cls[4 * B + 4] (zeroed by the caller), its graphs from cls[4 * B + 5] on.
+// graphs by size class, one thread per graph, warp-aggregated counters: classes 0..3 by word count (0 = 97..128 nodes ... 3 = up
+// to 32) for the v3 kernel, class 4 = more than 128 nodes for apsp_batched_large_kernel. cls[0..4) = the sizes of classes 0..3,
+// cls[4 + c * B ...) = the graphs of class c in arbitrary order; class 4 has its size at cls[4 * B + 4] and its graphs from
+// cls[4 * B + 5] on. The caller zeroes the size words. A batch without graphs of more than 128 nodes leaves class 4 empty and has
+// nothing written at or beyond cls[4 * B + 4] (order_ws [4 * B + 4]).
 // The v3 kernel walks the classes largest first: the expensive graphs start first, and the groups of a CTA run the same
 // instantiation of bv3_graph side by side (the instantiations do not fit the instruction cache together).
-template <bool LARGE>
 __global__ void bv3_classify_kernel(const int32_t *__restrict__ node_off, int B, int32_t *__restrict__ cls)
 {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     const bool ok = b < B;
-    int c = LARGE ? 5 : 4;                                                // (no graph: a value of no class)
+    int c = 5;                                                            // (no graph: a value of no class)
     if (ok) {
         const int n = node_off[b + 1] - node_off[b];
-        c = LARGE && n > 32 * BV3_MAX_W ? 4 : 3 - min(3, max(0, (n - 1) >> 5));
+        c = n > 32 * BV3_MAX_W ? 4 : 3 - min(3, max(0, (n - 1) >> 5));
     }
     const uint32_t peers = __match_any_sync(0xffffffffu, c);
     const int lane = threadIdx.x & 31, leader = __ffs(peers) - 1;
     int base = 0;
-    if constexpr (LARGE) {
-        if (ok && lane == leader) base = atomicAdd(cls + (c < 4 ? c : 4 + 4 * B), __popc(peers));
-        base = __shfl_sync(0xffffffffu, base, leader);
-        if (ok) cls[4 + (size_t)c * B + (c >> 2) + base + __popc(peers & ((1u << lane) - 1))] = b;   // class 4: after its size word
-    } else {
-        if (ok && lane == leader) base = atomicAdd(cls + c, __popc(peers));
-        base = __shfl_sync(0xffffffffu, base, leader);
-        if (ok) cls[4 + (size_t)c * B + base + __popc(peers & ((1u << lane) - 1))] = b;
-    }
+    if (ok && lane == leader) base = atomicAdd(cls + (c < 4 ? c : 4 + 4 * B), __popc(peers));
+    base = __shfl_sync(0xffffffffu, base, leader);
+    if (ok) cls[4 + (size_t)c * B + (c >> 2) + base + __popc(peers & ((1u << lane) - 1))] = b;   // class 4: after its size word
 }
 
 struct Bv3Out {
@@ -1121,13 +1020,23 @@ extern "C" int gnan_apsp_msbfs(const int32_t *rowptr, const int32_t *col, int32_
     return GNAN_OK;
 }
 
-// v3 launch: groups of 4 warps; the group's slice holds one graph of 65..128 nodes, two of 33..64 or four of up to 32
+// bv3_classify_kernel into order_ws ([4*B+4] words, [5*B+5] when max_n > 128)
+static int classify_by_size(const int32_t *node_off, int32_t B, int32_t max_n, int32_t *order_ws, cudaStream_t st)
+{
+    GNAN_CUDA(cudaMemsetAsync(order_ws, 0, 4 * sizeof(int32_t), st));
+    if (max_n > 32 * BV3_MAX_W) GNAN_CUDA(cudaMemsetAsync(order_ws + 4 * (size_t)B + 4, 0, sizeof(int32_t), st));
+    bv3_classify_kernel<<<(unsigned)ceil_div64(B, 256), 256, 0, st>>>(node_off, B, order_ws);
+    GNAN_LAUNCH_OK();
+    return GNAN_OK;
+}
+
+// v3 launch on classes 0..3 of order_ws: groups of 4 warps; the group's slice holds one graph of 65..128 nodes, two of 33..64 or
+// four of up to 32. max_n (at most 128) sizes the slices.
 // CC > 0: the BFS fused with the graph readout (bv3_readout_run; ro holds its tensors, hop / cnt / rscale are NULL)
-// large: the batch also has graphs of more than 128 nodes (order_ws [5*B+5]; max_n = 128 sizes the slices of the others)
 template <bool LOCAL, int CC = 0>
 static int launch_bv3(const int32_t *rowptr, const int32_t *col, const int32_t *node_off, const int64_t *hop_off, int32_t B, int32_t max_n,
                       uint8_t *hop, int32_t *cnt, float *rscale, int nb, bool levels, int32_t *overflow_flag, int32_t *max_level,
-                      int32_t *order_ws, Bv3Edges le, cudaStream_t st, Bv3Readout ro = Bv3Readout{}, bool large = false)
+                      const int32_t *order_ws, Bv3Edges le, cudaStream_t st, Bv3Readout ro = Bv3Readout{})
 {
     const int Wmax = (max_n + 31) / 32;
     auto need = [&](int cap, int W, int G) {
@@ -1148,36 +1057,8 @@ static int launch_bv3(const int32_t *rowptr, const int32_t *col, const int32_t *
         cached_smem3 = smem3; cached_gpc = gpc;
     }
     const int blocks3 = (int)std::min<int64_t>(ceil_div64(B, gpc), (int64_t)std::max(cached_per_sm3, 1) * gnan_sm_count());
-    GNAN_CUDA(cudaMemsetAsync(order_ws, 0, 4 * sizeof(int32_t), st));
-    if (large) {
-        GNAN_CUDA(cudaMemsetAsync(order_ws + 4 * (size_t)B + 4, 0, sizeof(int32_t), st));
-        bv3_classify_kernel<true><<<(unsigned)ceil_div64(B, 256), 256, 0, st>>>(node_off, B, order_ws);
-    } else {
-        bv3_classify_kernel<false><<<(unsigned)ceil_div64(B, 256), 256, 0, st>>>(node_off, B, order_ws);
-    }
-    GNAN_LAUNCH_OK();
     kernel<<<blocks3, 32 * BV3_GW * gpc, smem3, st>>>(rowptr, col, node_off, hop_off, B, max_n, gpc, (int)slice, hop, cnt, rscale, nb,
                                                       overflow_flag, max_level, order_ws, le, ro);
-    GNAN_LAUNCH_OK();
-    return GNAN_OK;
-}
-
-// the lane-per-source kernel for graphs of up to 256 nodes (the caller has checked the arguments)
-static int launch_batched_lanes(const int32_t *rowptr, const int32_t *col, const int32_t *node_off, const int64_t *hop_off, int32_t B,
-                                int32_t max_n, int64_t total_nodes, int64_t total_hop_bytes, uint8_t *hop, int32_t *cnt, int32_t nbins,
-                                int32_t *overflow_flag, int32_t *max_level, cudaStream_t st)
-{
-    const size_t smem = sizeof(uint32_t) * 8 * (size_t)max_n * ((max_n + 31) / 32);
-    GNAN_CUDA(cudaFuncSetAttribute(apsp_batched_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const int blocks = (int)std::min<int64_t>(ceil_div64(B, 8), 16 * gnan_sm_count());
-    // with the totals known on the host the 255 / 0 background is two memsets at HBM speed instead of per-lane store loops
-    const int prefilled = total_nodes > 0 && total_hop_bytes > 0;
-    if (prefilled) {
-        GNAN_CUDA(cudaMemsetAsync(hop, GNAN_HOP_UNREACHABLE, (size_t)total_hop_bytes, st));
-        if (cnt) GNAN_CUDA(cudaMemsetAsync(cnt, 0, sizeof(int32_t) * (size_t)total_nodes * nbins, st));
-    }
-    apsp_batched_kernel<<<blocks, 256, smem, st>>>(rowptr, col, node_off, hop_off, B, max_n, hop, cnt,
-                                                   cnt ? nbins : 256, overflow_flag, prefilled, max_level);
     GNAN_LAUNCH_OK();
     return GNAN_OK;
 }
@@ -1197,21 +1078,19 @@ static int launch_batched_large(const int32_t *rowptr, const int32_t *col, const
     return GNAN_OK;
 }
 
-// graphs of at most 128 nodes with known totals: v3; at most 256 nodes otherwise: the lane-per-source kernel; larger graphs (up to
-// GNAN_APSP_BATCHED_MAX_NODES, totals known): v3 for the graphs of at most 128 nodes and apsp_batched_large_kernel for the others.
+// graphs of at most 128 nodes: v3; graphs of 129..GNAN_APSP_BATCHED_MAX_NODES nodes: apsp_batched_large_kernel, one CTA each.
 // rscale (optional): 1/count per (node, level) as fp32, what gnan_level_rscale would compute from cnt; cnt may then be NULL
 extern "C" int gnan_apsp_bfs_batched_ex(const int32_t *rowptr, const int32_t *col, const int32_t *node_off, const int64_t *hop_off,
-                                        int32_t B, int32_t max_n, int64_t total_nodes, int64_t total_hop_bytes, uint8_t *hop,
-                                        int32_t *cnt, float *rscale, int32_t nbins, int32_t *overflow_flag, int32_t *max_level,
-                                        int32_t *order_ws, gnan_stream_t stream)
+                                        int32_t B, int32_t max_n, uint8_t *hop, int32_t *cnt, float *rscale, int32_t nbins,
+                                        int32_t *overflow_flag, int32_t *max_level, int32_t *order_ws, gnan_stream_t stream)
 {
     GNAN_REQUIRE(B >= 0, "apsp_bfs_batched: negative batch");
     if (B == 0) return GNAN_OK;
     GNAN_REQUIRE(rowptr && node_off && hop_off && hop && overflow_flag, "apsp_bfs_batched: NULL pointer");
     GNAN_REQUIRE(order_ws, "apsp_bfs_batched: NULL order_ws");
     GNAN_REQUIRE(!(cnt || rscale) || (nbins >= 2 && nbins <= 256), "apsp_bfs_batched: nbins %d out of [2,256]", nbins);
-    if (rscale && !(max_n <= 32 * BV3_MAX_W && total_nodes > 0)) {
-        gnan_set_error("apsp_bfs_batched: the fused 1/count output needs graphs of at most %d nodes and the totals", 32 * BV3_MAX_W);
+    if (rscale && max_n > 32 * BV3_MAX_W) {
+        gnan_set_error("apsp_bfs_batched: the fused 1/count output needs graphs of at most %d nodes", 32 * BV3_MAX_W);
         return GNAN_ERR_UNSUPPORTED;
     }
     if (max_n < 1 || max_n > GNAN_APSP_BATCHED_MAX_NODES) {
@@ -1219,32 +1098,16 @@ extern "C" int gnan_apsp_bfs_batched_ex(const int32_t *rowptr, const int32_t *co
                        max_n, GNAN_APSP_BATCHED_MAX_NODES);
         return GNAN_ERR_UNSUPPORTED;
     }
-    if (max_n > 32 * BW_MAX && total_nodes <= 0) {
-        gnan_set_error("apsp_bfs_batched: graphs of %d..%d (GNAN_APSP_BATCHED_MAX_NODES) nodes need the totals (total_nodes > 0)",
-                       32 * BW_MAX + 1, GNAN_APSP_BATCHED_MAX_NODES);
-        return GNAN_ERR_UNSUPPORTED;
-    }
     cudaStream_t st = (cudaStream_t)stream;
-    if (max_n <= 32 * BV3_MAX_W && total_nodes > 0) {
-        const bool levels = cnt || rscale;
-        const int rc = launch_bv3<false>(rowptr, col, node_off, hop_off, B, max_n, hop, cnt, rscale, levels ? nbins : 256, levels,
-                                         overflow_flag, max_level, order_ws, Bv3Edges{}, st);
-        if (rc == GNAN_ERR_UNSUPPORTED) gnan_set_error("apsp_bfs_batched: level table too wide for the shared-memory slice");
-        return rc;
-    }
-    if (max_n > 32 * BW_MAX) {
-        const int nb = cnt ? nbins : 256;
-        const int rc = launch_bv3<false>(rowptr, col, node_off, hop_off, B, 32 * BV3_MAX_W, hop, cnt, nullptr, nb, cnt != nullptr,
-                                         overflow_flag, max_level, order_ws, Bv3Edges{}, st, Bv3Readout{}, true);
-        if (rc == GNAN_ERR_UNSUPPORTED) {
-            gnan_set_error("apsp_bfs_batched: level table too wide for the shared-memory slice");
-            return rc;
-        }
-        if (rc != GNAN_OK) return rc;
-        return launch_batched_large(rowptr, col, node_off, hop_off, B, hop, cnt, nb, overflow_flag, max_level, order_ws, st);
-    }
-    return launch_batched_lanes(rowptr, col, node_off, hop_off, B, max_n, total_nodes, total_hop_bytes, hop, cnt, nbins, overflow_flag,
-                                max_level, st);
+    const bool levels = cnt || rscale;
+    const int nb = levels ? nbins : 256;
+    int rc = classify_by_size(node_off, B, max_n, order_ws, st);
+    if (rc != GNAN_OK) return rc;
+    rc = launch_bv3<false>(rowptr, col, node_off, hop_off, B, std::min(max_n, 32 * BV3_MAX_W), hop, cnt, rscale, nb, levels,
+                           overflow_flag, max_level, order_ws, Bv3Edges{}, st);
+    if (rc == GNAN_ERR_UNSUPPORTED) gnan_set_error("apsp_bfs_batched: level table too wide for the shared-memory slice");
+    if (rc != GNAN_OK || max_n <= 32 * BV3_MAX_W) return rc;
+    return launch_batched_large(rowptr, col, node_off, hop_off, B, hop, cnt, nb, overflow_flag, max_level, order_ws, st);
 }
 
 // The batched BFS straight from the batch's edge list in its transfer form (no CSR): see include/gnan_b200.h
@@ -1267,8 +1130,10 @@ extern "C" int gnan_apsp_bfs_batched_local(const uint8_t *src, const uint8_t *ds
     }
     const bool levels = cnt || rscale;
     const Bv3Edges le{src, dst, edge_off, status};
-    const int rc = launch_bv3<true>(nullptr, nullptr, node_off, hop_off, B, max_n, hop, cnt, rscale, levels ? nbins : 256, levels,
-                                    overflow_flag, max_level, order_ws, le, st);
+    int rc = classify_by_size(node_off, B, max_n, order_ws, st);
+    if (rc != GNAN_OK) return rc;
+    rc = launch_bv3<true>(nullptr, nullptr, node_off, hop_off, B, max_n, hop, cnt, rscale, levels ? nbins : 256, levels,
+                          overflow_flag, max_level, order_ws, le, st);
     if (rc == GNAN_ERR_UNSUPPORTED) gnan_set_error("apsp_bfs_batched_local: level table too wide for the shared-memory slice");
     return rc;
 }
@@ -1300,23 +1165,12 @@ extern "C" int gnan_bfs_graph_readout_fwd(const uint8_t *src, const uint8_t *dst
         return launch_bv3<true, decltype(cc)::value>(nullptr, nullptr, node_off, nullptr, B, max_n, nullptr, nullptr, nullptr, nbins, false,
                                                      overflow_flag, max_level, order_ws, le, st, ro);
     };
-    const int rc = C == 1 ? launch(std::integral_constant<int, 1>{}) : C == 2 ? launch(std::integral_constant<int, 2>{})
-                                                                             : launch(std::integral_constant<int, 4>{});
+    int rc = classify_by_size(node_off, B, max_n, order_ws, st);
+    if (rc != GNAN_OK) return rc;
+    rc = C == 1 ? launch(std::integral_constant<int, 1>{}) : C == 2 ? launch(std::integral_constant<int, 2>{})
+                                                                   : launch(std::integral_constant<int, 4>{});
     if (rc == GNAN_ERR_UNSUPPORTED) gnan_set_error("bfs_graph_readout_fwd: per-graph state too large for the shared-memory slice");
     return rc;
-}
-
-extern "C" int gnan_apsp_bfs_batched(const int32_t *rowptr, const int32_t *col, const int32_t *node_off, const int64_t *hop_off,
-                                     int32_t B, uint8_t *hop, int32_t *cnt, int32_t nbins, int32_t *overflow_flag,
-                                     gnan_stream_t stream)
-{
-    GNAN_REQUIRE(B >= 0, "apsp_bfs_batched: negative batch");
-    if (B == 0) return GNAN_OK;
-    GNAN_REQUIRE(rowptr && node_off && hop_off && hop && overflow_flag, "apsp_bfs_batched: NULL pointer");
-    GNAN_REQUIRE(!cnt || (nbins >= 2 && nbins <= 256), "apsp_bfs_batched: nbins %d out of [2,256]", nbins);
-    // without a host-side size hint assume the largest supported graph
-    return launch_batched_lanes(rowptr, col, node_off, hop_off, B, 32 * BW_MAX, 0, 0, hop, cnt, nbins, overflow_flag, nullptr,
-                                (cudaStream_t)stream);
 }
 
 extern "C" int gnan_hops_to_reference(const uint8_t *hop, int64_t R, int64_t N, int64_t ld_hop, const int32_t *cnt,

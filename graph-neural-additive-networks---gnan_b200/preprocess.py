@@ -406,9 +406,9 @@ def apsp_batched(edge_index, node_off, device="cuda", x=None, y=None, node_off_d
                  hop_off_device=None, rscale=False, pair_stats=False):
     """Hop blocks of B graphs in one launch. edge_index uses GLOBAL node ids of the
     concatenated node set; node_off [B+1] are the graph boundaries. Graphs of up to _lib.APSP_BATCHED_MAX_NODES (1024) nodes run
-    in the batched BFS (graphs of more than 128 nodes on one CTA each). A batch with a larger graph goes through per-graph `apsp`
-    calls in the free mode (slow, one synchronisation per graph) and raises ValueError in the fixed-width mode (nbins=...), before
-    any launch. edge_index may also be a `LocalEdges` (the batch's edge list
+    in the batched BFS, each by its own size: up to 128 nodes on groups of 4 warps, more on one CTA each. A batch with a larger
+    graph goes through per-graph `apsp` calls in the free mode (slow, one synchronisation per graph) and raises ValueError in the
+    fixed-width mode (nbins=...), before any launch. edge_index may also be a `LocalEdges` (the batch's edge list
     in its transfer form): batches of graphs with at most 128 nodes then skip the CSR builder altogether — every 4-warp group of
     the BFS kernel builds its graph's adjacency bit matrix in shared memory from the graph's own edge segment
     (gnan_apsp_bfs_batched_local); other batches expand it to the int64 list first.
@@ -469,17 +469,17 @@ def apsp_batched(edge_index, node_off, device="cuda", x=None, y=None, node_off_d
     if local is None:
         rowptr, col, _ = build_csr(edge_index, sumN, device, status=st[0:1])
 
-    def bfs(hop, cnt_t, rs_t, order_ws):
+    def bfs(hop, cnt_t, rs_t):
+        # scratch of the size classes the BFS groups the graphs by (a fifth class above 128 nodes)
+        order_ws = torch.empty(5 * B + 5 if max_n > 128 else 4 * B + 4, dtype=torch.int32, device=device)
         if local is not None:
             check(lib.gnan_apsp_bfs_batched_local(ptr(local.src), ptr(local.dst), ptr(local.edge_off), ptr(node_off_d), ptr(hop_off), B, max_n,
                                                   ptr(hop), ptr(cnt_t), ptr(rs_t), nb, st.data_ptr(), st.data_ptr() + 4, st.data_ptr() + 8,
                                                   ptr(order_ws), stream_handle()), "gnan_apsp_bfs_batched_local")
         else:
-            check(lib.gnan_apsp_bfs_batched_ex(ptr(rowptr), ptr(col), ptr(node_off_d), ptr(hop_off), B, max_n, sumN, total, ptr(hop), ptr(cnt_t),
+            check(lib.gnan_apsp_bfs_batched_ex(ptr(rowptr), ptr(col), ptr(node_off_d), ptr(hop_off), B, max_n, ptr(hop), ptr(cnt_t),
                                                ptr(rs_t), nb, st.data_ptr() + 4, st.data_ptr() + 8, ptr(order_ws), stream_handle()),
                   "gnan_apsp_bfs_batched_ex")
-    def order_ws():                              # graphs are processed grouped by size class (a fifth class above 256 nodes)
-        return torch.empty(5 * B + 5 if max_n > 256 else 4 * B + 4, dtype=torch.int32, device=device)
     nb_full = min(256, max_n + 1)                # a finite hop inside a graph is at most max_n - 1; last column = unreachable
     nb = min(nb_full, _level_table_width) if _level_table_width else nb_full
     if nbins is not None:
@@ -493,25 +493,23 @@ def apsp_batched(edge_index, node_off, device="cuda", x=None, y=None, node_off_d
             def materialise():
                 hop = torch.empty(max(total, 1), dtype=torch.uint8, device=device)
                 rs = torch.empty(sumN, nb, dtype=torch.float32, device=device)
-                order_ws = torch.empty(4 * B + 4, dtype=torch.int32, device=device)
                 with _timed("apsp_bfs_batched"):
-                    bfs(hop, None, rs, order_ws)
+                    bfs(hop, None, rs)
                 return hop, rs
             pk = _DeferredBatch(x, hop_off, node_off_d, y, max_n, nb, local, materialise)
             pk.status = st
             return pk
         hop = torch.empty(max(total, 1), dtype=torch.uint8, device=device)
         rs = torch.empty(sumN, nb, dtype=torch.float32, device=device)
-        order_ws = torch.empty(4 * B + 4, dtype=torch.int32, device=device)
         with _timed("apsp_bfs_batched"):
-            bfs(hop, None, rs, order_ws)
+            bfs(hop, None, rs)
         pk = PackedBatch(x, hop, hop_off, node_off_d, None, y, max_n, level_rscale=rs)
         pk.status = st
         return pk
     hop = torch.empty(max(total, 1), dtype=torch.uint8, device=device)
     cnt = torch.empty(sumN, nb, dtype=torch.int32, device=device)
     with _timed("apsp_bfs_batched"):
-        bfs(hop, cnt, None, order_ws())
+        bfs(hop, cnt, None)
     if nbins is not None:
         pk = PackedBatch(x, hop, hop_off, node_off_d, cnt, y, max_n)
         pk.status = st

@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define GNAN_B200_VERSION 100
+#define GNAN_B200_VERSION 101
 
 enum {
     GNAN_OK = 0,
@@ -35,7 +35,7 @@ enum {
 };
 
 #define GNAN_HOP_UNREACHABLE 255 /* byte value of an unreachable / masked pair in a hop matrix */
-#define GNAN_APSP_BATCHED_MAX_NODES 1024 /* largest graph of gnan_apsp_bfs_batched_ex (with the totals known) */
+#define GNAN_APSP_BATCHED_MAX_NODES 1024 /* largest graph of gnan_apsp_bfs_batched_ex */
 
 typedef void *gnan_stream_t;
 
@@ -318,31 +318,22 @@ int gnan_apsp_msbfs(const int32_t *rowptr, const int32_t *col, int32_t N, int32_
                     int64_t ld_hop, int32_t *cnt, int32_t nbins, int32_t *overflow_flag, void *workspace,
                     size_t workspace_bytes, gnan_stream_t stream);
 
-/* B small graphs in one launch; CSR over the concatenated node set with GLOBAL column ids. */
-int gnan_apsp_bfs_batched(const int32_t *rowptr /* [sumN+1] */, const int32_t *col, const int32_t *node_off /* [B+1] */,
-                          const int64_t *hop_off /* [B+1] */, int32_t B, uint8_t *hop, int32_t *cnt /* [sumN,nbins] or NULL */,
-                          int32_t nbins, int32_t *overflow_flag, gnan_stream_t stream);
-
-/* same with host-side size hints: max_n = the largest graph (sizes shared memory; 1..GNAN_APSP_BATCHED_MAX_NODES); total_nodes =
- * node_off[B] and total_hop_bytes = hop_off[B] (0 = unknown); max_level (optional, zero-initialised by the caller) receives the
- * largest finite hop of the batch (atomicMax), which sizes the trimmed level table. order_ws is required scratch: [4*B+4] words,
- * [5*B+5] when max_n > 256.
- * Routing by max_n:
- *  - at most 128 nodes with the totals known: the graphs are grouped by size class, and a GROUP OF 4 WARPS works on one graph of
- *    65..128 nodes, two of 33..64 or four of up to 32 nodes at a time (one vertex per lane, a named barrier with an OR reduction
- *    per BFS level);
- *  - at most 256 nodes otherwise: one lane per source; with both totals > 0 the unreachable / zero background of hop and cnt is
- *    then written by two memsets at HBM speed instead of per-source store loops;
- *  - 257..GNAN_APSP_BATCHED_MAX_NODES nodes, totals required: the graphs of at most 128 nodes as in the first case, the others
- *    on one CTA each (one or two vertices per thread, 128 sources at a time). Both launches go on `stream`, no synchronisation.
- * Larger graphs, or max_n > 256 without the totals: GNAN_ERR_UNSUPPORTED before any CUDA call (gnan_apsp_bfs takes one graph of
- * any size).
+/* B graphs in one launch; CSR over the concatenated node set with GLOBAL column ids. max_n = the largest graph (sizes shared
+ * memory; 1..GNAN_APSP_BATCHED_MAX_NODES); max_level (optional, zero-initialised by the caller) receives the largest finite hop of
+ * the batch (atomicMax), which sizes the trimmed level table. order_ws is required scratch: [4*B+4] words, [5*B+5] when
+ * max_n > 128.
+ * Each graph runs by its own size:
+ *  - at most 128 nodes: the graphs are grouped by size class, and a GROUP OF 4 WARPS works on one graph of 65..128 nodes, two of
+ *    33..64 or four of up to 32 nodes at a time (one vertex per lane, a named barrier with an OR reduction per BFS level);
+ *  - 129..GNAN_APSP_BATCHED_MAX_NODES nodes: one CTA per graph (one or two vertices per thread, 128 sources at a time).
+ * Both launches go on `stream`, no synchronisation. max_n outside 1..GNAN_APSP_BATCHED_MAX_NODES: GNAN_ERR_UNSUPPORTED before any
+ * CUDA call (gnan_apsp_bfs takes one graph of any size).
  * rscale (optional) [sumN,nbins] fp32 = 1/count (0 for an empty level), i.e. what gnan_level_rscale computes from cnt
- * (models.py:368-370 divides by the level size); cnt may then be NULL. Needs the totals and graphs of at most 128 nodes. */
-int gnan_apsp_bfs_batched_ex(const int32_t *rowptr, const int32_t *col, const int32_t *node_off, const int64_t *hop_off,
-                             int32_t B, int32_t max_n, int64_t total_nodes, int64_t total_hop_bytes, uint8_t *hop, int32_t *cnt,
-                             float *rscale, int32_t nbins, int32_t *overflow_flag, int32_t *max_level,
-                             int32_t *order_ws /* [4*B+4], [5*B+5] if max_n > 256 */, gnan_stream_t stream);
+ * (models.py:368-370 divides by the level size); cnt may then be NULL. Needs graphs of at most 128 nodes. */
+int gnan_apsp_bfs_batched_ex(const int32_t *rowptr /* [sumN+1] */, const int32_t *col, const int32_t *node_off /* [B+1] */,
+                             const int64_t *hop_off /* [B+1] */, int32_t B, int32_t max_n, uint8_t *hop,
+                             int32_t *cnt /* [sumN,nbins] or NULL */, float *rscale, int32_t nbins, int32_t *overflow_flag,
+                             int32_t *max_level, int32_t *order_ws /* [4*B+4], [5*B+5] if max_n > 128 */, gnan_stream_t stream);
 
 /* gnan_apsp_bfs_batched_ex WITHOUT a CSR: the batch's edges in their transfer form (gnan_edges_from_local: src / dst uint8 indices
  * inside the graph, edge_off [B+1], edges grouped by graph). Every 4-warp group builds its graph's adjacency bit matrix in shared

@@ -35,7 +35,7 @@ def test_python_binding_covers_header(lib_path):
     from gnan_b200 import _lib
     assert sorted(_lib.SIGNATURES) == header_functions()
     lib = _lib.load()
-    assert lib.gnan_version() == 100
+    assert lib.gnan_version() == 101
     assert lib.gnan_last_error() is not None
 
 
@@ -50,7 +50,7 @@ def test_argument_validation_without_gpu(lib_path):
     assert rc == 1
     arr = (ctypes.c_int64 * 8)()
     buf = ctypes.addressof(arr)
-    rc =lib.gnan_apsp_bfs_batched_ex(buf, buf, buf, buf, 1, 4, 4, 16, buf, None, None, 0, buf, None, None, None)   # order_ws NULL
+    rc = lib.gnan_apsp_bfs_batched_ex(buf, buf, buf, buf, 1, 4, buf, None, None, 0, buf, None, None, None)   # order_ws NULL
     assert rc == 1 and b"order_ws" in lib.gnan_last_error()
     assert lib.gnan_mlp_workspace_bytes(0, ctypes.byref(p), 0, 0) == 0
 
@@ -97,7 +97,7 @@ def test_c99_consumer_compiles_against_the_header_and_calls_the_library(lib_path
     subprocess.run(["gcc", "-std=c99", "-Wall", "-Wextra", "-Werror", "-pedantic", "-I", os.path.join(ROOT, "include"), str(src), "-o", str(exe), "-ldl"],
                    check=True, capture_output=True, text=True)
     out = subprocess.run([str(exe), lib_path], check=True, capture_output=True, text=True).stdout.split(None, 4)
-    assert out[0] == "100" and int(out[1]) != 0 and out[2] == "1" and int(out[3]) >= 0 and "level_rscale" in out[4]
+    assert out[0] == "101" and int(out[1]) != 0 and out[2] == "1" and int(out[3]) >= 0 and "level_rscale" in out[4]
     # and as C++ (the reference-side binding may be either)
     subprocess.run(["g++", "-std=c++11", "-Wall", "-Werror", "-fsyntax-only", "-x", "c++", "-I", os.path.join(ROOT, "include"), str(src)],
                    check=True, capture_output=True, text=True)

@@ -108,10 +108,12 @@ def mixed_batch(directed, seed=5):
     return [(varied_graph(rng, n, directed), n) for n in sizes]
 
 
-@pytest.mark.parametrize("directed", [False, True])
-def test_mixed_batch_exact_free_and_fixed_width(directed):
+@pytest.mark.parametrize("directed,cap", [(False, 1024), (True, 1024), (False, 256), (True, 256)],
+                         ids=["False", "True", "False-256", "True-256"])
+def test_mixed_batch_exact_free_and_fixed_width(directed, cap):
+    """cap: the batch keeps the graphs of mixed_batch with at most cap nodes (256: the largest graph has 129..256 nodes)"""
     from gnan_b200.preprocess import apsp_batched, check_batched_status
-    graphs = mixed_batch(directed)
+    graphs = [(e, n) for e, n in mixed_batch(directed) if n <= cap]
     ei, node_off = concat(graphs)
     pk = apsp_batched(ei, node_off, device=DEV)
     dmax = assert_batch_equals_oracle(pk, graphs, node_off)
@@ -136,20 +138,20 @@ def _has(names, kernel):
 
 
 def test_routing_of_large_and_small_graphs():
+    """Each graph runs by its own size: at most 128 nodes on the v3 kernel, more on the large kernel, whatever the rest of the batch"""
     from gnan_b200.preprocess import apsp_batched
     graphs = mixed_batch(False)
-    ei, node_off = concat(graphs)
-    apsp_batched(ei, node_off, device=DEV)                                  # warm-up (module load, attribute setting)
-    names = _kernel_names(lambda: apsp_batched(ei, node_off, device=DEV))
-    assert _has(names, "apsp_batched_v3_kernel") and _has(names, "apsp_batched_large_kernel"), names
-    assert not _has(names, "apsp_batched_kernel"), names
-    # max_n = 256: the lane-per-source kernel alone, as before graphs above 256 nodes were batched
-    small = [(e, n) for e, n in graphs if n <= 256]
-    ei2, node_off2 = concat(small)
-    apsp_batched(ei2, node_off2, device=DEV)
-    names = _kernel_names(lambda: apsp_batched(ei2, node_off2, device=DEV))
-    assert _has(names, "apsp_batched_kernel"), names
-    assert not any(_has(names, k) for k in ("apsp_batched_v3_kernel", "apsp_batched_large_kernel", "bv3_classify_kernel")), names
+    batches = {"up to 1024": (graphs, True, True), "up to 256": ([g for g in graphs if g[1] <= 256], True, True),
+               "129..256 only": ([g for g in graphs if 128 < g[1] <= 256], False, True),
+               "up to 128": ([g for g in graphs if g[1] <= 128], True, False)}
+    for name, (gs, v3, large) in batches.items():
+        ei, node_off = concat(gs)
+        apsp_batched(ei, node_off, device=DEV)                              # warm-up (module load, attribute setting)
+        names = _kernel_names(lambda: apsp_batched(ei, node_off, device=DEV))
+        assert _has(names, "bv3_classify_kernel"), (name, names)
+        assert not v3 or _has(names, "apsp_batched_v3_kernel"), (name, names)
+        assert _has(names, "apsp_batched_large_kernel") == large, (name, names)
+        assert not _has(names, "apsp_batched_kernel"), (name, names)
 
 
 def test_deep_large_graph_redo_and_hop_overflow():

@@ -1,4 +1,4 @@
-"""Batched BFS on datasets with graphs of more than 256 nodes (apsp_batched_large_kernel). Needs a GPU.
+"""Batched BFS on datasets with graphs of more than 128 nodes (apsp_batched_large_kernel). Needs a GPU.
 
     python tests/tools/bench_apsp_large.py [--out result.json] [--reps 20]
 
@@ -8,6 +8,10 @@
 (b) the Mutagenicity-shaped batch in the fixed-width mode (nbins=64, no host synchronisation) with and without its tail: CUDA events
     over --reps calls; the difference is about the large-graph kernel's own time, which torch.profiler also reports in a separate run.
 (c) 1000 graphs of 257..1024 nodes: graphs/s and GB/s of hop bytes written (fixed-width mode, CUDA events).
+(d) batches whose largest graph has 129..256 nodes: d1 = 4000 molecule-like graphs of 129..256 nodes (about 150 MB of hop bytes,
+    more than L2), d2 = the PROTEINS-shaped size draw without its tail (4..256 nodes) four times over. Fixed-width calls (nbins=64,
+    CUDA events, three windows of --reps calls) and PackedDataset.from_graphs (host clock), each also with one extra edgeless
+    257-node graph appended, and that graph alone. The extra graph costs one CTA of the large kernel, three chunks of one level.
 The card's name and power limit are read in the same run."""
 import argparse
 import json
@@ -15,6 +19,7 @@ import os
 import subprocess
 import sys
 import time
+from types import SimpleNamespace
 
 import numpy as np
 import torch
@@ -29,8 +34,9 @@ DEV = "cuda"
 
 def proteins_sizes(rng, n_graphs=1113, n_tail=12):
     sizes = np.clip(np.round(rng.lognormal(3.4, 0.6, size=n_graphs)), 4, 256).astype(np.int64)
-    sizes[-n_tail:] = rng.integers(257, 621, size=n_tail)
-    sizes[-1] = 620
+    if n_tail:
+        sizes[-n_tail:] = rng.integers(257, 621, size=n_tail)
+        sizes[-1] = 620
     return sizes
 
 
@@ -143,6 +149,26 @@ def main():
                                 "large_kernel_ms_profiler": k_big,
                                 "hop_GB_per_s_kernel": hop_bytes / (k_big / 1e3) / 1e9 if k_big else None}
     print(res["large_graphs_1000"], flush=True)
+
+    # (d) largest graph of 129..256 nodes, alone and with one edgeless 257-node graph
+    rng = np.random.default_rng(2)
+    mid = {"d1_129_to_256": molecule_like_graphs(rng, rng.integers(129, 257, size=4000)),
+           "d2_proteins_shaped_no_tail_x4": molecule_like_graphs(rng, np.tile(proteins_sizes(rng, n_tail=0), 4))}
+    extra = SimpleNamespace(x=torch.zeros(257, 14), edge_index=torch.zeros(2, 0, dtype=torch.int64), y=torch.tensor([0.0]))
+    for name, graphs in mid.items():
+        r = {}
+        for key, gs in (("", graphs), ("_plus_257", graphs + [extra]), ("_257_alone", [extra])):
+            ei, node_off, sizes = packed_inputs(gs)
+            eid = ei.to(DEV)
+            pk = apsp_batched(eid, node_off, device=DEV, nbins=nb)
+            check_batched_status(pk.status)
+            r["graphs" + key] = len(gs)
+            r["hop_bytes" + key] = int((sizes ** 2).sum())
+            r["call_ms" + key] = [event_time_ms(lambda: apsp_batched(eid, node_off, device=DEV, nbins=nb), args.reps) for _ in range(3)]
+            r["bfs_kernels_ms_profiler" + key] = kernel_time_ms(lambda: apsp_batched(eid, node_off, device=DEV, nbins=nb), "apsp_batched_")
+            r["from_graphs_s" + key] = host_time(lambda: PackedDataset.from_graphs(gs, device=DEV), reps=3)
+        res[name] = r
+        print(name, r, flush=True)
     print(json.dumps(res))
     if args.out:
         os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
