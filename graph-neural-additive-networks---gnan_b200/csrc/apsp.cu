@@ -1153,8 +1153,8 @@ extern "C" int gnan_bfs_graph_readout_fwd(const uint8_t *src, const uint8_t *dst
     cudaStream_t st = (cudaStream_t)stream;
     GNAN_CUDA(cudaMemsetAsync(status, 0, sizeof(int32_t), st));
     if (B == 0) return GNAN_OK;
-    GNAN_REQUIRE(src && dst && edge_off && node_off && T && S && out && colw && Q && overflow_flag && order_ws,
-                 "bfs_graph_readout_fwd: NULL pointer");
+    // src / dst are read only inside the graphs' edge segments: NULL is fine for a batch without edges (an empty edge list)
+    GNAN_REQUIRE(edge_off && node_off && T && S && out && colw && Q && overflow_flag && order_ws, "bfs_graph_readout_fwd: NULL pointer");
     if (max_n < 1 || max_n > 32 * BV3_MAX_W) {
         gnan_set_error("bfs_graph_readout_fwd: graphs with %d nodes unsupported (1..%d)", max_n, 32 * BV3_MAX_W);
         return GNAN_ERR_UNSUPPORTED;
