@@ -42,7 +42,6 @@ SIGNATURES = {
     "gnan_mlp_bwd_ext": (c_int, [c_void_p, c_int64, c_int64, ctypes.POINTER(MlpParams), c_float, c_uint64, c_void_p, c_int, c_void_p,
                                  c_void_p, c_void_p, ctypes.POINTER(MlpGrads), c_void_p, c_size_t, c_void_p]),
     "gnan_mlp_entries_workspace_bytes": (c_size_t, [c_int64, ctypes.POINTER(MlpParams), c_int, c_int]),
-    "gnan_mlp_entries_fwd": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int64, ctypes.POINTER(MlpParams), c_void_p, c_void_p]),
     "gnan_mlp_entries_fwd_ex": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int64, ctypes.POINTER(MlpParams), c_int, c_void_p, c_void_p]),
     "gnan_mlp_entries_bwd": (c_int, [c_void_p, c_void_p, c_int64, c_int64, ctypes.POINTER(MlpParams), c_int, c_void_p,
                                      ctypes.POINTER(MlpGrads), c_void_p, c_size_t, c_void_p]),
@@ -53,11 +52,6 @@ SIGNATURES = {
     "gnan_gather_segment_sum": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_void_p, c_void_p]),
     "gnan_rho_table_inputs": (c_int, [c_void_p, c_int64, c_int32, c_int, c_void_p, c_void_p]),
     "gnan_level_rscale": (c_int, [c_void_p, c_int64, c_int32, c_void_p, c_void_p]),
-    "gnan_aggregate_rows_fwd": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_int32, c_int32, c_void_p,
-                                        c_void_p, c_int32, c_void_p, c_void_p]),
-    "gnan_aggregate_rows_fwd_save": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_int32, c_int32, c_void_p,
-                                             c_void_p, c_int32, c_void_p, c_void_p, c_void_p]),
-    "gnan_aggregate_rows_tc_supported": (c_int, [c_int64, c_int64, c_int64, c_int32, c_int32]),
     "gnan_aggregate_rows_fwd_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64, c_int32, c_int32]),
     "gnan_aggregate_rows_fwd_ws": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_int32, c_int32, c_void_p,
                                            c_void_p, c_int32, c_void_p, c_void_p, c_int, c_void_p, c_size_t, c_void_p]),
@@ -65,12 +59,6 @@ SIGNATURES = {
     "gnan_aggregate_rows_bwd_ws": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_int32, c_int32, c_void_p,
                                            c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_size_t,
                                            c_void_p]),
-    "gnan_aggregate_rows_bwd_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int32, c_int32, c_int32]),
-    "gnan_aggregate_rows_bwd": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_int32, c_int32, c_void_p,
-                                        c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
-    "gnan_aggregate_rows_bwd_saved": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_int32, c_int32, c_void_p,
-                                              c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t,
-                                              c_void_p]),
     "gnan_aggregate_blockdiag_fwd": (c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_int, c_int32, c_int32,
                                              c_void_p, c_void_p, c_int32, c_int, c_void_p, c_void_p]),
     "gnan_aggregate_blockdiag_graph_supported": (c_int, [c_int32, c_int32, c_int32]),

@@ -580,10 +580,10 @@ extern "C" int gnan_level_rscale(const int32_t *cnt, int64_t rows, int32_t nbins
     return GNAN_OK;
 }
 
-// forward with optional Bsum save (internal symbol also exported for the Python autograd wrapper)
-extern "C" int gnan_aggregate_rows_fwd_save(const uint8_t *hop, int64_t R, int64_t N, int64_t ld_hop, const float *T,
-                                            int table_per_row, int32_t nbins, int32_t Cr, const float *rscale,
-                                            const float *S, int32_t C, float *out, float *Bsum, gnan_stream_t stream)
+// CUDA-core path of gnan_aggregate_rows_fwd_ws (agg_tc.cu), with optional Bsum save
+int gnan_agg_rows_fwd_cuda_cores(const uint8_t *hop, int64_t R, int64_t N, int64_t ld_hop, const float *T, int table_per_row,
+                                 int32_t nbins, int32_t Cr, const float *rscale, const float *S, int32_t C, float *out, float *Bsum,
+                                 gnan_stream_t stream)
 {
     int rc = check_agg("aggregate_rows_fwd", hop, R, N, ld_hop, T, nbins, Cr, S, C);
     if (rc) return rc;
@@ -616,14 +616,7 @@ extern "C" int gnan_aggregate_rows_fwd_save(const uint8_t *hop, int64_t R, int64
     return GNAN_OK;
 }
 
-extern "C" int gnan_aggregate_rows_fwd(const uint8_t *hop, int64_t R, int64_t N, int64_t ld_hop, const float *T,
-                                       int table_per_row, int32_t nbins, int32_t Cr, const float *rscale, const float *S,
-                                       int32_t C, float *out, gnan_stream_t stream)
-{
-    return gnan_aggregate_rows_fwd_save(hop, R, N, ld_hop, T, table_per_row, nbins, Cr, rscale, S, C, out, nullptr, stream);
-}
-
-extern "C" size_t gnan_aggregate_rows_bwd_workspace_bytes(int64_t R, int64_t N, int32_t nbins, int32_t Cr, int32_t C)
+size_t gnan_agg_rows_bwd_cuda_cores_bytes(int64_t R, int64_t N, int32_t nbins, int32_t C)
 {
     if (R <= 0 || N <= 0) return 0;
     const DsPlan p = plan_ds(R, N);
@@ -631,11 +624,12 @@ extern "C" size_t gnan_aggregate_rows_bwd_workspace_bytes(int64_t R, int64_t N, 
     return sizeof(float) * ((size_t)p.nsb * N * C + (size_t)R * nbins * C);
 }
 
-// backward given saved Bsum (may be NULL -> recomputed into the workspace with one extra pass)
-extern "C" int gnan_aggregate_rows_bwd_saved(const uint8_t *hop, int64_t R, int64_t N, int64_t ld_hop, const float *T,
-                                             int table_per_row, int32_t nbins, int32_t Cr, const float *rscale,
-                                             const float *S, int32_t C, const float *g, const float *Bsum, float *dS,
-                                             float *dT, void *workspace, size_t workspace_bytes, gnan_stream_t stream)
+// CUDA-core path of gnan_aggregate_rows_bwd_ws (agg_tc.cu), given saved Bsum (may be NULL -> recomputed into the workspace with
+// one extra pass)
+int gnan_agg_rows_bwd_cuda_cores(const uint8_t *hop, int64_t R, int64_t N, int64_t ld_hop, const float *T, int table_per_row,
+                                 int32_t nbins, int32_t Cr, const float *rscale, const float *S, int32_t C, const float *g,
+                                 const float *Bsum, float *dS, float *dT, void *workspace, size_t workspace_bytes,
+                                 gnan_stream_t stream)
 {
     int rc = check_agg("aggregate_rows_bwd", hop, R, N, ld_hop, T, nbins, Cr, S, C);
     if (rc) return rc;
@@ -660,7 +654,7 @@ extern "C" int gnan_aggregate_rows_bwd_saved(const uint8_t *hop, int64_t R, int6
         const float *bs = Bsum;
         if (!bs) {  // one extra pass to rebuild the bin sums; its `out` lands in the (not yet used) dS partial area
             float *tmp_bs = dSpart + (size_t)p.nsb * N * C;
-            rc = gnan_aggregate_rows_fwd_save(hop, R, N, ld_hop, T, table_per_row, nbins, Cr, rscale, S, C, dSpart, tmp_bs, stream);
+            rc = gnan_agg_rows_fwd_cuda_cores(hop, R, N, ld_hop, T, table_per_row, nbins, Cr, rscale, S, C, dSpart, tmp_bs, stream);
             if (rc) return rc;
             bs = tmp_bs;
         }
@@ -689,15 +683,6 @@ extern "C" int gnan_aggregate_rows_bwd_saved(const uint8_t *hop, int64_t R, int6
         }
     }
     return GNAN_OK;
-}
-
-extern "C" int gnan_aggregate_rows_bwd(const uint8_t *hop, int64_t R, int64_t N, int64_t ld_hop, const float *T,
-                                       int table_per_row, int32_t nbins, int32_t Cr, const float *rscale, const float *S,
-                                       int32_t C, const float *g, float *dS, float *dT, void *workspace,
-                                       size_t workspace_bytes, gnan_stream_t stream)
-{
-    return gnan_aggregate_rows_bwd_saved(hop, R, N, ld_hop, T, table_per_row, nbins, Cr, rscale, S, C, g, nullptr, dS, dT,
-                                         workspace, workspace_bytes, stream);
 }
 
 static int check_bd(const char *who, const uint8_t *hop, const int64_t *hop_off, const int32_t *node_off, int B, const float *T,

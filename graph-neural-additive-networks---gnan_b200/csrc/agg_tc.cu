@@ -782,18 +782,28 @@ inline int fwd_lanes_per_row(int nbins, int NP)
     return (NP >= 64 && even < 16) ? even : 16;
 }
 
+// true when the tensor-core path covers the shape (nbins <= 32, accumulator columns <= 256, a matrix worth a TMA pipeline)
+bool tc_supported(int64_t R, int64_t N, int64_t ld_hop, int32_t nbins, int32_t C)
+{
+    if (R < 1 || N < 256 || ld_hop < TCOLS || nbins < 2 || nbins > 32 || C < 1) return false;
+    return digit_plan(C).NP <= 256;
+}
+
 }  // namespace
 
-// 1 when the tensor-core path covers the shape (nbins <= 32, accumulator columns <= 256, a matrix worth a TMA pipeline)
-extern "C" int gnan_aggregate_rows_tc_supported(int64_t R, int64_t N, int64_t ld_hop, int32_t nbins, int32_t C)
-{
-    if (R < 1 || N < 256 || ld_hop < TCOLS || nbins < 2 || nbins > 32 || C < 1) return 0;
-    return digit_plan(C).NP <= 256 ? 1 : 0;
-}
+// CUDA-core path (agg.cu)
+int gnan_agg_rows_fwd_cuda_cores(const uint8_t *hop, int64_t R, int64_t N, int64_t ld_hop, const float *T, int table_per_row,
+                                 int32_t nbins, int32_t Cr, const float *rscale, const float *S, int32_t C, float *out, float *Bsum,
+                                 gnan_stream_t stream);
+size_t gnan_agg_rows_bwd_cuda_cores_bytes(int64_t R, int64_t N, int32_t nbins, int32_t C);
+int gnan_agg_rows_bwd_cuda_cores(const uint8_t *hop, int64_t R, int64_t N, int64_t ld_hop, const float *T, int table_per_row,
+                                 int32_t nbins, int32_t Cr, const float *rscale, const float *S, int32_t C, const float *g,
+                                 const float *Bsum, float *dS, float *dT, void *workspace, size_t workspace_bytes,
+                                 gnan_stream_t stream);
 
 extern "C" size_t gnan_aggregate_rows_fwd_workspace_bytes(int64_t R, int64_t N, int64_t ld_hop, int32_t nbins, int32_t C)
 {
-    if (!gnan_aggregate_rows_tc_supported(R, N, ld_hop, nbins, C)) return 0;
+    if (!tc_supported(R, N, ld_hop, nbins, C)) return 0;
     return fwd_ws_layout(nullptr, N, C).total;
 }
 
@@ -802,11 +812,11 @@ extern "C" int gnan_aggregate_rows_fwd_ws(const uint8_t *hop, int64_t R, int64_t
                                           int32_t C, float *out, float *Bsum, int algo, void *workspace, size_t workspace_bytes,
                                           gnan_stream_t stream)
 {
-    const bool can_tc = gnan_aggregate_rows_tc_supported(R, N, ld_hop, nbins, C) != 0;
+    const bool can_tc = tc_supported(R, N, ld_hop, nbins, C);
     // auto: with a single channel the CUDA-core bin sums stream the hop bytes faster (measured 1.6 TB/s vs 1.0 TB/s at the
     // ogbn-arxiv shape); from two channels on they re-stream per channel chunk and the tensor-core pass wins
     if (algo == GNAN_AGG_CUDA_CORES || (algo == GNAN_AGG_AUTO && (!can_tc || C < 2)))
-        return gnan_aggregate_rows_fwd_save(hop, R, N, ld_hop, T, table_per_row, nbins, Cr, rscale, S, C, out, Bsum, stream);
+        return gnan_agg_rows_fwd_cuda_cores(hop, R, N, ld_hop, T, table_per_row, nbins, Cr, rscale, S, C, out, Bsum, stream);
     GNAN_REQUIRE(algo == GNAN_AGG_AUTO || algo == GNAN_AGG_TENSOR_CORES, "aggregate_rows_fwd_ws: unknown algo %d", algo);
     if (!can_tc) {
         gnan_set_error("aggregate_rows_fwd_ws: the tensor-core path needs N >= 256, nbins <= 32 and <= 256 accumulator columns "
@@ -924,8 +934,8 @@ int launch_ds_nb(const DsTcArgs &a, const BwdPlan &p, cudaStream_t st)
 
 extern "C" size_t gnan_aggregate_rows_bwd_ws_bytes(int64_t R, int64_t N, int64_t ld_hop, int32_t nbins, int32_t Cr, int32_t C, int algo)
 {
-    const size_t legacy = gnan_aggregate_rows_bwd_workspace_bytes(R, N, nbins, Cr, C);
-    if (algo == GNAN_AGG_CUDA_CORES || !gnan_aggregate_rows_tc_supported(R, N, ld_hop, nbins, C)) return legacy;
+    if (algo == GNAN_AGG_CUDA_CORES || !tc_supported(R, N, ld_hop, nbins, C))
+        return gnan_agg_rows_bwd_cuda_cores_bytes(R, N, nbins, C);
     const BwdPlan p = bwd_plan(R, N, nbins, C);
     return bwd_ws_layout(nullptr, R, N, C, p).total;       // dT needs no workspace when the bin sums were saved
 }
@@ -935,10 +945,10 @@ extern "C" int gnan_aggregate_rows_bwd_ws(const uint8_t *hop, int64_t R, int64_t
                                           int32_t C, const float *g, const float *Bsum, float *dS, float *dT, int algo,
                                           void *workspace, size_t workspace_bytes, gnan_stream_t stream)
 {
-    const bool can_tc = gnan_aggregate_rows_tc_supported(R, N, ld_hop, nbins, C) != 0 && Bsum != nullptr;
+    const bool can_tc = tc_supported(R, N, ld_hop, nbins, C) && Bsum != nullptr;
     if (algo == GNAN_AGG_CUDA_CORES || (algo == GNAN_AGG_AUTO && !can_tc))
-        return gnan_aggregate_rows_bwd_saved(hop, R, N, ld_hop, T, table_per_row, nbins, Cr, rscale, S, C, g, Bsum, dS, dT, workspace,
-                                             workspace_bytes, stream);
+        return gnan_agg_rows_bwd_cuda_cores(hop, R, N, ld_hop, T, table_per_row, nbins, Cr, rscale, S, C, g, Bsum, dS, dT, workspace,
+                                            workspace_bytes, stream);
     GNAN_REQUIRE(algo == GNAN_AGG_AUTO || algo == GNAN_AGG_TENSOR_CORES, "aggregate_rows_bwd_ws: unknown algo %d", algo);
     if (!can_tc) {
         gnan_set_error("aggregate_rows_bwd_ws: the tensor-core path needs saved bin sums, N >= 256, nbins <= 32 and <= 256 accumulator "
@@ -950,7 +960,7 @@ extern "C" int gnan_aggregate_rows_bwd_ws(const uint8_t *hop, int64_t R, int64_t
     GNAN_REQUIRE(R < (int64_t)1 << 31, "aggregate_rows_bwd_ws: too many rows");
     cudaStream_t st = (cudaStream_t)stream;
     if (dT) {   // from the saved bin sums, no pass over the hop block (the CUDA-core helper with dS = NULL)
-        int rc = gnan_aggregate_rows_bwd_saved(hop, R, N, ld_hop, T, table_per_row, nbins, Cr, rscale, S, C, g, Bsum, nullptr, dT, nullptr, 0, stream);
+        int rc = gnan_agg_rows_bwd_cuda_cores(hop, R, N, ld_hop, T, table_per_row, nbins, Cr, rscale, S, C, g, Bsum, nullptr, dT, nullptr, 0, stream);
         if (rc) return rc;
     }
     if (!dS) return GNAN_OK;

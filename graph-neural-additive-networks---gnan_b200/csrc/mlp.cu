@@ -1060,12 +1060,6 @@ extern "C" size_t gnan_mlp_entries_workspace_bytes(int64_t max_group_entries, co
     return pl.nchunk > 1 ? sizeof(float) * (size_t)pl.nchunk * grad_floats(p) : 0;
 }
 
-extern "C" int gnan_mlp_entries_fwd(const float *val, const int64_t *grp_ptr, int64_t E, const int32_t *items, int64_t n_items,
-                                    const gnan_mlp_params *p, float *Y, gnan_stream_t stream)
-{
-    return gnan_mlp_entries_fwd_ex(val, grp_ptr, E, items, n_items, p, GNAN_PREC_FP32, Y, stream);
-}
-
 extern "C" int gnan_mlp_entries_fwd_ex(const float *val, const int64_t *grp_ptr, int64_t E, const int32_t *items, int64_t n_items,
                                        const gnan_mlp_params *p, int precision, float *Y, gnan_stream_t stream)
 {
@@ -1102,8 +1096,7 @@ extern "C" int gnan_mlp_entries_bwd(const float *val, const int64_t *grp_ptr, in
     GNAN_REQUIRE(grads->du == nullptr, "mlp_entries_bwd: input gradients are not available in entries mode");
     GNAN_REQUIRE(max_group_entries >= 0 && max_group_entries <= E, "mlp_entries_bwd: bad max_group_entries");
     cudaStream_t st = (cudaStream_t)stream;
-    static const bool no_small = getenv("GNAN_NO_SMALL_GROUPS") != nullptr;
-    if (E > 0 && p->H == SG_H && p->n_layers == 3 && p->C <= SG_C && E <= (int64_t)SG_AVG_MAX * p->G && max_group_entries <= SG_GROUP_MAX && !no_small) {
+    if (E > 0 && p->H == SG_H && p->n_layers == 3 && p->C <= SG_C && E <= (int64_t)SG_AVG_MAX * p->G && max_group_entries <= SG_GROUP_MAX) {
         // few rows per feature (bag-of-words columns): a CTA per feature on the CUDA cores, fp32 (both precision modes)
         MlpKArgs a = make_args(val, E, 1, p, 0.f, 0);
         a.grp_ptr = grp_ptr;

@@ -14,7 +14,6 @@
 // Two producer warps stage the next feature's W2 split + small vectors into a double-buffered shared-memory slot while the
 // current feature is consumed; the two row groups alternate so one group's CUDA-core work overlaps the other's MMAs.
 #include <algorithm>
-#include <cstdlib>
 
 #include "common.cuh"
 #include "tc_ptx.cuh"
@@ -68,7 +67,6 @@ struct TcArgs {
     uint64_t seed;
     const uint64_t *seed_dev;   // optional device-resident seed word XORed into `seed` at kernel start (CUDA-graph replays)
     int single_pass;  // 1 = plain tf32 (no lo terms)
-    int prof;         // debug: bit 0 = accumulate phase cycle counters (GNAN_TC_PROF), bit 1 = skip MMA3 (GNAN_TC_SKIP3)
     const int64_t *grp_ptr;   // backward, entries mode (gnan_mlp_entries_bwd): rows of group g = its entries; NULL = dense
     // backward over a channel slice [c_off, c_off + C) of Ctot channels (C > 8 runs as ceil(C/8) passes whose gradients add up:
     // everything downstream of dh = sum_c g_c wo_c is linear in g); chunk_off = first partial-gradient slot of the pass
@@ -623,17 +621,6 @@ template <> struct TmemIO<16> {
 
 struct TcGradPtrs { float *w1, *b1, *wh, *bh, *wo, *bo; size_t chunk_stride; };
 
-// phase cycle counters of the backward kernel (debug aid, read with gnan_debug_tc_prof): summed over the tiles of CTA (0,0)
-__device__ long long g_tc_prof[16];
-#ifdef GNAN_TC_PROFILE   // build with -DGNAN_TC_PROFILE and run with GNAN_TC_PROF=1 (costs ~40 registers: not in the default build)
-#define TC_PROF(slot)                                                     \
-    do {                                                                  \
-        if (prof_on) { const long long now_ = clock64(); pacc[slot] += now_ - tprev; tprev = now_; } \
-    } while (0)
-#else
-#define TC_PROF(slot) do { } while (0)
-#endif
-
 template <int CT, bool DROP, bool EXT = false>
 __global__ void __launch_bounds__(BWD_THREADS, 1)   // 17 warps occupy 20 warp slots (5 per scheduler): 96 registers is the cap
 mlp_tc_bwd_kernel(TcArgs a, const float *__restrict__ dS, TcGradPtrs gp, int64_t ntiles)
@@ -760,13 +747,11 @@ mlp_tc_bwd_kernel(TcArgs a, const float *__restrict__ dS, TcGradPtrs gp, int64_t
             if (lane == 0) {
                 // dW2 accumulation over the 128 rows of the tile: A = sZ (M = 128: hi|lo), B = sH hi then lo
                 const uint32_t za = smem_u32(sm.sZ), hh = smem_u32(sm.sH_hi), hl = smem_u32(sm.sH_lo);
-                if (!(a.prof & 2)) {     // GNAN_TC_SKIP3: timing experiment only (dW2 is wrong)
 #pragma unroll 4
                 for (int ks = 0; ks < 16; ++ks)
                     umma_tf32_ss(tmem + colD3, umma_desc_kmajor(za + ks * T_KSTEP, T_LBO, T_SBO),
                                  umma_desc_kmajor(hh + ks * T_KSTEP, T_LBO, T_SBO), idesc, (it > 0 || ks > 0) ? 1u : 0u);
-                }
-                if (!a.single_pass && !(a.prof & 2)) {
+                if (!a.single_pass) {
 #pragma unroll 4
                     for (int ks = 0; ks < 16; ++ks)
                         umma_tf32_ss(tmem + colD3, umma_desc_kmajor(za + ks * T_KSTEP, T_LBO, T_SBO),
@@ -787,13 +772,6 @@ mlp_tc_bwd_kernel(TcArgs a, const float *__restrict__ dS, TcGradPtrs gp, int64_t
 #pragma unroll
         for (int c = 0; c < CT; ++c) acc_wo[c] = 0.f;
         float p_b2 = 0.f, p_b1 = 0.f, p_w1 = 0.f;          // column (c0 + (lane & (NC-1))) sums over this warp's rows
-#ifdef GNAN_TC_PROFILE
-        const bool prof_on = (a.prof & 1) && tid == 0 && blockIdx.x == 0 && blockIdx.y == 0;
-        long long tprev = clock64();
-        long long pacc[16];                                // register-resident phase counters (static indices only)
-#pragma unroll
-        for (int i = 0; i < 16; ++i) pacc[i] = 0;
-#endif
         uint32_t it = 0;
         // x and dS of the next tile are fetched one tile ahead (their ~700-cycle latency was exposed in the gen phase)
         float x_n = 0.f, gv_n[CT];
@@ -841,7 +819,6 @@ mlp_tc_bwd_kernel(TcArgs a, const float *__restrict__ dS, TcGradPtrs gp, int64_t
 
         for (int64_t t = blockIdx.x; t < ntiles; t += gridDim.x, ++it) {
             const uint32_t ph = it & 1;
-            TC_PROF(7);
             const int64_t row = t * ROWS + r;
             const float x = x_n;
             const int64_t tn = t + gridDim.x, rown = tn * ROWS + r;
@@ -864,7 +841,6 @@ mlp_tc_bwd_kernel(TcArgs a, const float *__restrict__ dS, TcGradPtrs gp, int64_t
                     if (okn && c < a.C) gv_n[c] = ldg_prefetch(dS + rown * a.Ctot + c);
                 }
             }
-            TC_PROF(9);
             // ---- [A] gen: a0 for units c0..c0+NC-1 -> TMEM only (the A operand of MMA1); then release the tensor core
             uint32_t hi[NC], lo[NC];
 #pragma unroll
@@ -879,15 +855,11 @@ mlp_tc_bwd_kernel(TcArgs a, const float *__restrict__ dS, TcGradPtrs gp, int64_t
                     split_tf32(v[e], hi[i4 * 4 + e], lo[i4 * 4 + e]);
                 }
             }
-            TC_PROF(10);
             IO::st(lane_base + colA_hi + c0, hi);
             if (!a.single_pass) IO::st(lane_base + colA_lo + c0, lo);
-            TC_PROF(11);
             tmem_wait_st();
-            TC_PROF(12);
             tc_fence_before();
             mbar_arrive(smem_u32(&sm.a1_full));
-            TC_PROF(0);
             // ---- [B] under this tile's MMA1: once MMA3 of the previous tile is done (its smem operands are free) stage a0^T
             //          (B operand of this tile's MMA3; hi/lo die here), then run the previous tile's dWo phase
             if (it > 0) {
@@ -900,7 +872,6 @@ mlp_tc_bwd_kernel(TcArgs a, const float *__restrict__ dS, TcGradPtrs gp, int64_t
                 sm.sH_lo[tidx(c0 + i, r)] = __uint_as_float(lo[i]);
             }
             if (!EXT && it > 0) dwo_phase(t - gridDim.x, ph ^ 1);
-            TC_PROF(6);
             // ---- [D] epiC
             uint32_t dhv[NC];
             if (EXT) {                                         // dh of this (row, feature) straight from the caller's GEMM; the loads
@@ -914,7 +885,6 @@ mlp_tc_bwd_kernel(TcArgs a, const float *__restrict__ dS, TcGradPtrs gp, int64_t
             }
             mbar_wait(smem_u32(&sm.d1_full), ph);
             tc_fence_after();
-            TC_PROF(1);
             {
                 uint32_t d[NC];
                 IO::ld(lane_base + (ph ? colD1b : colD1) + c0, d);
@@ -957,11 +927,9 @@ mlp_tc_bwd_kernel(TcArgs a, const float *__restrict__ dS, TcGradPtrs gp, int64_t
                 mbar_arrive(smem_u32(&sm.a3_full));                  // MMA3 may start (after MMA2 in issue order)
                 p_b2 += warp_colsum<NC>(dz, lane);
             }
-            TC_PROF(2);
             // ---- [E] epiF
             mbar_wait(smem_u32(&sm.d2_full), ph);
             tc_fence_after();
-            TC_PROF(3);
             {
                 uint32_t d[NC];
                 IO::ld(lane_base + colD2 + c0, d);
@@ -984,17 +952,7 @@ mlp_tc_bwd_kernel(TcArgs a, const float *__restrict__ dS, TcGradPtrs gp, int64_t
                 p_b1 += warp_colsum<NC>(z0, lane);
                 p_w1 += warp_colsum<NC>(z1, lane);
             }
-            TC_PROF(4);
-#ifdef GNAN_TC_PROFILE
-            if (prof_on) pacc[8] += 1;
-#endif
         }
-#ifdef GNAN_TC_PROFILE
-        if (prof_on) {
-#pragma unroll
-            for (int i = 0; i < 16; ++i) g_tc_prof[i] += pacc[i];
-        }
-#endif
         // the last tile's dWo phase
         if (it > 0) {
             const int64_t tl = (int64_t)blockIdx.x + (int64_t)(it - 1) * gridDim.x;
@@ -1137,7 +1095,6 @@ TcArgs make_tc_args(const float *u, int64_t R, int64_t ldu, const gnan_mlp_param
     a.seed = seed;
     a.seed_dev = nullptr;
     a.single_pass = precision == GNAN_PREC_TF32;
-    a.prof = (getenv("GNAN_TC_PROF") != nullptr ? 1 : 0) | (getenv("GNAN_TC_SKIP3") != nullptr ? 2 : 0);
     a.grp_ptr = nullptr;
     a.Ctot = p->C; a.c_off = 0; a.chunk_off = 0;
     a.dh_ext = nullptr; a.a1_ext = nullptr;
@@ -1346,16 +1303,5 @@ int gnan_mlp_tc_bwd_ex(const float *u, int64_t R, int64_t ldu, const gnan_mlp_pa
         else dbo_colsum_kernel<<<(unsigned)C, 256, 0, st>>>(dS, R, (int)C, (int)G, grads->bo);
         GNAN_LAUNCH_OK();
     }
-    return GNAN_OK;
-}
-
-// debug aid: read (and clear) the backward kernel's phase cycle counters; slots: 0 gen, 1 wait MMA1, 2 epiC, 3 wait MMA2,
-// 4 epiF, 5 wait MMA3, 6 dWo, 7 loop overhead, 8 tiles
-extern "C" int gnan_debug_tc_prof(long long *out_host16)
-{
-    GNAN_CUDA(cudaDeviceSynchronize());
-    GNAN_CUDA(cudaMemcpyFromSymbol(out_host16, g_tc_prof, sizeof(long long) * 16));
-    long long zero[16] = {0};
-    GNAN_CUDA(cudaMemcpyToSymbol(g_tc_prof, zero, sizeof(zero)));
     return GNAN_OK;
 }

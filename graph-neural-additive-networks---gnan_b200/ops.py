@@ -254,7 +254,7 @@ def agg_rows_fwd(hop: Tensor, T: Tensor, rscale: Optional[Tensor], S: Tensor, pe
     with _timed("aggregate_rows_fwd_save"):
         check(lib.gnan_aggregate_rows_fwd_ws(ptr(hop), R, N, ld, ptr(T), int(per_row), nbins, Cr, ptr(rscale), ptr(S), C,
                                              ptr(out), ptr(bsum), int(algo), ptr(ws) if nws else None, nws, stream_handle()),
-              "gnan_aggregate_rows_fwd")
+              "gnan_aggregate_rows_fwd_ws")
     return out, bsum
 
 
@@ -279,7 +279,7 @@ def agg_rows_bwd(hop: Tensor, T: Tensor, rscale: Optional[Tensor], S: Tensor, pe
     with _timed("aggregate_rows_bwd_saved"):
         check(lib.gnan_aggregate_rows_bwd_ws(ptr(hop), R, N, ld, ptr(T), int(per_row), nbins, Cr, ptr(rscale), ptr(S), C,
                                              ptr(g), ptr(bsum) if bsum.numel() else None, ptr(dS), ptr(dT), int(algo), ptr(ws),
-                                             ws.numel(), stream_handle()), "gnan_aggregate_rows_bwd")
+                                             ws.numel(), stream_handle()), "gnan_aggregate_rows_bwd_ws")
     return dS, dT
 
 

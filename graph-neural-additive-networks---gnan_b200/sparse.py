@@ -18,7 +18,7 @@ column's most frequent value) plus the list of exceptions (row, value) that diff
 
     S[r,:] = sum_k Y[base_k,:] + sum_{e in exceptions(r)} (Y[e,:] - Y[base_k(e),:]),     Y[e,:] = f_k(e)(val[e])
 
-The C ABI side is gnan_mlp_entries_fwd/bwd + gnan_entries_to_rows / gnan_rows_to_entries (include/gnan_b200.h); all fp32
+The C ABI side is gnan_mlp_entries_fwd_ex/bwd + gnan_entries_to_rows / gnan_rows_to_entries (include/gnan_b200.h); all fp32
 kernels, deterministic. With dropout active the modules fall back to the dense kernels (per-row masks break the sharing).
 """
 from typing import Optional

@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define GNAN_B200_VERSION 101
+#define GNAN_B200_VERSION 102
 
 enum {
     GNAN_OK = 0,
@@ -113,14 +113,12 @@ int gnan_mlp_bwd_ext(const float *u, int64_t R, int64_t ldu, const gnan_mlp_para
  * The caller lists the distinct work as val[E] grouped by feature, group g owning entries [grp_ptr[g], grp_ptr[g+1]);
  * Y[e,:] = f_g(val[e]) and the weight gradients given dY[E,C] come back; how entries map to rows of S is the caller's
  * business (gnan_b200/sparse.py). items [n_items,2] = (group, 128-entry tile index inside the group): one CTA per item.
- * Forward: fp32 kernels (gnan_mlp_entries_fwd) or, with `precision` (gnan_mlp_entries_fwd_ex), the tcgen05 kernel for
- * H = 64, 3 layers, C <= 8; backward: fp32 or the tcgen05 kernel (`precision`), or — H = 64, 3 layers, C <= 8, at most 96 entries per
- * feature on average and 3 072 in any one — a CTA per feature on the CUDA cores in fp32 under either `precision` (bag-of-words columns:
- * a few dozen entries per feature, where a tensor-core tile would be a quarter full); n_layers >= 2; no dropout (the sharing would
- * be wrong with per-row masks). */
+ * Forward: fp32 kernels or, with `precision` != GNAN_PREC_FP32, the tcgen05 kernel for H = 64, 3 layers, C <= 8; backward: fp32
+ * or the tcgen05 kernel (`precision`), or — H = 64, 3 layers, C <= 8, at most 96 entries per feature on average and 3 072 in any
+ * one — a CTA per feature on the CUDA cores in fp32 under either `precision` (bag-of-words columns: a few dozen entries per
+ * feature, where a tensor-core tile would be a quarter full); n_layers >= 2; no dropout (the sharing would be wrong with per-row
+ * masks). */
 size_t gnan_mlp_entries_workspace_bytes(int64_t max_group_entries, const gnan_mlp_params *p, int backward, int precision);
-int gnan_mlp_entries_fwd(const float *val, const int64_t *grp_ptr /* [G+1] */, int64_t E, const int32_t *items, int64_t n_items,
-                         const gnan_mlp_params *p, float *Y /* [E,C] */, gnan_stream_t stream);
 int gnan_mlp_entries_fwd_ex(const float *val, const int64_t *grp_ptr /* [G+1] */, int64_t E, const int32_t *items, int64_t n_items,
                             const gnan_mlp_params *p, int precision, float *Y /* [E,C] */, gnan_stream_t stream);
 int gnan_mlp_entries_bwd(const float *val, const int64_t *grp_ptr, int64_t E, int64_t max_group_entries,
@@ -164,63 +162,46 @@ int gnan_level_rscale(const int32_t *cnt, int64_t rows, int32_t nbins, float *rs
  * b(h) = h for h <= nbins-2, nbins-1 for h == 255.  c' = c if Cr == C else 0 (Cr == 1: shared rho).
  * table_per_row: T is [R,nbins,Cr] (input-normalised rho, GNAN.py:65-67) else [nbins,Cr]; rscale may be NULL.
  * Replaces GNAN.py:67-73,159-170 and models.py:366-375 (the N*N rho evaluation, permutes, bmm and sums).
- * ---------------------------------------------------------------------------------------------- */
-int gnan_aggregate_rows_fwd(const uint8_t *hop, int64_t R, int64_t N, int64_t ld_hop, const float *T,
-                            int table_per_row, int32_t nbins, int32_t Cr, const float *rscale, const float *S,
-                            int32_t C, float *out /* [R,C] */, gnan_stream_t stream);
-
-/* training-mode forward: additionally saves the per-row bin sums Bsum[i,d,c] = sum_{j: b(hop[i,j]) = d} S[j,c]
- * ([R,nbins,C]; NULL = do not save) that the backward turns into dT without another pass over the hop block. */
-int gnan_aggregate_rows_fwd_save(const uint8_t *hop, int64_t R, int64_t N, int64_t ld_hop, const float *T,
-                                 int table_per_row, int32_t nbins, int32_t Cr, const float *rscale, const float *S,
-                                 int32_t C, float *out, float *Bsum, gnan_stream_t stream);
-
-/* ------------------------------------------------------------------------------------------------
- * Tensor-core form of the same aggregation (csrc/agg_tc.cu): the reference's matmul(m_dist_perm, fx_perm) (GNAN.py:70,
- * models.py:371-372) as Bsum[(i,d), c] = sum_j 1[b(hop[i,j]) = d] * S[j,c] on tcgen05 (kind::i8, int32 accumulation in
- * TMEM), the hop tiles streamed ONCE for all C channels by TMA and the 0/1 operand generated on the fly. S is quantised per
- * channel to 3-4 signed 8-bit digits of a common power-of-two scale (absolute error <= 2^-23 / 2^-31 of the column's largest
- * magnitude); the bin sums are exact integer sums of the quantised values (order-independent, deterministic), rounded to
- * fp32 once. Covers nbins <= 32 and <= 256 accumulator columns; `algo` selects the kernel family.
+ * Both directions go through the per-row bin sums Bsum[i,d,c] = sum_{j: b(hop[i,j]) = d} S[j,c] ([R,nbins,C]).
+ *
+ * Two kernel families, selected by `algo`:
+ *  - CUDA cores (csrc/agg.cu): fp32 bin sums;
+ *  - tensor cores (csrc/agg_tc.cu): the reference's matmul(m_dist_perm, fx_perm) (GNAN.py:70, models.py:371-372) as
+ *    Bsum[(i,d), c] = sum_j 1[b(hop[i,j]) = d] * S[j,c] on tcgen05 (kind::i8, int32 accumulation in TMEM), the hop tiles
+ *    streamed ONCE for all C channels by TMA and the 0/1 operand generated on the fly. S is quantised per channel to 3-4 signed
+ *    8-bit digits of a common power-of-two scale (absolute error <= 2^-23 / 2^-31 of the column's largest magnitude); the bin
+ *    sums are exact integer sums of the quantised values (order-independent, deterministic), rounded to fp32 once. Covers
+ *    N >= 256, nbins <= 32 and <= 256 accumulator columns (C <= 80).
  * ---------------------------------------------------------------------------------------------- */
 enum {
     GNAN_AGG_AUTO = 0,         /* tensor cores where the shape is covered, CUDA cores otherwise */
-    GNAN_AGG_CUDA_CORES = 1,   /* the fp32 bin-sum kernels of gnan_aggregate_rows_fwd_save / _bwd_saved */
+    GNAN_AGG_CUDA_CORES = 1,   /* the fp32 bin-sum kernels of csrc/agg.cu (the forward needs no workspace) */
     GNAN_AGG_TENSOR_CORES = 2  /* fail with GNAN_ERR_UNSUPPORTED when the shape is not covered */
 };
-int gnan_aggregate_rows_tc_supported(int64_t R, int64_t N, int64_t ld_hop, int32_t nbins, int32_t C);
+
+/* forward: out [R,C], and Bsum when it is not NULL (the training-mode forward saves it: the backward turns it into dT without
+ * another pass over the hop block). The workspace holds the digit matrix of S for the tensor-core path:
+ * gnan_aggregate_rows_fwd_workspace_bytes is 0 when that path does not cover the shape, and the CUDA-core path needs none. */
 size_t gnan_aggregate_rows_fwd_workspace_bytes(int64_t R, int64_t N, int64_t ld_hop, int32_t nbins, int32_t C);
-/* gnan_aggregate_rows_fwd_save with a kernel choice and a workspace (digit matrix of S; 0 bytes = CUDA-core path only) */
 int gnan_aggregate_rows_fwd_ws(const uint8_t *hop, int64_t R, int64_t N, int64_t ld_hop, const float *T, int table_per_row,
                                int32_t nbins, int32_t Cr, const float *rscale, const float *S, int32_t C, float *out,
                                float *Bsum /* or NULL */, int algo, void *workspace, size_t workspace_bytes,
                                gnan_stream_t stream);
 
-/* backward with a kernel choice. Tensor-core path (needs the saved Bsum): dT from the bin sums; dS[j,c] = sum_{i,d}
- * 1[b(hop[i,j]) = d] * TG[i,d,c] with TG = T*rscale*g quantised like S above, contracted on tcgen05 with a TMEM lane per hop
- * COLUMN. Rows whose g is entirely zero are skipped (their contribution is exactly zero): the hop bytes streamed are those of
- * the rows that carry a loss (a train mask: trainer.py:52-58). */
+/* backward, given g = dL/dout [R,C]:
+ *     dS[j,c] = sum_i W[i,j,c] g[i,c]   (overwritten; [N,C]; NULL = not wanted)
+ *     dT (same shape as T; overwritten; NULL = not wanted)  dT[ti,d,c'] = sum_{i in ti} rscale[i,d] * sum_c g[i,c] * Bsum[i,d,c]
+ * Bsum is the one the forward saved. With Bsum == NULL the CUDA-core backward recomputes it with one extra pass over the hop
+ * block; the tensor-core path needs it (AUTO then runs on the CUDA cores: size the workspace with GNAN_AGG_CUDA_CORES).
+ * Tensor-core path: dT from the bin sums; dS[j,c] = sum_{i,d} 1[b(hop[i,j]) = d] * TG[i,d,c] with TG = T*rscale*g quantised
+ * like S above, contracted on tcgen05 with a TMEM lane per hop COLUMN. Rows whose g is entirely zero are skipped (their
+ * contribution is exactly zero): the hop bytes streamed are those of the rows that carry a loss (a train mask:
+ * trainer.py:52-58). Workspace: gnan_aggregate_rows_bwd_ws_bytes with the same `algo`. */
 size_t gnan_aggregate_rows_bwd_ws_bytes(int64_t R, int64_t N, int64_t ld_hop, int32_t nbins, int32_t Cr, int32_t C, int algo);
 int gnan_aggregate_rows_bwd_ws(const uint8_t *hop, int64_t R, int64_t N, int64_t ld_hop, const float *T, int table_per_row,
                                int32_t nbins, int32_t Cr, const float *rscale, const float *S, int32_t C, const float *g,
                                const float *Bsum, float *dS, float *dT, int algo, void *workspace, size_t workspace_bytes,
                                gnan_stream_t stream);
-
-size_t gnan_aggregate_rows_bwd_workspace_bytes(int64_t R, int64_t N, int32_t nbins, int32_t Cr, int32_t C);
-
-/* given g = dL/dout [R,C]:  dS[j,c] = sum_i W[i,j,c] g[i,c]   (overwritten; [N,C])
- *                            dT (same shape as T; overwritten)  dT[ti,d,c'] = sum_{i in ti} rscale[i,d] * sum_c g[i,c] * Bsum[i,d,c]
- * with Bsum[i,d,c] = sum_{j: b(hop[i,j]) = d} S[j,c]. One pass over the hop block. */
-int gnan_aggregate_rows_bwd(const uint8_t *hop, int64_t R, int64_t N, int64_t ld_hop, const float *T,
-                            int table_per_row, int32_t nbins, int32_t Cr, const float *rscale, const float *S,
-                            int32_t C, const float *g, float *dS, float *dT, void *workspace, size_t workspace_bytes,
-                            gnan_stream_t stream);
-
-/* same, given the Bsum saved by gnan_aggregate_rows_fwd_save (NULL = recompute it, one extra pass) */
-int gnan_aggregate_rows_bwd_saved(const uint8_t *hop, int64_t R, int64_t N, int64_t ld_hop, const float *T,
-                                  int table_per_row, int32_t nbins, int32_t Cr, const float *rscale, const float *S,
-                                  int32_t C, const float *g, const float *Bsum, float *dS, float *dT, void *workspace,
-                                  size_t workspace_bytes, gnan_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Block-diagonal (batched small graphs) aggregation. Graph b owns nodes [node_off[b], node_off[b+1]) and the

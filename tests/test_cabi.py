@@ -1,4 +1,4 @@
-"""CPU: the C-ABI library builds, loads, and exports every symbol include/gnan_b200.h declares (no compute calls)."""
+"""CPU: the C-ABI library builds, loads, and exports exactly the symbols include/gnan_b200.h declares (no compute calls)."""
 import ctypes
 import os
 import re
@@ -31,22 +31,31 @@ def test_header_symbols_exported(lib_path):
         assert hasattr(lib, n), f"{n} declared in gnan_b200.h but not exported"
 
 
-def test_python_binding_covers_header(lib_path):
+def test_exports_are_exactly_the_header_functions(lib_path):
+    """No C entry point outside the header: a caller cannot reach a function the ABI does not document. C++ helpers shared between
+    the library's own files have mangled names (_Z...) and are not C entry points."""
+    import subprocess
+    out = subprocess.run(["nm", "-D", "--defined-only", lib_path], check=True, capture_output=True, text=True).stdout
+    exported = sorted({f[-1] for f in (line.split() for line in out.splitlines()) if f and f[-1].startswith("gnan_")})
+    assert exported == header_functions()
+
+
+def test_python_binding_covers_the_version_102_header(lib_path):
     from gnan_b200 import _lib
     assert sorted(_lib.SIGNATURES) == header_functions()
     lib = _lib.load()
-    assert lib.gnan_version() == 101
+    assert lib.gnan_version() == 102
     assert lib.gnan_last_error() is not None
 
 
-def test_argument_validation_without_gpu(lib_path):
+def test_argument_validation_of_the_surviving_entry_points_without_gpu(lib_path):
     """Validation happens before any CUDA call, so error codes can be checked on a CPU-only box."""
     from gnan_b200 import _lib
     lib = _lib.load()
     p = _lib.MlpParams(3, 24, 2, 3, None, None, None, None, None, None)   # H=24 unsupported, wo NULL
     rc = lib.gnan_mlp_fwd(None, 4, 3, ctypes.byref(p), 0.0, 0, None, 0, None, None, 0, None)
     assert rc == 1 and b"wo" in lib.gnan_last_error()
-    rc = lib.gnan_aggregate_rows_fwd(None, 4, 4, 16, None, 0, 5, 1, None, None, 1, None, None)
+    rc = lib.gnan_aggregate_rows_fwd_ws(None, 4, 4, 16, None, 0, 5, 1, None, None, 1, None, None, 0, None, 0, None)
     assert rc == 1
     arr = (ctypes.c_int64 * 8)()
     buf = ctypes.addressof(arr)
@@ -89,7 +98,7 @@ int main(int argc, char **argv)
 """
 
 
-def test_c99_consumer_compiles_against_the_header_and_calls_the_library(lib_path, tmp_path):
+def test_c99_consumer_compiles_against_the_version_102_header_and_calls_the_library(lib_path, tmp_path):
     import subprocess
     src = tmp_path / "consumer.c"
     src.write_text(C_CONSUMER)
@@ -97,7 +106,7 @@ def test_c99_consumer_compiles_against_the_header_and_calls_the_library(lib_path
     subprocess.run(["gcc", "-std=c99", "-Wall", "-Wextra", "-Werror", "-pedantic", "-I", os.path.join(ROOT, "include"), str(src), "-o", str(exe), "-ldl"],
                    check=True, capture_output=True, text=True)
     out = subprocess.run([str(exe), lib_path], check=True, capture_output=True, text=True).stdout.split(None, 4)
-    assert out[0] == "101" and int(out[1]) != 0 and out[2] == "1" and int(out[3]) >= 0 and "level_rscale" in out[4]
+    assert out[0] == "102" and int(out[1]) != 0 and out[2] == "1" and int(out[3]) >= 0 and "level_rscale" in out[4]
     # and as C++ (the reference-side binding may be either)
     subprocess.run(["g++", "-std=c++11", "-Wall", "-Werror", "-fsyntax-only", "-x", "c++", "-I", os.path.join(ROOT, "include"), str(src)],
                    check=True, capture_output=True, text=True)
