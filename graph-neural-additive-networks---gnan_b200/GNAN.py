@@ -154,19 +154,25 @@ class TensorGNAN(_Base):
         self.fs.xavier_normal_(0.01)
         self.rho.xavier_normal_(0.01)
 
+    def _aggregation(self, src, S):
+        """ops.Aggregation of a resolved HopData or a PackedBatch `src`, for feature sums shaped like S"""
+        dev = self._device()
+        packed = isinstance(src, PackedBatch)
+        kw = dict(hop_off=src.hop_off, node_off=src.node_off, reduce_graph=self.is_graph_task) if packed else {}
+        if self.normalize_rho:                                                       # GNAN.py:65-67: rho(nd / norm)
+            u = ops.rho_table_inputs(src.nbins, dev, cnt=src.level_counts)           # [R,nbins]
+            T = self._row_tables(src, u, src.level_counts).view(S.shape[0] if packed else src.rows, src.nbins, self.out_channels)
+            return ops.Aggregation(T, src.hop, per_row=True, **kw)
+        T = self._table(ops.rho_table_inputs(src.nbins, dev))                        # [nbins,C]
+        return ops.Aggregation(T, src.hop, **kw)
+
     def forward(self, inputs):
         if isinstance(inputs, PackedBatch):
             return self.forward_packed(inputs)
         dev = self._device()
         _, hd = resolve(inputs, dev, need_x=False)
         S = self._feature_sums(*self._features(inputs))                              # [N,C]   GNAN.py:57-62 (+ :73 by linearity)
-        if self.normalize_rho:                                                       # GNAN.py:65-67: rho(nd / norm)
-            u = ops.rho_table_inputs(hd.nbins, dev, cnt=hd.level_counts)             # [R,nbins]
-            T = self._row_tables(hd, u, hd.level_counts).view(hd.rows, hd.nbins, self.out_channels)
-            out = ops.aggregate_rows(hd.hop, T, S, per_row=True)
-        else:
-            T = self._table(ops.rho_table_inputs(hd.nbins, dev))                     # [nbins,C]
-            out = ops.aggregate_rows(hd.hop, T, S)
+        out = self._aggregation(hd, S)(S)
         if self.is_graph_task:
             out = out.sum(dim=0).view(1, -1).T                                        # [C,1]  GNAN.py:76-79
         return out
@@ -179,12 +185,7 @@ class TensorGNAN(_Base):
         if pk.hop.device != dev:
             pk = pk.to(dev)
         S = self._feature_sums(*self._features(pk))
-        if self.normalize_rho:
-            u = ops.rho_table_inputs(pk.nbins, dev, cnt=pk.level_counts)
-            T = self._row_tables(pk, u, pk.level_counts).view(S.shape[0], pk.nbins, self.out_channels)
-            return ops.aggregate_blockdiag(pk.hop, pk.hop_off, pk.node_off, T, S, per_row=True, reduce_graph=self.is_graph_task)
-        T = self._table(ops.rho_table_inputs(pk.nbins, dev))
-        return ops.aggregate_blockdiag(pk.hop, pk.hop_off, pk.node_off, T, S, reduce_graph=self.is_graph_task)
+        return self._aggregation(pk, S)(S)
 
 
 class GNAN(_Base):
@@ -212,14 +213,19 @@ class GNAN(_Base):
             self._register_state_dict_hook(_emit_rhos)
             self.register_load_state_dict_pre_hook(_absorb_rhos)
 
-    def forward(self, inputs, node_ids=None):
+    def _aggregation(self, hd, S=None, node_ids=None):
+        """ops.Aggregation of the rows `node_ids` (all rows when None) of a resolved HopData"""
         dev = self._device()
-        _, hd = resolve(inputs, dev, need_x=False)
-        S = self._feature_sums(*self._features(inputs))                              # f_sums, GNAN.py:150-157
         T = self._table(ops.rho_table_inputs(hd.nbins, dev))                         # [nbins,Cr]  rho(1/(1+d))
         hop, cnt = hd.hop, hd.level_counts
         if node_ids is not None:                                                     # row subset, GNAN.py:146-149
             ids = torch.as_tensor(node_ids, device=dev, dtype=torch.long)
             hop, cnt = hop.index_select(0, ids), cnt.index_select(0, ids)
         rs = ops.level_rscale(cnt) if self.normalize_rho else None                   # GNAN.py:163-168: rho(.) / norm
-        return ops.aggregate_rows(hop, T, S, rscale=rs)                              # [len(node_ids), C]
+        return ops.Aggregation(T, hop, rscale=rs)
+
+    def forward(self, inputs, node_ids=None):
+        dev = self._device()
+        _, hd = resolve(inputs, dev, need_x=False)
+        S = self._feature_sums(*self._features(inputs))                              # f_sums, GNAN.py:150-157
+        return self._aggregation(hd, S, node_ids)(S)                                 # [len(node_ids), C]

@@ -84,6 +84,12 @@ SIGNATURES = {
                                 c_void_p, c_size_t, c_void_p]),
     "gnan_apsp_bfs_batched_ex": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_int32,
                                          c_void_p, c_void_p, c_void_p, c_void_p]),
+    "gnan_explain_segments": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_int32, c_void_p, c_void_p]),
+    "gnan_explain_graph_features": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p,
+                                            c_void_p, c_void_p]),
+    "gnan_explain_rows_features": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_int32, c_int64, c_void_p, c_int64, c_void_p, c_int,
+                                           c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32,
+                                           c_void_p, c_void_p]),
     "gnan_loss_workspace_bytes": (c_size_t, []),
     "gnan_cross_entropy_rows": (c_int, [c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_int64, c_float, c_void_p, c_void_p, c_void_p,
                                         c_void_p, c_size_t, c_void_p]),

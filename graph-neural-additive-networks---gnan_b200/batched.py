@@ -67,11 +67,17 @@ class TensorGNAN(_Base):
         if pk.hop.device != dev:
             pk = pk.to(dev)
         S = self._feature_sums(*self._features(pk))
+        return self._aggregation(pk, S)(S)
+
+    def _aggregation(self, pk, S):
+        """ops.Aggregation of a PackedBatch `pk` on the device, for feature sums shaped like S"""
+        dev = self._device()
         nb = pk.nbins
         p = self.rho.dropout if self.training else 0.0
         keep = torch.ones(nb, 1, device=dev)
         keep[-1] = 0.0                                                                    # masked pairs: :158-159
         u = ops.rho_table_inputs(nb, dev, raw=True)                                       # d = 0..nbins-2
+        kw = dict(hop_off=pk.hop_off, node_off=pk.node_off, reduce_graph=self.is_graph_task)
         if p > 0:
             # The reference runs rho (with its Dropout) on every pair (:125-131,154): an independent mask per pair. A single
             # [nbins] table would share ONE mask between all pairs at the same distance; here every ROW gets its own table
@@ -81,6 +87,6 @@ class TensorGNAN(_Base):
             T = ops.mlp(u.repeat(n_rows).reshape(-1, 1), *self.rho.kernel_args(), dropout_p=p, seed=self._seed(),
                         precision=self.precision, seed_dev=self._seed_word())
             T = (T.view(n_rows, nb, -1) * keep).contiguous()
-            return ops.aggregate_blockdiag(pk.hop, pk.hop_off, pk.node_off, T, S, per_row=True, reduce_graph=self.is_graph_task)
+            return ops.Aggregation(T, pk.hop, per_row=True, **kw)
         T = ops.mlp(u.reshape(-1, 1), *self.rho.kernel_args(), precision=self.precision) * keep
-        return ops.aggregate_blockdiag(pk.hop, pk.hop_off, pk.node_off, T, S, reduce_graph=self.is_graph_task)
+        return ops.Aggregation(T, pk.hop, **kw)

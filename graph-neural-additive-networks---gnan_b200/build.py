@@ -15,7 +15,7 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(CSRC, "_build")
 LIB = os.path.join(HERE, "libgnan_b200.so")
-SOURCES = ["api.cu", "mlp.cu", "mlp_tc.cu", "agg.cu", "agg_tc.cu", "agg_bd.cu", "apsp.cu", "csr.cu", "entries.cu", "train.cu", "wide.cu"]
+SOURCES = ["api.cu", "mlp.cu", "mlp_tc.cu", "agg.cu", "agg_tc.cu", "agg_bd.cu", "apsp.cu", "csr.cu", "entries.cu", "train.cu", "wide.cu", "explain.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
          "-I" + os.path.join(ROOT, "include"), "-Xcompiler", "-fPIC"]

@@ -69,6 +69,23 @@ class TensorGNAN(_Base):
         return ops.mlp_per_group(x, *self.fs.kernel_args(), dropout_p=p, seed=self._seed() if p > 0 else 0,
                                  precision=self.precision, seed_dev=self._seed_word() if p > 0 else None).squeeze(-1)   # [N,K,1] -> [N,K]
 
+    def _aggregation(self, src, S):
+        """ops.Aggregation of a resolved HopData or a PackedBatch `src`, for feature sums shaped like S"""
+        dev = self._device()
+        T = self._table(ops.rho_table_inputs(src.nbins, dev))                        # [nbins,Cr]
+        if not isinstance(src, PackedBatch):
+            rs = ops.level_rscale(src.level_counts) if self.normalize_rho else None  # models.py:368-370
+            return ops.Aggregation(T, src.hop, rscale=rs)
+        if (src.deferred and self.normalize_rho and self.is_graph_task and T.dim() == 2 and ops.BLOCKDIAG_GRAPH_KERNEL
+                and ops.load().gnan_aggregate_blockdiag_graph_supported(T.shape[0], T.shape[1], S.shape[1])):
+            # distances not computed yet (preprocess.apsp_batched on a LocalEdges batch): the BFS and this readout run as one
+            # kernel, neither the hop bytes nor the normaliser table are ever written (models.py:366-384)
+            return ops.Aggregation(T, node_off=src.node_off, reduce_graph=True, fused=(src.edges, src.max_nodes, src.status))
+        rs = None
+        if self.normalize_rho:       # models.py:368-370; a batch straight from apsp_batched(..., rscale=True) carries it already
+            rs = src.level_rscale if getattr(src, "level_rscale", None) is not None else ops.level_rscale(src.level_counts)
+        return ops.Aggregation(T, src.hop, rscale=rs, hop_off=src.hop_off, node_off=src.node_off, reduce_graph=self.is_graph_task)
+
     def forward(self, inputs):
         if isinstance(inputs, PackedBatch):
             return self.forward_packed(inputs)
@@ -79,9 +96,7 @@ class TensorGNAN(_Base):
         else:
             _, hd = resolve(inputs, dev, need_x=False)
             S = self._feature_sums(*self._features(inputs))
-        T = self._table(ops.rho_table_inputs(hd.nbins, dev))                         # [nbins,Cr]
-        rs = ops.level_rscale(hd.level_counts) if self.normalize_rho else None       # models.py:368-370
-        out = ops.aggregate_rows(hd.hop, T, S, rscale=rs)
+        out = self._aggregation(hd, S)(S)
         if self._readout:
             hidden = out.sum(dim=0).view(1, -1)                                      # [1,K]  models.py:379
             return self.readout_nam(hidden).T                                        # [C,1]  models.py:380-384
@@ -96,17 +111,7 @@ class TensorGNAN(_Base):
         if pk.node_off.device != dev:
             pk = pk.to(dev)
         S = self._per_feature(pk.x.float().contiguous()) if self._readout else self._feature_sums(*self._features(pk))
-        T = self._table(ops.rho_table_inputs(pk.nbins, dev))
-        if (pk.deferred and self.normalize_rho and self.is_graph_task and T.dim() == 2 and ops.BLOCKDIAG_GRAPH_KERNEL
-                and ops.load().gnan_aggregate_blockdiag_graph_supported(T.shape[0], T.shape[1], S.shape[1])):
-            # distances not computed yet (preprocess.apsp_batched on a LocalEdges batch): the BFS and this readout run as one
-            # kernel, neither the hop bytes nor the normaliser table are ever written (models.py:366-384)
-            out = ops.bfs_graph_readout(pk.edges, pk.node_off, pk.max_nodes, T, S, pk.status)
-            return self.readout_nam(out) if self._readout else out
-        rs = None
-        if self.normalize_rho:       # models.py:368-370; a batch straight from apsp_batched(..., rscale=True) carries it already
-            rs = pk.level_rscale if getattr(pk, "level_rscale", None) is not None else ops.level_rscale(pk.level_counts)
-        out = ops.aggregate_blockdiag(pk.hop, pk.hop_off, pk.node_off, T, S, rscale=rs, reduce_graph=self.is_graph_task)
+        out = self._aggregation(pk, S)(S)
         return self.readout_nam(out) if self._readout else out                       # [B,K] -> [B,C]
 
 

@@ -555,6 +555,30 @@ def aggregate_blockdiag(hop, hop_off, node_off, T, S, rscale=None, per_row=False
     return agg_blockdiag_fwd(hop, hop_off, node_off, T, rscale, S, bool(per_row), bool(reduce_graph))
 
 
+class Aggregation:
+    """The aggregation a module applies to its feature sums S: the pair weights W[i,j,c'] = T[t_i, b(hop_ij), c'] * rscale[i, b(hop_ij)]
+    over its hop source (a dense row block `hop`; packed graphs `hop` / `hop_off` / `node_off`; or the edges of a deferred batch,
+    `fused` = (edges, max_nodes, status), whose distances the fused BFS + readout kernel computes on the fly) and whether rows are
+    summed per graph. Each module builds it in one place (`_aggregation`) for its forward and for gnan_b200.interpret.explain."""
+
+    def __init__(self, T, hop=None, rscale=None, per_row=False, hop_off=None, node_off=None, reduce_graph=False, fused=None):
+        self.T, self.hop, self.rscale, self.per_row = T, hop, rscale, bool(per_row)
+        self.hop_off, self.node_off, self.reduce_graph, self.fused = hop_off, node_off, bool(reduce_graph), fused
+
+    @property
+    def packed(self):
+        return self.node_off is not None
+
+    def __call__(self, S):
+        if self.fused is not None:
+            edges, max_n, status = self.fused
+            return bfs_graph_readout(edges, self.node_off, max_n, self.T, S, status)
+        if self.packed:
+            return aggregate_blockdiag(self.hop, self.hop_off, self.node_off, self.T, S, rscale=self.rscale, per_row=self.per_row,
+                                       reduce_graph=self.reduce_graph)
+        return aggregate_rows(self.hop, self.T, S, rscale=self.rscale, per_row=self.per_row)
+
+
 # ---------------------------------------------------------------------------------------------------------------------
 # row gather with a deterministic backward
 # ---------------------------------------------------------------------------------------------------------------------
@@ -589,6 +613,80 @@ class _GatherRows(torch.autograd.Function):
 
 def gather_rows(tq, inv, order, seg_ptr):
     return _GatherRows.apply(tq, inv, order, seg_ptr)
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# explanations: per-feature contributions to output rows on the compressed feature form (csrc/explain.cu; no autograd)
+# ---------------------------------------------------------------------------------------------------------------------
+def _i64(t: Tensor, name: str) -> Tensor:
+    if t.dtype != torch.int64:
+        raise TypeError(f"{name} must be int64, got {t.dtype}")
+    return t.contiguous()
+
+
+@torch.library.custom_op("gnan_b200::explain_segments", mutates_args=())
+def explain_segments(grp_ptr: Tensor, ent_row: Tensor, node_off: Tensor) -> Tensor:
+    lib = load()
+    if node_off.dtype != torch.int32:
+        raise TypeError("node_off must be int32 [B+1]")
+    K, B = grp_ptr.numel() - 1, node_off.numel() - 1
+    seg = torch.empty(K, B + 1, dtype=torch.int64, device=grp_ptr.device)
+    with _timed("explain_segments"):
+        check(lib.gnan_explain_segments(ptr(_i64(grp_ptr, "grp_ptr")), ptr(_i64(ent_row, "ent_row")), K, ptr(node_off.contiguous()), B,
+                                        ptr(seg), stream_handle()), "gnan_explain_segments")
+    return seg
+
+
+@explain_segments.register_fake
+def _(grp_ptr, ent_row, node_off):
+    return grp_ptr.new_empty(grp_ptr.numel() - 1, node_off.numel())
+
+
+@torch.library.custom_op("gnan_b200::explain_graph_features", mutates_args=())
+def explain_graph_features(Y: Tensor, grp_ptr: Tensor, ent_row: Tensor, seg: Tensor, colw: Tensor, colw_sum: Tensor) -> Tensor:
+    lib = load()
+    Y, colw, colw_sum = _f32(Y, "Y"), _f32(colw, "colw"), _f32(colw_sum, "colw_sum")
+    K, B, C = grp_ptr.numel() - 1, seg.shape[1] - 1, Y.shape[1]
+    if colw.shape[1] != C or tuple(colw_sum.shape) != (B, C):
+        raise ValueError(f"colw must be [N,{C}] and colw_sum [{B},{C}]")
+    F = torch.empty(B, K, C, dtype=torch.float32, device=Y.device)
+    with _timed("explain_graph_features"):
+        check(lib.gnan_explain_graph_features(ptr(Y), ptr(_i64(grp_ptr, "grp_ptr")), ptr(_i64(ent_row, "ent_row")), ptr(_i64(seg, "seg")),
+                                              K, B, C, ptr(colw), ptr(colw_sum), ptr(F), stream_handle()), "gnan_explain_graph_features")
+    return F
+
+
+@explain_graph_features.register_fake
+def _(Y, grp_ptr, ent_row, seg, colw, colw_sum):
+    return Y.new_empty(seg.shape[1] - 1, grp_ptr.numel() - 1, Y.shape[1])
+
+
+@torch.library.custom_op("gnan_b200::explain_rows_features", mutates_args=())
+def explain_rows_features(hop: Tensor, hop_off: Optional[Tensor], node_off: Tensor, ncols: int, rows: Optional[Tensor], n_rows: int,
+                          T: Tensor, per_row: bool, rscale: Optional[Tensor], Y: Tensor, grp_ptr: Tensor, ent_row: Tensor,
+                          seg: Tensor) -> Tensor:
+    lib = load()
+    T, Y = _f32(T, "T"), _f32(Y, "Y")
+    rscale = None if rscale is None else _f32(rscale, "rscale")
+    if hop.dtype != torch.uint8 or node_off.dtype != torch.int32:
+        raise TypeError("hop uint8 and node_off int32 expected")
+    R = rows.numel() if rows is not None else int(n_rows)
+    K, B, C = grp_ptr.numel() - 1, node_off.numel() - 1, Y.shape[1]
+    nbins, Cr = T.shape[-2], T.shape[-1]
+    F = torch.empty(R, K, C, dtype=torch.float32, device=Y.device)
+    with _timed("explain_rows_features"):
+        check(lib.gnan_explain_rows_features(ptr(hop), hop.shape[-1] if hop_off is None else 0, ptr(None if hop_off is None else _i64(hop_off, "hop_off")),
+                                             ptr(node_off.contiguous()), B, int(ncols), ptr(None if rows is None else _i64(rows, "rows")), R,
+                                             ptr(T), int(per_row), nbins, Cr, ptr(rscale), ptr(Y), ptr(_i64(grp_ptr, "grp_ptr")),
+                                             ptr(_i64(ent_row, "ent_row")), ptr(_i64(seg, "seg")), K, C, ptr(F), stream_handle()),
+              "gnan_explain_rows_features")
+    return F
+
+
+@explain_rows_features.register_fake
+def _(hop, hop_off, node_off, ncols, rows, n_rows, T, per_row, rscale, Y, grp_ptr, ent_row, seg):
+    R = rows.numel() if rows is not None else int(n_rows)
+    return Y.new_empty(R, grp_ptr.numel() - 1, Y.shape[1])
 
 
 # ---------------------------------------------------------------------------------------------------------------------

@@ -350,16 +350,24 @@ def _e2r_backward(ctx, dS):
 entries_to_rows.register_autograd(_e2r_backward, setup_context=_e2r_setup)
 
 
-def feature_sums(cx: CompressedFeatures, w1, b1, wh, bh, wo, bo, n_layers, precision="fp32") -> Tensor:
-    """S [N,C] = sum_k f_k(x[:,k]) from the compressed form; differentiable w.r.t. the weights. `precision` selects the
-    kernels (fp32 FFMA, or the tcgen05 3xTF32 kernels for H = 64, 3 layers, C <= 8), forward and backward."""
+def entry_values(cx: CompressedFeatures, w1, b1, wh, bh, wo, bo, n_layers, precision="fp32") -> Tensor:
+    """Y [E,C] = f_k(val[e]) for every entry e of the compressed form (k = ent_grp[e]); differentiable w.r.t. the weights.
+    `precision` selects the kernels (fp32 FFMA, or the tcgen05 3xTF32 kernels for H = 64, 3 layers, C <= 8), forward and
+    backward. A single Linear(1,C) (n_layers = 1, which the entries kernels do not take) is an affine map per feature."""
     if wo.shape[0] != cx.num_features:
         raise ValueError(f"compressed x has {cx.num_features} features, the model {wo.shape[0]}")
+    if int(n_layers) == 1:
+        g = cx.ent_grp.long()
+        return cx.val[:, None] * wo[g, :, 0] + bo[g]
     from ._lib import PRECISIONS
     sh = cx.shared
     if sh is not None:      # one evaluation per distinct (feature, value); entries gather it (backward: fixed-order segment sums)
         Yq = mlp_entries_fwd(sh.val, sh.grp_ptr, sh.items, w1, b1, wh, bh, wo, bo, int(n_layers), sh.max_group, PRECISIONS[precision])
-        Y = ops.gather_rows(Yq, sh.inv, sh.order, sh.seg_ptr)
-    else:
-        Y = mlp_entries_fwd(cx.val, cx.grp_ptr, cx.items, w1, b1, wh, bh, wo, bo, int(n_layers), cx.max_group, PRECISIONS[precision])
+        return ops.gather_rows(Yq, sh.inv, sh.order, sh.seg_ptr)
+    return mlp_entries_fwd(cx.val, cx.grp_ptr, cx.items, w1, b1, wh, bh, wo, bo, int(n_layers), cx.max_group, PRECISIONS[precision])
+
+
+def feature_sums(cx: CompressedFeatures, w1, b1, wh, bh, wo, bo, n_layers, precision="fp32") -> Tensor:
+    """S [N,C] = sum_k f_k(x[:,k]) from the compressed form (entry_values, then the baseline + exceptions sum of each row)."""
+    Y = entry_values(cx, w1, b1, wh, bh, wo, bo, n_layers, precision)
     return entries_to_rows(Y, cx.grp_ptr, cx.csr_ptr, cx.csr_eid, cx.ent_grp, cx.ent_row)

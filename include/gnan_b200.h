@@ -239,6 +239,34 @@ int gnan_aggregate_blockdiag_graph_bwd(const int32_t *node_off, int32_t B, int32
                                        void *workspace, size_t workspace_bytes, gnan_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * Explanations (csrc/explain.cu; gnan_b200.interpret.explain): the contribution of each shape function k to an output row, the
+ * reference's mf = matmul(W, fx) of GNAN.py:68-70 before its sum over features, with W[i,j,c'] = T[t_i, b(hop[i,j]), c'] *
+ * rscale[i, b(hop[i,j])] as in gnan_aggregate_rows_fwd_ws. The features come in the compressed form of gnan_mlp_entries_*:
+ * group k = [baseline entry, exceptions sorted by row], Y [E,C] the entry values f_k(val[e]), ent_row [E] (-1 for a baseline).
+ * Graph b owns nodes [node_off[b], node_off[b+1]) (a dense single graph: B = 1, node_off = {0, N}).
+ * seg [K, B+1] (gnan_explain_segments): seg[k,b] = first exception of k with a row >= node_off[b], so the exceptions of feature k
+ * inside graph b are [seg[k,b], seg[k,b+1]).
+ * Graph rows:  F[b,k,c] = Y[base_k,c] * colw_sum[b,c] + sum_{e in seg(k,b)} colw[row(e),c] * (Y[e,c] - Y[base_k,c])   [B,K,C]
+ *   colw [N,C] = sum_{i in graph(j)} W[i,j,c'] (the aggregation's dS for a unit output gradient), colw_sum [B,C] its sum per graph.
+ * Node rows:   F[r,k,c] = Y[base_k,c] * sum_j W[i,j,c'] + sum_{e in seg(k,b(i))} W[i,row(e),c'] * (Y[e,c] - Y[base_k,c])   [R,K,C]
+ *   i = rows[r] (rows NULL: i = r). hop_off == NULL: a dense row block, hop row i at hop + i*ld_hop with ncols = N columns (B = 1);
+ *   else packed graphs as in gnan_aggregate_blockdiag_fwd, i a global node id, ncols >= the largest graph. T (table_per_row) and
+ *   rscale rows are indexed by i; every i must be a row of the block / a node of the batch (not checked on the device). Any C;
+ *   GNAN_ERR_UNSUPPORTED when one hop row with its weights and histogram does not fit shared memory. B >= 1 here, B >= 0 for
+ *   the segment table and the graph rows (no graphs: nothing to do).
+ * Work is rows x exceptions, each output element is a fixed-order sum written once (deterministic, no workspace). */
+int gnan_explain_segments(const int64_t *grp_ptr /* [K+1] */, const int64_t *ent_row /* [E] */, int32_t K, const int32_t *node_off /* [B+1] */,
+                          int32_t B, int64_t *seg /* [K,B+1] */, gnan_stream_t stream);
+int gnan_explain_graph_features(const float *Y, const int64_t *grp_ptr, const int64_t *ent_row, const int64_t *seg, int32_t K, int32_t B,
+                                int32_t C, const float *colw /* [N,C] */, const float *colw_sum /* [B,C] */, float *F /* [B,K,C] */,
+                                gnan_stream_t stream);
+int gnan_explain_rows_features(const uint8_t *hop, int64_t ld_hop, const int64_t *hop_off /* [B+1] or NULL */, const int32_t *node_off,
+                               int32_t B, int64_t ncols, const int64_t *rows /* [R] or NULL */, int64_t R, const float *T, int table_per_row,
+                               int32_t nbins, int32_t Cr, const float *rscale /* or NULL */, const float *Y, const int64_t *grp_ptr,
+                               const int64_t *ent_row, const int64_t *seg, int32_t K, int32_t C, float *F /* [R,K,C] */,
+                               gnan_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------------
  * The tail of the training step (csrc/train.cu; replaces trainer.py:52-67 and torch.optim.Adam.step, main.py:141).
  * Losses: *loss (device float, overwritten) = scale * sum of the per-sample terms (scale = 1/M for the reference's mean
  * reduction) and, when dlogits != NULL, d(loss)/d(logits) for an upstream gradient of 1 in the same pass.
