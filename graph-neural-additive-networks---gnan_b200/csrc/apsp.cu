@@ -250,18 +250,24 @@ __global__ void bv3_classify_kernel(const int32_t *__restrict__ node_off, int B,
     if (ok) cls[4 + (size_t)c * B + (c >> 2) + base + __popc(peers & ((1u << lane) - 1))] = b;   // class 4: after its size word
 }
 
-struct Bv3Out {
+template <typename IT>
+struct Bv3OutT {
     uint8_t *hop;
     int32_t *cnt;
     float *rscale;
     const float *rcp_tab;
     int nbins;
-    // LOCAL: the batch's edges grouped by graph, endpoints as indices inside the graph; *status |= 1 for an endpoint >= n (edge
-    // dropped), |= 2 for a repeated (src,dst) pair (gnan_build_csr's status bits)
-    const uint8_t *lsrc, *ldst;
+    // LOCAL: the batch's edges grouped by graph, endpoints as indices inside the graph (uint8, or int16 for the fused readout);
+    // *status |= 1 for an endpoint >= n (edge dropped), |= 2 for a repeated (src,dst) pair (gnan_build_csr's status bits)
+    const IT *lsrc, *ldst;
     const int32_t *edge_off;
     int32_t *status;
 };
+using Bv3Out = Bv3OutT<uint8_t>;
+
+// an endpoint of the transfer form as an unsigned index: a negative int16 becomes >= 32768, i.e. out of every graph's range
+__device__ __forceinline__ uint32_t local_index(uint8_t x) { return x; }
+__device__ __forceinline__ uint32_t local_index(int16_t x) { return (uint16_t)x; }
 
 // graph b on the G warps of a sub-group: fill the slice, BFS, write the level table and the hop block out
 template <int W, int G, bool LOCAL>
@@ -379,9 +385,9 @@ __device__ __forceinline__ void bv3_ro_fold(int d, float p, const float (&s)[CC]
     }
 }
 
-template <int W, int G, int CC>
+template <int W, int G, int CC, typename IT>
 __device__ __forceinline__ int bv3_readout_run(const int32_t *__restrict__ node_off, int64_t b, int ts, int bar, uint8_t *slice,
-                                               const Bv3Out &o, const Bv3Readout &r, int32_t *overflow)
+                                               const Bv3OutT<IT> &o, const Bv3Readout &r, int32_t *overflow)
 {
     constexpr int T = 32 * G, WS = bv3_ws(W);
     const int n0 = node_off[b], n = node_off[b + 1] - n0, nbins = o.nbins, nq = nbins * CC;
@@ -398,7 +404,7 @@ __device__ __forceinline__ int bv3_readout_run(const int32_t *__restrict__ node_
     const int e0 = o.edge_off[b], e1 = o.edge_off[b + 1];
     int flags = 0;                                                             // status bits as gnan_apsp_bfs_batched_local
     for (int e = e0 + ts; e < e1; e += T) {
-        const uint32_t s = o.lsrc[e], d = o.ldst[e];
+        const uint32_t s = local_index(o.lsrc[e]), d = local_index(o.ldst[e]);
         if (s < (uint32_t)n && d < (uint32_t)n) {
             const uint32_t bit = 1u << (d & 31);
             if (atomicOr(adj + s * WS + (d >> 5), bit) & bit) flags |= 2;
@@ -410,7 +416,7 @@ __device__ __forceinline__ int bv3_readout_run(const int32_t *__restrict__ node_
     bv3_sync<G>(bar);
     bool asym = false;
     for (int e = e0 + ts; e < e1; e += T) {
-        const uint32_t s = o.lsrc[e], d = o.ldst[e];
+        const uint32_t s = local_index(o.lsrc[e]), d = local_index(o.ldst[e]);
         if (s < (uint32_t)n && d < (uint32_t)n && !((adj[d * WS + (s >> 5)] >> (s & 31)) & 1u)) asym = true;
     }
     const bool sym = !bv3_any<G>(bar, asym);
@@ -541,31 +547,34 @@ __device__ __forceinline__ int bv3_readout_run(const int32_t *__restrict__ node_
 }
 
 // one work item of the v3 kernel: the BFS of bv3_run, or (CC > 0) the BFS fused with the graph readout
-template <int W, int G, bool LOCAL, int CC>
+template <int W, int G, bool LOCAL, int CC, typename IT>
 __device__ __forceinline__ int bv3_item(const int32_t *__restrict__ rowptr, const int32_t *__restrict__ col,
                                         const int32_t *__restrict__ node_off, const int64_t *__restrict__ hop_off, int64_t b, int cap,
-                                        int ts, int bar, uint8_t *slice, const Bv3Out &o, const Bv3Readout &r, bool levels, int32_t *overflow)
+                                        int ts, int bar, uint8_t *slice, const Bv3OutT<IT> &o, const Bv3Readout &r, bool levels,
+                                        int32_t *overflow)
 {
-    if constexpr (CC > 0) return bv3_readout_run<W, G, CC>(node_off, b, ts, bar, slice, o, r, overflow);
+    if constexpr (CC > 0) return bv3_readout_run<W, G, CC, IT>(node_off, b, ts, bar, slice, o, r, overflow);
     else return bv3_run<W, G, LOCAL>(rowptr, col, node_off, hop_off, b, cap, ts, bar, slice, o, levels, overflow);
 }
 
-// the batch's edge list in its transfer form (LOCAL instantiation: no CSR; rowptr / col are NULL)
-struct Bv3Edges {
-    const uint8_t *src, *dst;
+// the batch's edge list in its transfer form (LOCAL instantiation: no CSR; rowptr / col are NULL); IT = int16 only with CC > 0
+template <typename IT>
+struct Bv3EdgesT {
+    const IT *src, *dst;
     const int32_t *edge_off;
     int32_t *status;
 };
+using Bv3Edges = Bv3EdgesT<uint8_t>;
 
 // order = the output of bv3_classify_kernel
 // (the multi-channel readout instantiations keep the level's new bits across the barrier: 4 groups per CTA give them 64 registers)
 constexpr int bv3_max_groups(int cc) { return cc > 1 ? BV3_MAX_GROUPS - 1 : BV3_MAX_GROUPS; }
-template <bool LOCAL, int CC = 0>
+template <bool LOCAL, int CC = 0, typename IT = uint8_t>
 __global__ void __launch_bounds__(32 * BV3_GW * bv3_max_groups(CC), 2)
 apsp_batched_v3_kernel(const int32_t *__restrict__ rowptr, const int32_t *__restrict__ col, const int32_t *__restrict__ node_off,
                        const int64_t *__restrict__ hop_off, int B, int max_n, int groups_per_cta, int slice_bytes, uint8_t *__restrict__ hop,
                        int32_t *__restrict__ cnt, float *__restrict__ rscale, int nbins, int32_t *__restrict__ overflow,
-                       int32_t *__restrict__ max_level, const int32_t *__restrict__ order, Bv3Edges le, Bv3Readout ro)
+                       int32_t *__restrict__ max_level, const int32_t *__restrict__ order, Bv3EdgesT<IT> le, Bv3Readout ro)
 {
     extern __shared__ __align__(16) uint8_t sm3[];
     __shared__ float rcp_tab[256];
@@ -577,7 +586,7 @@ apsp_batched_v3_kernel(const int32_t *__restrict__ rowptr, const int32_t *__rest
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, g = warp / BV3_GW, wq = warp % BV3_GW;
     uint8_t *gslice = sm3 + (size_t)g * slice_bytes;
     const int bar_group = 1 + 3 * g;
-    const Bv3Out out{hop, cnt, rscale, rcp_tab, nbins, le.src, le.dst, le.edge_off, le.status};
+    const Bv3OutT<IT> out{hop, cnt, rscale, rcp_tab, nbins, le.src, le.dst, le.edge_off, le.status};
     const int c0 = order[0], c_big = c0 + order[1], c2 = order[2], c3 = order[3];
     const int32_t *ord0 = order + 4, *ord1 = ord0 + B, *ord2 = ord1 + B, *ord3 = ord2 + B;
     const int items2 = (c2 + 1) / 2, items1 = (c3 + 3) / 4;
@@ -590,19 +599,19 @@ apsp_batched_v3_kernel(const int32_t *__restrict__ rowptr, const int32_t *__rest
             const int64_t b = t < c0 ? ord0[t] : ord1[t - c0];
             const int n = node_off[b + 1] - node_off[b];
             const int ts = wq * 32 + lane;
-            const int lm = n <= 96 ? bv3_item<3, 4, LOCAL, CC>(rowptr, col, node_off, hop_off, b, max_n, ts, bar_group, gslice, out, ro, levels, overflow)
-                                   : bv3_item<4, 4, LOCAL, CC>(rowptr, col, node_off, hop_off, b, max_n, ts, bar_group, gslice, out, ro, levels, overflow);
+            const int lm = n <= 96 ? bv3_item<3, 4, LOCAL, CC, IT>(rowptr, col, node_off, hop_off, b, max_n, ts, bar_group, gslice, out, ro, levels, overflow)
+                                   : bv3_item<4, 4, LOCAL, CC, IT>(rowptr, col, node_off, hop_off, b, max_n, ts, bar_group, gslice, out, ro, levels, overflow);
             lvl_max = max(lvl_max, lm);
         } else if (t < c_big + items2) {                             // 33..64 nodes: two graphs on the two warp pairs
             const int pr = wq >> 1;
             const int64_t idx = 2 * (t - c_big) + pr;
             if (idx < c2)
-                lvl_max = max(lvl_max, bv3_item<2, 2, LOCAL, CC>(rowptr, col, node_off, hop_off, ord2[idx], cap2, (wq & 1) * 32 + lane,
+                lvl_max = max(lvl_max, bv3_item<2, 2, LOCAL, CC, IT>(rowptr, col, node_off, hop_off, ord2[idx], cap2, (wq & 1) * 32 + lane,
                                                      bar_group + 1 + pr, gslice + (size_t)pr * half, out, ro, levels, overflow));
         } else {                                                     // up to 32 nodes: four graphs, a warp each
             const int64_t idx = 4 * (t - c_big - items2) + wq;
             if (idx < c3)
-                lvl_max = max(lvl_max, bv3_item<1, 1, LOCAL, CC>(rowptr, col, node_off, hop_off, ord3[idx], cap1, lane, 0,
+                lvl_max = max(lvl_max, bv3_item<1, 1, LOCAL, CC, IT>(rowptr, col, node_off, hop_off, ord3[idx], cap1, lane, 0,
                                                      gslice + (size_t)wq * quarter, out, ro, levels, overflow));
         }
         bv3_sync<BV3_GW>(bar_group);                                 // the slice is re-partitioned / refilled by the next item
@@ -620,14 +629,17 @@ apsp_batched_v3_kernel(const int32_t *__restrict__ rowptr, const int32_t *__rest
 // hop[v][s0+s] = L and popc(new[v]) adds to row v's level-L count. A thread owns rows v of hop and cnt: no atomics. One
 // __syncthreads_or per level ends the level loop of a chunk. The CTA first writes its graph's 255 / 0 background (coalesced
 // 16-byte stores), then scatters the reached bytes and adds each chunk's counts into the rows. Neighbours come from the CSR.
+// rscale (1/count, gnan_level_rscale's 1.0f / (float)count) without cnt: the counts are summed in the rscale rows themselves (exact
+// integers in fp32) and each owner thread inverts its rows once after the last chunk.
 constexpr int BL_THREADS = 512;
 constexpr int BL_VPT = GNAN_APSP_BATCHED_MAX_NODES / BL_THREADS;   // vertices per thread
 constexpr int BL_W = 4;                                              // source words per vertex: 128 sources per chunk
 
 __global__ void __launch_bounds__(BL_THREADS, 2)
 apsp_batched_large_kernel(const int32_t *__restrict__ rowptr, const int32_t *__restrict__ col, const int32_t *__restrict__ node_off,
-                          const int64_t *__restrict__ hop_off, int B, uint8_t *__restrict__ hop, int32_t *__restrict__ cnt, int nbins,
-                          int32_t *__restrict__ overflow, int32_t *__restrict__ max_level, const int32_t *__restrict__ order)
+                          const int64_t *__restrict__ hop_off, int B, uint8_t *__restrict__ hop, int32_t *__restrict__ cnt,
+                          float *__restrict__ rscale, int nbins, int32_t *__restrict__ overflow, int32_t *__restrict__ max_level,
+                          const int32_t *__restrict__ order)
 {
     __shared__ __align__(16) uint32_t fr[2][GNAN_APSP_BATCHED_MAX_NODES * BL_W];   // frontier rows [n][BL_W], by level parity
     const int tid = threadIdx.x;
@@ -639,6 +651,8 @@ apsp_batched_large_kernel(const int32_t *__restrict__ rowptr, const int32_t *__r
         const int n0 = node_off[b], n = node_off[b + 1] - n0;
         uint8_t *gb = hop + hop_off[b];
         int32_t *gc = cnt ? cnt + (int64_t)n0 * nbins : nullptr;
+        float *gr = rscale ? rscale + (int64_t)n0 * nbins : nullptr;
+        float *gf = gc ? nullptr : gr;                               // the count rows in fp32 when there is no int32 table
         // background: head bytes up to the first 16-byte boundary, vector body, tail bytes
         const int total = n * n;
         const int head = min(total, (int)((16 - (reinterpret_cast<uintptr_t>(gb) & 15)) & 15));
@@ -650,6 +664,8 @@ apsp_batched_large_kernel(const int32_t *__restrict__ rowptr, const int32_t *__r
         if (tid < 16 && tail0 + tid < total) gb[tail0 + tid] = GNAN_HOP_UNREACHABLE;
         if (gc)
             for (int i = tid; i < n * nbins; i += BL_THREADS) gc[i] = 0;
+        if (gf)
+            for (int i = tid; i < n * nbins; i += BL_THREADS) gf[i] = 0.f;
         __syncthreads();
         int reached[BL_VPT];
 #pragma unroll
@@ -659,6 +675,7 @@ apsp_batched_large_kernel(const int32_t *__restrict__ rowptr, const int32_t *__r
             if (v < n) {
                 gb[(size_t)v * n + v] = 0;
                 if (gc) gc[(int64_t)v * nbins] = 1;
+                if (gf) gf[(int64_t)v * nbins] = 1.f;
             }
         }
         for (int s0 = 0; s0 < n; s0 += 32 * BL_W) {
@@ -707,6 +724,7 @@ apsp_batched_large_kernel(const int32_t *__restrict__ rowptr, const int32_t *__r
                             }
                             if (level > 254 || level >= nbins - 1) atomicExch(overflow, 1);
                             else if (gc) gc[(int64_t)v * nbins + level] += newc;
+                            else if (gf) gf[(int64_t)v * nbins + level] += (float)newc;
                             reached[k] += newc;
                         }
                     }
@@ -715,13 +733,260 @@ apsp_batched_large_kernel(const int32_t *__restrict__ rowptr, const int32_t *__r
                 lvl_max = max(lvl_max, level);
             }
         }
-        if (gc) {
 #pragma unroll
-            for (int k = 0; k < BL_VPT; ++k) {
-                const int v = tid + k * BL_THREADS;
-                if (v < n) gc[(int64_t)v * nbins + nbins - 1] = n - reached[k];
+        for (int k = 0; k < BL_VPT; ++k) {
+            const int v = tid + k * BL_THREADS;
+            if (v >= n) continue;
+            if (gc) gc[(int64_t)v * nbins + nbins - 1] = n - reached[k];
+            if (gf) gf[(int64_t)v * nbins + nbins - 1] = (float)(n - reached[k]);
+            if (gr)
+                for (int d = 0; d < nbins; ++d) {                   // as level_rscale_kernel
+                    const float c = gc ? (float)gc[(int64_t)v * nbins + d] : gr[(int64_t)v * nbins + d];
+                    gr[(int64_t)v * nbins + d] = c > 0.f ? 1.0f / c : 0.f;
+                }
+        }
+    }
+    if (max_level && tid == 0 && lvl_max > 0) atomicMax(max_level, lvl_max);   // lvl_max is uniform over the CTA
+}
+
+// ---- the fused BFS + graph readout on graphs of 129..GNAN_APSP_BATCHED_MAX_NODES nodes: one CTA per graph -------------------
+// The sources advance 128 at a time as in apsp_batched_large_kernel, but the pull runs over IN-neighbours: vertex v keeps the bits
+// of the chunk's sources s that reach it, and a new bit (v, s) at level L means d(s -> v) = L, i.e. hop[s][v] = L. So v is column
+// j = v of the readout and the level size count(s, L) = cnt[s][L] of row s is a column count over the CTA's vertices: every new
+// bit adds 1 to the chunk's shared-memory integer counter of its source, and the counters are complete when the level's barrier
+// has passed. Each vertex then adds P[v,L] = sum over its new sources (ascending) of 1/count(s,L) and folds it at once, as the v3
+// readout does: colw[v,:] += T[L,:] p in registers, Q[L,:] += S[v,:] p as one warp sum into the warp's own [nbins][C] slot (added
+// to across chunks; the slots are added in warp order at the end). colw sums one term per (chunk, level), up to 8 x 63 for a graph
+// of 1024 nodes, and the unreachable bin one term per source that does not reach v, up to 1023: both are accumulated in fp64 (in
+// fp32, 1024-node graphs missed the 1e-5 * A bound of the float64 reference). Exact on directed graphs in one pass, no symmetry test. The
+// unreachable bin: after each chunk, 1/(n - reached_s) over the chunk's sources that did not reach v, in a register until the end.
+// Level 0 contributes 1 to every vertex once. The in-neighbour bit matrix [n][ceil(n/32)] is built in shared memory from the
+// graph's own edge segment (atomicOr: duplicates and endpoints beyond the graph set the status bits, as the v3 kernels); up to 4
+// in-neighbours of a vertex are cached as 16-bit halves of two registers, longer rows walk their bit row. Nothing but out, colw,
+// Q and the status words reaches global memory. Dynamic shared memory and the block size follow the batch's largest graph.
+constexpr int BRL_MAX_THREADS = 512;
+constexpr int BRL_VPT = GNAN_APSP_BATCHED_MAX_NODES / BRL_MAX_THREADS;   // vertices per thread
+constexpr int BRL_SRC = 32 * BL_W;                                       // sources per chunk
+
+// threads per CTA: one per vertex up to 512 nodes (a batch holds few large graphs, so each one's latency is what counts), two above;
+// at least one per source of a chunk
+inline int brl_threads(int cap) { return std::min(BRL_MAX_THREADS, std::max(BRL_SRC, (cap + 31) / 32 * 32)); }
+// frontier rows [2][cap][BL_W], in-neighbour bits [cap][ceil(cap/32)], per-warp Q [NW][nbins][CC] + out [NW][CC], source counters
+// [3][BRL_SRC] (by level mod 3: filled at L, read after the barrier of L, zeroed at L + 2), 1/(n - reached) [BRL_SRC]
+inline size_t brl_need(int cap, int nthreads, int nbins, int CC)
+{
+    return (size_t)2 * cap * BL_W * 4 + (size_t)cap * ((cap + 31) / 32) * 4 + (size_t)(nthreads / 32) * (nbins + 1) * CC * 4 +
+           (size_t)4 * BRL_SRC * 4;
+}
+
+// the vertex share of bin d: colw += T[d,:] p, the warp's Q slot [d,:] += the warp sum of S[v,:] p (all threads call it)
+template <int CC, typename PT>
+__device__ __forceinline__ void brl_fold(int d, const PT (&p)[BRL_VPT], const float (&s)[BRL_VPT][CC], double (&cw)[BRL_VPT][CC],
+                                         float *sqw, const Bv3Readout &r, int lane)
+{
+#pragma unroll
+    for (int c = 0; c < CC; ++c) {
+        if (c < r.Cr) {
+            const double t = __ldg(r.T + d * r.Cr + c);
+#pragma unroll
+            for (int k = 0; k < BRL_VPT; ++k) cw[k][c] = fma(t, (double)p[k], cw[k][c]);
+        }
+        if (c < r.C) {
+            float q = s[0][c] * (float)p[0];
+#pragma unroll
+            for (int k = 1; k < BRL_VPT; ++k) q = fmaf(s[k][c], (float)p[k], q);
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) q += __shfl_xor_sync(0xffffffffu, q, o);
+            if (lane == 0) sqw[d * CC + c] += q;
+        }
+    }
+}
+
+template <typename IT, int CC>
+__global__ void __launch_bounds__(BRL_MAX_THREADS, CC > 1 ? 1 : 2)
+bfs_readout_large_kernel(const IT *__restrict__ src, const IT *__restrict__ dst, const int32_t *__restrict__ edge_off,
+                         const int32_t *__restrict__ node_off, int B, int cap, int nbins, Bv3Readout r, int32_t *__restrict__ status,
+                         int32_t *__restrict__ overflow, int32_t *__restrict__ max_level, const int32_t *__restrict__ order)
+{
+    extern __shared__ __align__(16) uint8_t smL[];
+    const int tid = threadIdx.x, NT = blockDim.x, lane = tid & 31, warp = tid >> 5, NW = NT >> 5, nq = nbins * CC;
+    uint32_t *fr = reinterpret_cast<uint32_t *>(smL);                     // [2][cap][BL_W]
+    uint32_t *adj = fr + 2 * cap * BL_W;                                   // [n][AW] of [cap][ceil(cap/32)]
+    float *sq = reinterpret_cast<float *>(adj + cap * ((cap + 31) / 32));  // [NW][nbins][CC]
+    float *so = sq + NW * nq;                                              // [NW][CC]
+    int *cnt = reinterpret_cast<int *>(so + NW * CC);                      // [3][BRL_SRC]
+    float *urc = reinterpret_cast<float *>(cnt + 3 * BRL_SRC);             // [BRL_SRC]
+    float *sqw = sq + warp * nq;
+    const int n_large = order[4 + 4 * (size_t)B];
+    const int32_t *list = order + 5 + 4 * (size_t)B;
+    int lvl_max = 0;
+    for (int t = blockIdx.x; t < n_large; t += gridDim.x) {
+        const int64_t b = list[t];
+        const int n0 = node_off[b], n = node_off[b + 1] - n0, AW = (n + 31) / 32;
+        for (int i = tid; i < n * AW; i += NT) adj[i] = 0u;
+        for (int i = tid; i < NW * (nq + CC); i += NT) sq[i] = 0.f;
+        __syncthreads();
+        const int e0 = edge_off[b], e1 = edge_off[b + 1];
+        int flags = 0;
+        for (int e = e0 + tid; e < e1; e += NT) {                          // edge s -> d: bit s of d's in-neighbour row
+            const uint32_t s = local_index(src[e]), d = local_index(dst[e]);
+            if (s < (uint32_t)n && d < (uint32_t)n) {
+                const uint32_t bit = 1u << (s & 31);
+                if (atomicOr(adj + d * AW + (s >> 5), bit) & bit) flags |= 2;
+            } else {
+                flags |= 1;
             }
         }
+        if (flags) atomicOr(status, flags);
+        __syncthreads();
+
+        float s[BRL_VPT][CC], p[BRL_VPT];
+        double cw[BRL_VPT][CC], U[BRL_VPT];
+        uint32_t nb[BRL_VPT][2];
+        int dg[BRL_VPT];                                                   // in-degree; > 4: walk the bit row
+#pragma unroll
+        for (int k = 0; k < BRL_VPT; ++k) {
+            const int v = tid + k * NT;
+            const bool mine = v < n;
+#pragma unroll
+            for (int c = 0; c < CC; ++c) {
+                s[k][c] = (mine && c < r.C) ? r.S[(int64_t)(n0 + v) * r.C + c] : 0.f;
+                cw[k][c] = 0.0;
+            }
+            U[k] = 0.0;
+            p[k] = mine ? 1.f : 0.f;                                       // level 0: v itself, count 1
+            nb[k][0] = nb[k][1] = 0u;
+            dg[k] = 0;
+            if (mine) {
+                const uint32_t *arow = adj + v * AW;
+                for (int ww = 0; ww < AW; ++ww) dg[k] += __popc(arow[ww]);
+                if (dg[k] <= 4) {
+                    int j = 0;
+                    for (int ww = 0; ww < AW; ++ww)
+                        for (uint32_t m = arow[ww]; m; m &= m - 1, ++j) {
+                            const uint32_t u = (uint32_t)(ww * 32 + __ffs(m) - 1) << (16 * (j & 1));
+                            if (j < 2) nb[k][0] |= u;
+                            else nb[k][1] |= u;
+                        }
+                }
+            }
+        }
+        brl_fold<CC>(0, p, s, cw, sqw, r, lane);
+        for (int s0 = 0; s0 < n; s0 += BRL_SRC) {
+            uint32_t vis[BRL_VPT][BL_W];
+#pragma unroll
+            for (int k = 0; k < BRL_VPT; ++k) {
+                const int v = tid + k * NT, rel = v - s0;
+#pragma unroll
+                for (int ww = 0; ww < BL_W; ++ww) vis[k][ww] = (rel >= 0 && (rel >> 5) == ww) ? 1u << (rel & 31) : 0u;
+                if (v < n) bv3_store_row<BL_W>(fr + v * BL_W, vis[k]);
+            }
+            for (int i = tid; i < 3 * BRL_SRC; i += NT) cnt[i] = 0;
+            int reach = 1;                                                 // thread tid < BRL_SRC: vertices reached by source s0 + tid
+            __syncthreads();
+            for (int level = 1; level <= n; ++level) {
+                const uint32_t *fc = fr + ((level - 1) & 1) * cap * BL_W;
+                uint32_t *fn = fr + (level & 1) * cap * BL_W;
+                int *cl = cnt + (level % 3) * BRL_SRC;
+                if (tid < BRL_SRC) cnt[((level + 1) % 3) * BRL_SRC + tid] = 0;
+                bool any = false;
+#pragma unroll
+                for (int k = 0; k < BRL_VPT; ++k) {
+                    const int v = tid + k * NT;
+                    if (v >= n) continue;
+                    uint32_t acc[BL_W] = {0u, 0u, 0u, 0u};
+                    if (dg[k] <= 4) {
+#pragma unroll
+                        for (int j = 0; j < 4; ++j)
+                            if (j < dg[k]) bv3_or_row<BL_W>(fc + ((nb[k][j >> 1] >> (16 * (j & 1))) & 0xffffu) * BL_W, acc);
+                    } else {
+                        const uint32_t *arow = adj + v * AW;
+                        for (int ww = 0; ww < AW; ++ww)
+                            for (uint32_t m = arow[ww]; m; m &= m - 1) bv3_or_row<BL_W>(fc + (ww * 32 + __ffs(m) - 1) * BL_W, acc);
+                    }
+                    bool nw = false;
+#pragma unroll
+                    for (int ww = 0; ww < BL_W; ++ww) {
+                        acc[ww] &= ~vis[k][ww];
+                        vis[k][ww] |= acc[ww];
+                        nw |= acc[ww] != 0u;
+                        for (uint32_t m = acc[ww]; m; m &= m - 1) atomicAdd(cl + ww * 32 + __ffs(m) - 1, 1);
+                    }
+                    bv3_store_row<BL_W>(fn + v * BL_W, acc);
+                    if (nw) {
+                        any = true;
+                        if (level >= nbins - 1) atomicExch(overflow, 1);
+                    }
+                }
+                if (!__syncthreads_or(any)) break;
+                lvl_max = max(lvl_max, level);
+                if (tid < BRL_SRC) reach += cl[tid];
+                if (level < nbins - 1) {                                   // P[v, level] over v's new sources, from its frontier row
+#pragma unroll
+                    for (int k = 0; k < BRL_VPT; ++k) {
+                        const int v = tid + k * NT;
+                        p[k] = 0.f;
+                        if (v >= n) continue;
+                        const uint4 q = *reinterpret_cast<const uint4 *>(fn + v * BL_W);
+                        const uint32_t w4[BL_W] = {q.x, q.y, q.z, q.w};
+#pragma unroll
+                        for (int ww = 0; ww < BL_W; ++ww)
+                            for (uint32_t m = w4[ww]; m; m &= m - 1) p[k] += __frcp_rn((float)cl[ww * 32 + __ffs(m) - 1]);
+                    }
+                    brl_fold<CC>(level, p, s, cw, sqw, r, lane);
+                }
+            }
+            if (tid < BRL_SRC) urc[tid] = (s0 + tid < n && reach < n) ? __frcp_rn((float)(n - reach)) : 0.f;
+            __syncthreads();
+            const int nsrc = min(BRL_SRC, n - s0);
+#pragma unroll
+            for (int k = 0; k < BRL_VPT; ++k) {
+                if (tid + k * NT >= n) continue;
+#pragma unroll
+                for (int ww = 0; ww < BL_W; ++ww) {
+                    const int left = nsrc - ww * 32;
+                    for (uint32_t m = ~vis[k][ww] & (left >= 32 ? 0xffffffffu : (left > 0 ? (1u << left) - 1u : 0u)); m; m &= m - 1)
+                        U[k] += urc[ww * 32 + __ffs(m) - 1];
+                }
+            }
+            __syncthreads();                                               // the next chunk rewrites fr, cnt and urc
+        }
+        brl_fold<CC>(nbins - 1, U, s, cw, sqw, r, lane);
+#pragma unroll
+        for (int k = 0; k < BRL_VPT; ++k) {
+            const int v = tid + k * NT;
+            if (v < n) {
+#pragma unroll
+                for (int c = 0; c < CC; ++c)
+                    if (c < r.Cr) r.colw[(int64_t)(n0 + v) * r.Cr + c] = (float)cw[k][c];
+            }
+        }
+        // out[b,c] = sum_v S[v,c] colw[v,c']: a warp sum each, then the warps in order
+#pragma unroll
+        for (int c = 0; c < CC; ++c) {
+            if (c < r.C) {
+                const int cc = r.Cr == 1 ? 0 : c;
+                float q = s[0][c] * (float)cw[0][cc];
+#pragma unroll
+                for (int k = 1; k < BRL_VPT; ++k) q = fmaf(s[k][c], (float)cw[k][cc], q);
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) q += __shfl_xor_sync(0xffffffffu, q, o);
+                if (lane == 0) so[warp * CC + c] = q;
+            }
+        }
+        __syncthreads();
+        for (int i = tid; i < nbins * r.C; i += NT) {                      // Q[b] in full (empty bins: 0), coalesced
+            const int d = i / r.C, c = i - d * r.C;
+            float q = 0.f;
+            for (int w = 0; w < NW; ++w) q += sq[w * nq + d * CC + c];
+            r.Q[(int64_t)b * nbins * r.C + i] = q;
+        }
+        if (tid < r.C) {
+            float q = 0.f;
+            for (int w = 0; w < NW; ++w) q += so[w * CC + tid];
+            r.out[b * r.C + tid] = q;
+        }
+        __syncthreads();                                                   // the next graph rewrites the shared memory
     }
     if (max_level && tid == 0 && lvl_max > 0) atomicMax(max_level, lvl_max);   // lvl_max is uniform over the CTA
 }
@@ -1033,10 +1298,10 @@ static int classify_by_size(const int32_t *node_off, int32_t B, int32_t max_n, i
 // v3 launch on classes 0..3 of order_ws: groups of 4 warps; the group's slice holds one graph of 65..128 nodes, two of 33..64 or
 // four of up to 32. max_n (at most 128) sizes the slices.
 // CC > 0: the BFS fused with the graph readout (bv3_readout_run; ro holds its tensors, hop / cnt / rscale are NULL)
-template <bool LOCAL, int CC = 0>
+template <bool LOCAL, int CC = 0, typename IT = uint8_t>
 static int launch_bv3(const int32_t *rowptr, const int32_t *col, const int32_t *node_off, const int64_t *hop_off, int32_t B, int32_t max_n,
                       uint8_t *hop, int32_t *cnt, float *rscale, int nb, bool levels, int32_t *overflow_flag, int32_t *max_level,
-                      const int32_t *order_ws, Bv3Edges le, cudaStream_t st, Bv3Readout ro = Bv3Readout{})
+                      const int32_t *order_ws, Bv3EdgesT<IT> le, cudaStream_t st, Bv3Readout ro = Bv3Readout{})
 {
     const int Wmax = (max_n + 31) / 32;
     auto need = [&](int cap, int W, int G) {
@@ -1048,7 +1313,7 @@ static int launch_bv3(const int32_t *rowptr, const int32_t *col, const int32_t *
     const int gpc = (int)std::min<size_t>(bv3_max_groups(CC), (112 * 1024) / slice);     // two CTAs per SM
     if (gpc < 1) return GNAN_ERR_UNSUPPORTED;
     const size_t smem3 = slice * gpc;
-    auto kernel = apsp_batched_v3_kernel<LOCAL, CC>;
+    auto kernel = apsp_batched_v3_kernel<LOCAL, CC, IT>;
     static thread_local size_t cached_smem3 = 0;
     static thread_local int cached_gpc = 0, cached_per_sm3 = 0;
     if (cached_smem3 != smem3 || cached_gpc != gpc || cached_per_sm3 == 0) {
@@ -1066,14 +1331,14 @@ static int launch_bv3(const int32_t *rowptr, const int32_t *col, const int32_t *
 // graphs of more than 128 nodes in the batch: class 4 of bv3_classify_kernel (the caller has run it into order_ws [5*B+5]).
 // B bounds the number of such graphs; CTAs past the end of the class exit at once.
 static int launch_batched_large(const int32_t *rowptr, const int32_t *col, const int32_t *node_off, const int64_t *hop_off, int32_t B,
-                                uint8_t *hop, int32_t *cnt, int nb, int32_t *overflow_flag, int32_t *max_level, const int32_t *order_ws,
-                                cudaStream_t st)
+                                uint8_t *hop, int32_t *cnt, float *rscale, int nb, int32_t *overflow_flag, int32_t *max_level,
+                                const int32_t *order_ws, cudaStream_t st)
 {
     static thread_local int per_sm = 0;
     if (per_sm == 0) GNAN_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, apsp_batched_large_kernel, BL_THREADS, 0));
     const int blocks = (int)std::min<int64_t>(B, (int64_t)std::max(per_sm, 1) * gnan_sm_count());
-    apsp_batched_large_kernel<<<blocks, BL_THREADS, 0, st>>>(rowptr, col, node_off, hop_off, B, hop, cnt, nb, overflow_flag, max_level,
-                                                             order_ws);
+    apsp_batched_large_kernel<<<blocks, BL_THREADS, 0, st>>>(rowptr, col, node_off, hop_off, B, hop, cnt, rscale, nb, overflow_flag,
+                                                             max_level, order_ws);
     GNAN_LAUNCH_OK();
     return GNAN_OK;
 }
@@ -1089,10 +1354,6 @@ extern "C" int gnan_apsp_bfs_batched_ex(const int32_t *rowptr, const int32_t *co
     GNAN_REQUIRE(rowptr && node_off && hop_off && hop && overflow_flag, "apsp_bfs_batched: NULL pointer");
     GNAN_REQUIRE(order_ws, "apsp_bfs_batched: NULL order_ws");
     GNAN_REQUIRE(!(cnt || rscale) || (nbins >= 2 && nbins <= 256), "apsp_bfs_batched: nbins %d out of [2,256]", nbins);
-    if (rscale && max_n > 32 * BV3_MAX_W) {
-        gnan_set_error("apsp_bfs_batched: the fused 1/count output needs graphs of at most %d nodes", 32 * BV3_MAX_W);
-        return GNAN_ERR_UNSUPPORTED;
-    }
     if (max_n < 1 || max_n > GNAN_APSP_BATCHED_MAX_NODES) {
         gnan_set_error("apsp_bfs_batched: graphs with %d nodes unsupported (1..%d = GNAN_APSP_BATCHED_MAX_NODES); use gnan_apsp_bfs",
                        max_n, GNAN_APSP_BATCHED_MAX_NODES);
@@ -1107,7 +1368,7 @@ extern "C" int gnan_apsp_bfs_batched_ex(const int32_t *rowptr, const int32_t *co
                            overflow_flag, max_level, order_ws, Bv3Edges{}, st);
     if (rc == GNAN_ERR_UNSUPPORTED) gnan_set_error("apsp_bfs_batched: level table too wide for the shared-memory slice");
     if (rc != GNAN_OK || max_n <= 32 * BV3_MAX_W) return rc;
-    return launch_batched_large(rowptr, col, node_off, hop_off, B, hop, cnt, nb, overflow_flag, max_level, order_ws, st);
+    return launch_batched_large(rowptr, col, node_off, hop_off, B, hop, cnt, rscale, nb, overflow_flag, max_level, order_ws, st);
 }
 
 // The batched BFS straight from the batch's edge list in its transfer form (no CSR): see include/gnan_b200.h
@@ -1138,39 +1399,86 @@ extern "C" int gnan_apsp_bfs_batched_local(const uint8_t *src, const uint8_t *ds
     return rc;
 }
 
-// The batched BFS fused with the output-normalised graph readout, straight from the batch's edge list: see include/gnan_b200.h
-extern "C" int gnan_bfs_graph_readout_fwd(const uint8_t *src, const uint8_t *dst, const int32_t *edge_off, const int32_t *node_off,
-                                          int32_t B, int32_t max_n, int32_t nbins, const float *T, int32_t Cr, const float *S, int32_t C,
-                                          float *out, float *colw, float *Q, int32_t *status, int32_t *overflow_flag, int32_t *max_level,
-                                          int32_t *order_ws, gnan_stream_t stream)
+// graphs of more than 128 nodes of a fused readout batch: class 4 of order_ws [5*B+5], one CTA each, sized by max_n
+template <typename IT, int CC>
+static int launch_readout_large(Bv3EdgesT<IT> le, const int32_t *node_off, int32_t B, int32_t max_n, int nbins, const Bv3Readout &ro,
+                                int32_t *overflow_flag, int32_t *max_level, const int32_t *order_ws, cudaStream_t st)
 {
-    GNAN_REQUIRE(B >= 0, "bfs_graph_readout_fwd: negative batch");
-    GNAN_REQUIRE(status != nullptr, "bfs_graph_readout_fwd: NULL status");
+    const int nt = brl_threads(max_n);
+    const size_t smem = brl_need(max_n, nt, nbins, CC);
+    auto kernel = bfs_readout_large_kernel<IT, CC>;
+    static thread_local size_t cached_smem = 0;
+    static thread_local int cached_nt = 0, per_sm = 0;
+    if (cached_smem != smem || cached_nt != nt || per_sm == 0) {
+        GNAN_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        GNAN_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, nt, smem));
+        cached_smem = smem; cached_nt = nt;
+    }
+    if (per_sm < 1) return GNAN_ERR_UNSUPPORTED;
+    const int blocks = (int)std::min<int64_t>(B, (int64_t)per_sm * gnan_sm_count());
+    kernel<<<blocks, nt, smem, st>>>(le.src, le.dst, le.edge_off, node_off, B, max_n, nbins, ro, le.status, overflow_flag, max_level,
+                                     order_ws);
+    GNAN_LAUNCH_OK();
+    return GNAN_OK;
+}
+
+// The batched BFS fused with the output-normalised graph readout, straight from the batch's edge list: graphs of at most 128 nodes
+// on the v3 kernel, larger ones (up to max_cap) on bfs_readout_large_kernel. See include/gnan_b200.h
+template <typename IT>
+static int bfs_graph_readout(const char *who, int max_cap, const IT *src, const IT *dst, const int32_t *edge_off, const int32_t *node_off,
+                             int32_t B, int32_t max_n, int32_t nbins, const float *T, int32_t Cr, const float *S, int32_t C, float *out,
+                             float *colw, float *Q, int32_t *status, int32_t *overflow_flag, int32_t *max_level, int32_t *order_ws,
+                             cudaStream_t st)
+{
+    GNAN_REQUIRE(B >= 0, "%s: negative batch", who);
+    GNAN_REQUIRE(status != nullptr, "%s: NULL status", who);
     if (!gnan_aggregate_blockdiag_graph_supported(nbins, Cr, C)) {
-        gnan_set_error("bfs_graph_readout_fwd: needs 2 <= nbins <= 64, C <= 4, Cr in {1,C} (nbins=%d Cr=%d C=%d)", nbins, Cr, C);
+        gnan_set_error("%s: needs 2 <= nbins <= 64, C <= 4, Cr in {1,C} (nbins=%d Cr=%d C=%d)", who, nbins, Cr, C);
         return GNAN_ERR_UNSUPPORTED;
     }
-    cudaStream_t st = (cudaStream_t)stream;
+    if (B > 0 && (max_n < 1 || max_n > max_cap)) {
+        gnan_set_error("%s: graphs with %d nodes unsupported (1..%d)", who, max_n, max_cap);
+        return GNAN_ERR_UNSUPPORTED;
+    }
     GNAN_CUDA(cudaMemsetAsync(status, 0, sizeof(int32_t), st));
     if (B == 0) return GNAN_OK;
     // src / dst are read only inside the graphs' edge segments: NULL is fine for a batch without edges (an empty edge list)
-    GNAN_REQUIRE(edge_off && node_off && T && S && out && colw && Q && overflow_flag && order_ws, "bfs_graph_readout_fwd: NULL pointer");
-    if (max_n < 1 || max_n > 32 * BV3_MAX_W) {
-        gnan_set_error("bfs_graph_readout_fwd: graphs with %d nodes unsupported (1..%d)", max_n, 32 * BV3_MAX_W);
-        return GNAN_ERR_UNSUPPORTED;
-    }
-    const Bv3Edges le{src, dst, edge_off, status};
+    GNAN_REQUIRE(edge_off && node_off && T && S && out && colw && Q && overflow_flag && order_ws, "%s: NULL pointer", who);
+    const Bv3EdgesT<IT> le{src, dst, edge_off, status};
     const Bv3Readout ro{T, S, Cr, C, out, colw, Q};
+    const int small_n = std::min(max_n, 32 * BV3_MAX_W);
     auto launch = [&](auto cc) {
-        return launch_bv3<true, decltype(cc)::value>(nullptr, nullptr, node_off, nullptr, B, max_n, nullptr, nullptr, nullptr, nbins, false,
-                                                     overflow_flag, max_level, order_ws, le, st, ro);
+        constexpr int CC = decltype(cc)::value;
+        int rc = launch_bv3<true, CC, IT>(nullptr, nullptr, node_off, nullptr, B, small_n, nullptr, nullptr, nullptr, nbins, false,
+                                          overflow_flag, max_level, order_ws, le, st, ro);
+        if (rc == GNAN_OK && max_n > 32 * BV3_MAX_W)
+            rc = launch_readout_large<IT, CC>(le, node_off, B, max_n, nbins, ro, overflow_flag, max_level, order_ws, st);
+        return rc;
     };
     int rc = classify_by_size(node_off, B, max_n, order_ws, st);
     if (rc != GNAN_OK) return rc;
     rc = C == 1 ? launch(std::integral_constant<int, 1>{}) : C == 2 ? launch(std::integral_constant<int, 2>{})
                                                                    : launch(std::integral_constant<int, 4>{});
-    if (rc == GNAN_ERR_UNSUPPORTED) gnan_set_error("bfs_graph_readout_fwd: per-graph state too large for the shared-memory slice");
+    if (rc == GNAN_ERR_UNSUPPORTED) gnan_set_error("%s: per-graph state too large for shared memory", who);
     return rc;
+}
+
+extern "C" int gnan_bfs_graph_readout_fwd(const uint8_t *src, const uint8_t *dst, const int32_t *edge_off, const int32_t *node_off,
+                                          int32_t B, int32_t max_n, int32_t nbins, const float *T, int32_t Cr, const float *S, int32_t C,
+                                          float *out, float *colw, float *Q, int32_t *status, int32_t *overflow_flag, int32_t *max_level,
+                                          int32_t *order_ws, gnan_stream_t stream)
+{
+    return bfs_graph_readout<uint8_t>("bfs_graph_readout_fwd", 256, src, dst, edge_off, node_off, B, max_n, nbins, T, Cr, S, C, out,
+                                      colw, Q, status, overflow_flag, max_level, order_ws, (cudaStream_t)stream);
+}
+
+extern "C" int gnan_bfs_graph_readout_fwd_i16(const int16_t *src, const int16_t *dst, const int32_t *edge_off, const int32_t *node_off,
+                                              int32_t B, int32_t max_n, int32_t nbins, const float *T, int32_t Cr, const float *S,
+                                              int32_t C, float *out, float *colw, float *Q, int32_t *status, int32_t *overflow_flag,
+                                              int32_t *max_level, int32_t *order_ws, gnan_stream_t stream)
+{
+    return bfs_graph_readout<int16_t>("bfs_graph_readout_fwd_i16", GNAN_APSP_BATCHED_MAX_NODES, src, dst, edge_off, node_off, B, max_n,
+                                      nbins, T, Cr, S, C, out, colw, Q, status, overflow_flag, max_level, order_ws, (cudaStream_t)stream);
 }
 
 extern "C" int gnan_hops_to_reference(const uint8_t *hop, int64_t R, int64_t N, int64_t ld_hop, const int32_t *cnt,

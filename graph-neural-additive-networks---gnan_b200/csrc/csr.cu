@@ -76,9 +76,10 @@ __global__ void csr_duplicates_long_kernel(const int32_t *__restrict__ rowptr, c
     }
 }
 
-// edge list of a batch of small graphs from its compact transfer form: endpoints as uint8 indices inside their graph, the graph
-// of edge e found by a binary search in the per-graph edge offsets (B + 1 int32 values: L1 / L2 resident)
-__global__ void edges_from_local_kernel(const uint8_t *__restrict__ src, const uint8_t *__restrict__ dst,
+// edge list of a batch of small graphs from its compact transfer form: endpoints as uint8 (or int16) indices inside their graph,
+// the graph of edge e found by a binary search in the per-graph edge offsets (B + 1 int32 values: L1 / L2 resident)
+template <typename IT>
+__global__ void edges_from_local_kernel(const IT *__restrict__ src, const IT *__restrict__ dst,
                                         const int32_t *__restrict__ edge_off, const int32_t *__restrict__ node_off, int32_t B, int64_t E,
                                         int64_t *__restrict__ out)
 {
@@ -94,18 +95,32 @@ __global__ void edges_from_local_kernel(const uint8_t *__restrict__ src, const u
     out[E + e] = base + dst[e];
 }
 
+template <typename IT>
+int edges_from_local(const char *who, const IT *src, const IT *dst, const int32_t *edge_off, const int32_t *node_off, int32_t B, int64_t E,
+                     int64_t *edge_index, gnan_stream_t stream)
+{
+    GNAN_REQUIRE(B >= 0 && E >= 0, "%s: negative sizes", who);
+    GNAN_REQUIRE(E == 0 || (B > 0 && src && dst && edge_off && node_off && edge_index), "%s: NULL pointer", who);
+    if (E) {
+        edges_from_local_kernel<IT><<<(unsigned)ceil_div64(E, 256), 256, 0, (cudaStream_t)stream>>>(src, dst, edge_off, node_off, B, E,
+                                                                                                  edge_index);
+        GNAN_LAUNCH_OK();
+    }
+    return GNAN_OK;
+}
+
 }  // namespace
 
 extern "C" int gnan_edges_from_local(const uint8_t *src, const uint8_t *dst, const int32_t *edge_off, const int32_t *node_off, int32_t B,
                                      int64_t E, int64_t *edge_index, gnan_stream_t stream)
 {
-    GNAN_REQUIRE(B >= 0 && E >= 0, "edges_from_local: negative sizes");
-    GNAN_REQUIRE(E == 0 || (B > 0 && src && dst && edge_off && node_off && edge_index), "edges_from_local: NULL pointer");
-    if (E) {
-        edges_from_local_kernel<<<(unsigned)ceil_div64(E, 256), 256, 0, (cudaStream_t)stream>>>(src, dst, edge_off, node_off, B, E, edge_index);
-        GNAN_LAUNCH_OK();
-    }
-    return GNAN_OK;
+    return edges_from_local("edges_from_local", src, dst, edge_off, node_off, B, E, edge_index, stream);
+}
+
+extern "C" int gnan_edges_from_local_i16(const int16_t *src, const int16_t *dst, const int32_t *edge_off, const int32_t *node_off,
+                                         int32_t B, int64_t E, int64_t *edge_index, gnan_stream_t stream)
+{
+    return edges_from_local("edges_from_local_i16", src, dst, edge_off, node_off, B, E, edge_index, stream);
 }
 
 extern "C" size_t gnan_build_csr_workspace_bytes(int32_t N, int64_t E)

@@ -499,9 +499,9 @@ agg_bd_graph_fwd.register_autograd(_bdg_backward, setup_context=_bdg_setup)
 
 
 def bfs_graph_readout_fwd(edges, node_off: Tensor, max_n: int, T: Tensor, S: Tensor, status: Tensor) -> Tuple[Tensor, Tensor, Tensor]:
-    """The batched BFS of a LocalEdges batch fused with the output-normalised graph readout (gnan_bfs_graph_readout_fwd): the
-    (out, colw, Q) of agg_bd_graph_fwd on the batch's hop bytes and normaliser table, without writing either. status: the batch's
-    device int32 [3] (edge status bits, overflow flag, largest hop), filled as apsp_batched's BFS fills it."""
+    """The batched BFS of a LocalEdges batch fused with the output-normalised graph readout (gnan_bfs_graph_readout_fwd, or _i16 for
+    int16 endpoints): the (out, colw, Q) of agg_bd_graph_fwd on the batch's hop bytes and normaliser table, without writing either.
+    status: the batch's device int32 [3] (edge status bits, overflow flag, largest hop), filled as apsp_batched's BFS fills it."""
     lib = load()
     T, S = _f32(T, "T"), _f32(S, "S")
     if node_off.dtype != torch.int32 or status.dtype != torch.int32 or status.numel() != 3:
@@ -512,11 +512,15 @@ def bfs_graph_readout_fwd(edges, node_off: Tensor, max_n: int, T: Tensor, S: Ten
     out = torch.empty(B, C, dtype=torch.float32, device=S.device)
     colw = torch.empty(N, Cr, dtype=torch.float32, device=S.device)
     Q = torch.empty(B, nbins, C, dtype=torch.float32, device=S.device)
-    order_ws = torch.empty(4 * B + 4, dtype=torch.int32, device=S.device)
+    # scratch of the size classes (a fifth class, one CTA per graph, above 128 nodes)
+    order_ws = torch.empty(5 * B + 5 if max_n > 128 else 4 * B + 4, dtype=torch.int32, device=S.device)
+    name = {torch.uint8: "gnan_bfs_graph_readout_fwd", torch.int16: "gnan_bfs_graph_readout_fwd_i16"}.get(edges.src.dtype)
+    if name is None:
+        raise TypeError(f"bfs_graph_readout_fwd: endpoints must be uint8 or int16, got {edges.src.dtype}")
     with _timed("bfs_graph_readout_fwd"):
-        check(lib.gnan_bfs_graph_readout_fwd(ptr(edges.src), ptr(edges.dst), ptr(edges.edge_off), ptr(node_off), B, int(max_n), nbins, ptr(T),
-                                             Cr, ptr(S), C, ptr(out), ptr(colw), ptr(Q), status.data_ptr(), status.data_ptr() + 4,
-                                             status.data_ptr() + 8, ptr(order_ws), stream_handle()), "gnan_bfs_graph_readout_fwd")
+        check(getattr(lib, name)(ptr(edges.src), ptr(edges.dst), ptr(edges.edge_off), ptr(node_off), B, int(max_n), nbins, ptr(T), Cr, ptr(S),
+                                 C, ptr(out), ptr(colw), ptr(Q), status.data_ptr(), status.data_ptr() + 4, status.data_ptr() + 8,
+                                 ptr(order_ws), stream_handle()), name)
     return out, colw, Q
 
 

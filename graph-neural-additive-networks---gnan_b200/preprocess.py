@@ -287,7 +287,7 @@ class PackedBatch:
 
 class _DeferredBatch(PackedBatch):
     """What apsp_batched returns for the configuration of a training step that preprocesses its own batch (LocalEdges, nbins,
-    rscale=True, graphs of at most 128 nodes): the batched BFS has not run yet. models.TensorGNAN's output-normalised graph readout
+    rscale=True, graphs of up to 1024 nodes): the batched BFS has not run yet. models.TensorGNAN's output-normalised graph readout
     consumes the edge segments `edges` directly (ops.bfs_graph_readout: the BFS and the readout in one kernel, neither hop bytes
     nor a normaliser table in memory). The first read of `hop` or `level_rscale` runs the batched BFS once, exactly as
     apsp_batched runs it otherwise, and keeps the result; `deferred` is False from then on."""
@@ -329,25 +329,33 @@ class _DeferredBatch(PackedBatch):
 
 
 class LocalEdges:
-    """The edge list of a batch of small graphs as it should cross PCIe: src / dst uint8 [E] = node indices INSIDE the edge's
-    graph, edge_off int32 [B+1] = first edge of every graph (edges grouped by graph). 2 bytes per directed edge instead of the
-    16 of PyG's int64 [2,E] (batched_pyg_main.py:54-91 hands the model the latter). `expand` rebuilds the global int64
-    edge_index on the device (gnan_edges_from_local), bit-identical up to the order of the graphs' edge groups."""
+    """The edge list of a batch of graphs as it should cross PCIe: src / dst [E] = node indices INSIDE the edge's graph, edge_off
+    int32 [B+1] = first edge of every graph (edges grouped by graph). uint8 endpoints (graphs of up to 256 nodes) take 2 bytes per
+    directed edge, int16 endpoints (up to _lib.APSP_BATCHED_MAX_NODES = 1024 nodes: Mutagenicity, PROTEINS) 4, instead of the 16
+    of PyG's int64 [2,E] (batched_pyg_main.py:54-91 hands the model the latter). `expand` rebuilds the global int64 edge_index on
+    the device (gnan_edges_from_local / _i16), bit-identical up to the order of the graphs' edge groups."""
+
+    MAX_NODES = {torch.uint8: 256, torch.int16: _lib.APSP_BATCHED_MAX_NODES}     # largest graph each endpoint width addresses
 
     def __init__(self, src, dst, edge_off):
         self.src, self.dst, self.edge_off = src, dst, edge_off
 
     @classmethod
-    def from_edge_index(cls, edge_index, node_off):
-        """Host-side, once per batch / dataset. edge_index int64 [2,E] with global ids, node_off [B+1]. Edges are grouped by the
-        graph of their source (stable: the order inside a graph is kept); an edge across graphs or a graph of more than 256
-        nodes raises."""
+    def from_edge_index(cls, edge_index, node_off, dtype=torch.uint8):
+        """Host-side, once per batch / dataset. edge_index int64 [2,E] with global ids, node_off [B+1], dtype the endpoint width
+        (torch.uint8 or torch.int16). Edges are grouped by the graph of their source (stable: the order inside a graph is kept); an
+        edge across graphs or a graph larger than the width addresses (256 nodes for uint8, 1024 for int16) raises."""
         import numpy as np
+        if dtype not in cls.MAX_NODES:
+            raise TypeError(f"LocalEdges: endpoint dtype must be torch.uint8 or torch.int16, got {dtype}")
+        cap = cls.MAX_NODES[dtype]
         ei = torch.as_tensor(edge_index).cpu().numpy().astype(np.int64)
         no = np.asarray(torch.as_tensor(node_off).cpu().numpy(), dtype=np.int64)
         B = no.shape[0] - 1
-        if B > 0 and int((no[1:] - no[:-1]).max()) > 256:
-            raise ValueError("LocalEdges: graphs of more than 256 nodes")
+        largest = int((no[1:] - no[:-1]).max()) if B > 0 else 0
+        if largest > cap:
+            hint = f"; dtype=torch.int16 takes up to {cls.MAX_NODES[torch.int16]}" if dtype == torch.uint8 else ""
+            raise ValueError(f"LocalEdges: a graph of {largest} nodes, {dtype} endpoints address at most {cap}{hint}")
         g = np.searchsorted(no, ei[0], side="right") - 1
         if ei.shape[1] and (ei.min() < 0 or ei.max() >= no[-1] or np.any(np.searchsorted(no, ei[1], side="right") - 1 != g)):
             raise ValueError("LocalEdges: an edge leaves its graph or the node range")
@@ -357,15 +365,20 @@ class LocalEdges:
         edge_off = np.zeros(B + 1, dtype=np.int64)
         np.cumsum(np.bincount(g, minlength=B), out=edge_off[1:])
         base = no[g]
-        return cls(torch.from_numpy((ei[0] - base).astype(np.uint8)), torch.from_numpy((ei[1] - base).astype(np.uint8)),
+        npt = np.uint8 if dtype == torch.uint8 else np.int16
+        return cls(torch.from_numpy((ei[0] - base).astype(npt)), torch.from_numpy((ei[1] - base).astype(npt)),
                    torch.from_numpy(edge_off.astype(np.int32)))
 
     @property
     def num_edges(self):
         return self.src.numel()
 
+    @property
+    def dtype(self):
+        return self.src.dtype
+
     def nbytes(self):
-        return self.src.numel() + self.dst.numel() + 4 * self.edge_off.numel()
+        return (self.src.numel() + self.dst.numel()) * self.src.element_size() + 4 * self.edge_off.numel()
 
     def to(self, device):
         return LocalEdges(*[t.to(device, non_blocking=True) for t in (self.src, self.dst, self.edge_off)])
@@ -384,8 +397,9 @@ class LocalEdges:
             out = torch.empty(2, E, dtype=torch.int64, device=self.src.device)
         elif out.shape != (2, E) or out.dtype != torch.int64 or not out.is_contiguous():
             raise TypeError("LocalEdges.expand: out must be contiguous int64 [2,E]")
-        check(lib.gnan_edges_from_local(ptr(self.src), ptr(self.dst), ptr(self.edge_off), ptr(node_off.contiguous()), B, E, ptr(out),
-                                        stream_handle()), "gnan_edges_from_local")
+        name = "gnan_edges_from_local" if self.src.dtype == torch.uint8 else "gnan_edges_from_local_i16"
+        check(getattr(lib, name)(ptr(self.src), ptr(self.dst), ptr(self.edge_off), ptr(node_off.contiguous()), B, E, ptr(out),
+                                 stream_handle()), name)
         return out
 
 
@@ -409,23 +423,24 @@ def apsp_batched(edge_index, node_off, device="cuda", x=None, y=None, node_off_d
     in the batched BFS, each by its own size: up to 128 nodes on groups of 4 warps, more on one CTA each. A batch with a larger
     graph goes through per-graph `apsp` calls in the free mode (slow, one synchronisation per graph) and raises ValueError in the
     fixed-width mode (nbins=...), before any launch. edge_index may also be a `LocalEdges` (the batch's edge list
-    in its transfer form): batches of graphs with at most 128 nodes then skip the CSR builder altogether — every 4-warp group of
-    the BFS kernel builds its graph's adjacency bit matrix in shared memory from the graph's own edge segment
-    (gnan_apsp_bfs_batched_local); other batches expand it to the int64 list first.
+    in its transfer form): batches of graphs with at most 128 nodes in uint8 endpoints then skip the CSR builder altogether — every
+    4-warp group of the BFS kernel builds its graph's adjacency bit matrix in shared memory from the graph's own edge segment
+    (gnan_apsp_bfs_batched_local); other batches (int16 endpoints, larger graphs) expand it to the int64 list first.
 
     nbins: fixed level-table width (levels 0..nbins-2, last column = unreachable). The call then never synchronises with the
     host (it can be captured in a CUDA graph with the rest of a training step); empty levels carry a zero count and
     contribute nothing. The returned batch has `.status` (device int32 [3]: CSR status, overflow flag, largest hop) to be
     checked lazily with check_batched_status. hop_off_device: optional int64 device copy of the block offsets
     (cumsum of n_b^2, B+1 entries; with node_off_device it removes every host -> device copy from the call).
-    rscale=True (fixed-width mode, graphs of at most 128 nodes): the BFS writes the output normaliser 1/level_counts
+    rscale=True (fixed-width mode, graphs of up to _lib.APSP_BATCHED_MAX_NODES nodes): the BFS writes the output normaliser 1/level_counts
     (`PackedBatch.level_rscale`, fp32) INSTEAD of the int32 level counts, which the output-normalised models
     (models.TensorGNAN, normalize_rho=True) consume directly: one table written, none converted.
     With a `LocalEdges` input the distances are DEFERRED: the call launches nothing and returns a batch
     that holds the edge segments (`deferred` is True). models.TensorGNAN's output-normalised graph readout then runs the BFS and
     the readout as one kernel (ops.bfs_graph_readout) and never materialises hop bytes or the normaliser table; the first read of
-    `hop` or `level_rscale` runs this BFS once and caches both. `status` is the same device word either way, filled by the
-    first kernel that consumes the edges (check it after the forward).
+    `hop` or `level_rscale` runs this BFS once and caches both (int16 endpoints or a graph over 128 nodes: after expanding the
+    edge list and building its CSR, as for an int64 input). Either endpoint width and graphs of up to 1024 nodes defer. `status`
+    is the same device word either way, filled by the first kernel that consumes the edges (check it after the forward).
     pair_stats=True (`LocalEdges` input only) returns the same deferred batch as rscale=True: the pair statistics of the graph
     readout are formed only inside the fused BFS + readout kernel.
 
@@ -459,15 +474,17 @@ def apsp_batched(edge_index, node_off, device="cuda", x=None, y=None, node_off_d
     hop_off = hop_off_device if hop_off_device is not None else torch.from_numpy(hop_off_h).to(device, non_blocking=True)
     st = torch.zeros(3, dtype=torch.int32, device=device)              # [csr status, overflow, largest finite hop]
     local = None
+    deferred = isinstance(edge_index, LocalEdges) and bool(rscale or pair_stats)
     if isinstance(edge_index, LocalEdges):
         if not edge_index.src.is_cuda:
             edge_index = edge_index.to(device)
-        if max_n <= 128 and sumN > 0 and B > 0:
+        if max_n <= 128 and sumN > 0 and B > 0 and edge_index.dtype == torch.uint8:
             local = edge_index
-        else:
+        elif not deferred:
             edge_index = edge_index.expand(node_off_d)
-    if local is None:
-        rowptr, col, _ = build_csr(edge_index, sumN, device, status=st[0:1])
+    csr = []                                     # rowptr, col (a deferred batch builds them when it materialises)
+    if local is None and not deferred:
+        csr[:] = build_csr(edge_index, sumN, device, status=st[0:1])[:2]
 
     def bfs(hop, cnt_t, rs_t):
         # scratch of the size classes the BFS groups the graphs by (a fifth class above 128 nodes)
@@ -477,6 +494,7 @@ def apsp_batched(edge_index, node_off, device="cuda", x=None, y=None, node_off_d
                                                   ptr(hop), ptr(cnt_t), ptr(rs_t), nb, st.data_ptr(), st.data_ptr() + 4, st.data_ptr() + 8,
                                                   ptr(order_ws), stream_handle()), "gnan_apsp_bfs_batched_local")
         else:
+            rowptr, col = csr
             check(lib.gnan_apsp_bfs_batched_ex(ptr(rowptr), ptr(col), ptr(node_off_d), ptr(hop_off), B, max_n, ptr(hop), ptr(cnt_t),
                                                ptr(rs_t), nb, st.data_ptr() + 4, st.data_ptr() + 8, ptr(order_ws), stream_handle()),
                   "gnan_apsp_bfs_batched_ex")
@@ -484,19 +502,22 @@ def apsp_batched(edge_index, node_off, device="cuda", x=None, y=None, node_off_d
     nb = min(nb_full, _level_table_width) if _level_table_width else nb_full
     if nbins is not None:
         nb = int(nbins)
-    if pair_stats and (local is None or nbins is None):
-        raise ValueError("pair_stats=True needs a LocalEdges edge list, graphs of at most 128 nodes and the fixed-width mode (nbins=...)")
+    cap = _lib.APSP_BATCHED_MAX_NODES
+    if pair_stats and (not deferred or nbins is None):
+        raise ValueError(f"pair_stats=True needs a LocalEdges edge list, graphs of at most {cap} nodes and the fixed-width mode (nbins=...)")
     if rscale or pair_stats:
-        if nbins is None or max_n > 128 or sumN == 0:
-            raise ValueError("rscale=True needs the fixed-width mode (nbins=...) and graphs of at most 128 nodes")
-        if local is not None:
+        if nbins is None or sumN == 0:
+            raise ValueError(f"rscale=True needs the fixed-width mode (nbins=...), graphs of at most {cap} nodes and at least one node")
+        if deferred:
             def materialise():
+                if local is None:                # int16 endpoints or a graph over 128 nodes: the int64 list and its CSR first
+                    csr[:] = build_csr(edge_index.expand(node_off_d), sumN, device, status=st[0:1])[:2]
                 hop = torch.empty(max(total, 1), dtype=torch.uint8, device=device)
                 rs = torch.empty(sumN, nb, dtype=torch.float32, device=device)
                 with _timed("apsp_bfs_batched"):
                     bfs(hop, None, rs)
                 return hop, rs
-            pk = _DeferredBatch(x, hop_off, node_off_d, y, max_n, nb, local, materialise)
+            pk = _DeferredBatch(x, hop_off, node_off_d, y, max_n, nb, edge_index, materialise)
             pk.status = st
             return pk
         hop = torch.empty(max(total, 1), dtype=torch.uint8, device=device)

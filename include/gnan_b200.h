@@ -310,6 +310,9 @@ int gnan_build_csr(const int64_t *src, const int64_t *dst, int64_t E, int32_t N,
  * takes): 2 bytes per directed edge cross PCIe instead of 16 (batched_pyg_main.py:54-91 loader output). */
 int gnan_edges_from_local(const uint8_t *src, const uint8_t *dst, const int32_t *edge_off, const int32_t *node_off, int32_t B,
                           int64_t E, int64_t *edge_index, gnan_stream_t stream);
+/* The same with int16 endpoints (graphs of up to GNAN_APSP_BATCHED_MAX_NODES nodes; 4 bytes per directed edge). */
+int gnan_edges_from_local_i16(const int16_t *src, const int16_t *dst, const int32_t *edge_off, const int32_t *node_off, int32_t B,
+                              int64_t E, int64_t *edge_index, gnan_stream_t stream);
 
 size_t gnan_apsp_bfs_workspace_bytes(int32_t N, int32_t n_sources);
 
@@ -338,7 +341,8 @@ int gnan_apsp_msbfs(const int32_t *rowptr, const int32_t *col, int32_t N, int32_
  * Both launches go on `stream`, no synchronisation. max_n outside 1..GNAN_APSP_BATCHED_MAX_NODES: GNAN_ERR_UNSUPPORTED before any
  * CUDA call (gnan_apsp_bfs takes one graph of any size).
  * rscale (optional) [sumN,nbins] fp32 = 1/count (0 for an empty level), i.e. what gnan_level_rscale computes from cnt
- * (models.py:368-370 divides by the level size); cnt may then be NULL. Needs graphs of at most 128 nodes. */
+ * (models.py:368-370 divides by the level size); cnt may then be NULL. Bit-identical to gnan_level_rscale of cnt at every graph
+ * size: above 128 nodes the counts are summed across source chunks in the rscale rows (exact integers in fp32) and inverted once. */
 int gnan_apsp_bfs_batched_ex(const int32_t *rowptr /* [sumN+1] */, const int32_t *col, const int32_t *node_off /* [B+1] */,
                              const int64_t *hop_off /* [B+1] */, int32_t B, int32_t max_n, uint8_t *hop,
                              int32_t *cnt /* [sumN,nbins] or NULL */, float *rscale, int32_t nbins, int32_t *overflow_flag,
@@ -358,13 +362,23 @@ int gnan_apsp_bfs_batched_local(const uint8_t *src, const uint8_t *dst, const in
 /* gnan_apsp_bfs_batched_local fused with gnan_aggregate_blockdiag_graph_fwd on the output-normaliser table (models.py:366-384 with
  * normalize_rho, a global table T [nbins,Cr]): the same out [B,C], colw [sumN,Cr] and Q [B,nbins,C] (gnan_aggregate_blockdiag_graph_bwd
  * is the backward), computed inside the BFS level loop. No hop bytes, level table or pair statistics are written. Directed graphs
- * are exact too (a slower path per graph, chosen in the kernel). Same envelope as gnan_aggregate_blockdiag_graph_supported;
- * graphs of at most 128 nodes; *status (zeroed here), *overflow_flag and *max_level (optional) as gnan_apsp_bfs_batched_local.
- * Deterministic (fixed summation orders). */
+ * are exact too. Same envelope as gnan_aggregate_blockdiag_graph_supported; *status (zeroed here), *overflow_flag and *max_level
+ * (optional) as gnan_apsp_bfs_batched_local. Deterministic (fixed summation orders). Each graph runs by its own size:
+ *  - at most 128 nodes: 4-warp groups as gnan_apsp_bfs_batched_local (a slower per-graph path for directed graphs);
+ *  - 129..max_n nodes: one CTA per graph, 128 sources at a time, pulling over in-neighbours (exact for directed graphs in one pass);
+ *    the in-neighbour bit matrix lives in shared memory (max_n^2 / 8 bytes), so no graph is refused for its edge count.
+ * uint8 endpoints: max_n 1..256; order_ws [4*B+4] words, [5*B+5] when max_n > 128. A max_n outside the range is refused with
+ * GNAN_ERR_UNSUPPORTED before any CUDA call. */
 int gnan_bfs_graph_readout_fwd(const uint8_t *src, const uint8_t *dst, const int32_t *edge_off, const int32_t *node_off, int32_t B,
                                int32_t max_n, int32_t nbins, const float *T, int32_t Cr, const float *S, int32_t C, float *out,
-                               float *colw, float *Q, int32_t *status, int32_t *overflow_flag, int32_t *max_level, int32_t *order_ws,
-                               gnan_stream_t stream);
+                               float *colw, float *Q, int32_t *status, int32_t *overflow_flag, int32_t *max_level,
+                               int32_t *order_ws /* [4*B+4], [5*B+5] if max_n > 128 */, gnan_stream_t stream);
+/* The same with int16 endpoints (gnan_edges_from_local_i16's transfer form): max_n 1..GNAN_APSP_BATCHED_MAX_NODES. On the same
+ * batch the results are bit-identical to gnan_bfs_graph_readout_fwd's. */
+int gnan_bfs_graph_readout_fwd_i16(const int16_t *src, const int16_t *dst, const int32_t *edge_off, const int32_t *node_off, int32_t B,
+                                   int32_t max_n, int32_t nbins, const float *T, int32_t Cr, const float *S, int32_t C, float *out,
+                                   float *colw, float *Q, int32_t *status, int32_t *overflow_flag, int32_t *max_level,
+                                   int32_t *order_ws /* [4*B+4], [5*B+5] if max_n > 128 */, gnan_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Deep graphs (csrc/wide.cu): hop distances > 254. The reference has no depth limit (pre_process_datasets.py:109-121), so the
