@@ -23,6 +23,7 @@ constexpr int BINS_WARPS = 8;       // warps per CTA in the bins kernel (may be 
 constexpr int CHUNK_FLOATS = 4096;  // floats of S staged per sweep step: 4096 / CC columns
 constexpr int DS_THREADS = 256;
 constexpr int DS_RB = 8;            // rows per staged table group in the dS kernel
+constexpr size_t MAX_SMEM = 227 * 1024;   // dynamic shared memory one CTA may opt in to (sm_100)
 
 template <int CC> struct VecT;
 template <> struct VecT<1> { using type = float; };
@@ -391,15 +392,18 @@ agg_blockdiag_fwd_rows_kernel(BdArgs a, float *__restrict__ out)
     }
 }
 
-// backward: dS (lane owns column j), dT via shared-memory bins (per CTA for a global table, per row otherwise)
+// backward: dS (lane owns column j), dT via shared-memory bins (per CTA for a global table, per row otherwise). Without
+// SMEM_BINS the bins do not fit shared memory and the atomics go straight to dT: the caller zeroes a global table; a per-row
+// slice is zeroed by the one warp that owns the row.
+template <bool SMEM_BINS>
 __global__ void __launch_bounds__(256)
 agg_blockdiag_bwd_kernel(BdArgs a, const float *__restrict__ g, float *__restrict__ dS, float *__restrict__ dT)
 {
-    extern __shared__ float sb[];  // global table: [nbins*Cr] CTA-wide ; per-row: [8 warps][nbins*Cr]
+    extern __shared__ float sb[];  // global table: [nbins*Cr] CTA-wide ; per-row: [warps][nbins*Cr]
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     const int nT = a.nbins * a.Cr;
-    float *bins = a.per_row ? sb + w * nT : sb;
-    if (!a.per_row) {
+    float *bins = !SMEM_BINS ? dT : (a.per_row ? sb + w * nT : sb);
+    if (SMEM_BINS && !a.per_row) {
         for (int t = threadIdx.x; t < nT; t += blockDim.x) sb[t] = 0.f;
         __syncthreads();
     }
@@ -422,8 +426,10 @@ agg_blockdiag_bwd_kernel(BdArgs a, const float *__restrict__ g, float *__restric
         }
         // dT
         for (int i = 0; i < n; ++i) {
+            float *rb = bins;
             if (a.per_row) {
-                for (int t = lane; t < nT; t += 32) bins[t] = 0.f;
+                if (!SMEM_BINS) rb = dT + (int64_t)(n0 + i) * nT;
+                for (int t = lane; t < nT; t += 32) rb[t] = 0.f;
                 __syncwarp();
             }
             for (int j = lane; j < n; j += 32) {
@@ -431,17 +437,19 @@ agg_blockdiag_bwd_kernel(BdArgs a, const float *__restrict__ g, float *__restric
                 const float rs = a.rscale ? a.rscale[(int64_t)(n0 + i) * a.nbins + d] : 1.f;
                 for (int c = 0; c < a.C; ++c) {
                     const float gi = a.reduce_graph ? g[b * a.C + c] : g[(int64_t)(n0 + i) * a.C + c];
-                    atomicAdd(bins + d * a.Cr + (a.Cr == 1 ? 0 : c), rs * gi * a.S[(int64_t)(n0 + j) * a.C + c]);
+                    atomicAdd(rb + d * a.Cr + (a.Cr == 1 ? 0 : c), rs * gi * a.S[(int64_t)(n0 + j) * a.C + c]);
                 }
             }
             if (a.per_row) {
                 __syncwarp();
-                for (int t = lane; t < nT; t += 32) dT[(int64_t)(n0 + i) * nT + t] = bins[t];
-                __syncwarp();
+                if (SMEM_BINS) {
+                    for (int t = lane; t < nT; t += 32) dT[(int64_t)(n0 + i) * nT + t] = rb[t];
+                    __syncwarp();
+                }
             }
         }
     }
-    if (!a.per_row) {
+    if (SMEM_BINS && !a.per_row) {
         __syncthreads();
         for (int t = threadIdx.x; t < nT; t += blockDim.x)
             if (sb[t] != 0.f) atomicAdd(dT + t, sb[t]);
@@ -592,17 +600,21 @@ int gnan_agg_rows_fwd_cuda_cores(const uint8_t *hop, int64_t R, int64_t N, int64
     cudaStream_t st = (cudaStream_t)stream;
     AggArgs a{hop, R, N, ld_hop, T, table_per_row, nbins, Cr, rscale, S, C};
     const int CC = C >= 4 ? 4 : (C >= 2 ? 2 : 1);
-    const int WAYS = 2;
+    int ways = 2;
     int nwarps = BINS_WARPS;
-    auto smem_of = [&](int nw) { return sizeof(float) * ((size_t)CHUNK_FLOATS + 32 * CC + (size_t)CC * nw * WAYS * nbins * 32); };
+    auto smem_of = [&](int nw) { return sizeof(float) * ((size_t)CHUNK_FLOATS + 32 * CC + (size_t)CC * nw * ways * nbins * 32); };
+    if (smem_of(1) > MAX_SMEM) ways = 1;   // CC = 4 from nbins = 211 on: one bin copy per lane (148 KB at nbins = 256)
     while (nwarps > 1 && smem_of(nwarps) > 100 * 1024) nwarps >>= 1;   // keep >= 2 CTAs per SM
-    if (smem_of(nwarps) > 227 * 1024) {
+    if (smem_of(nwarps) > MAX_SMEM) {
         gnan_set_error("aggregate_rows_fwd: nbins %d too large for shared memory", nbins);
         return GNAN_ERR_UNSUPPORTED;
     }
     const size_t smem = smem_of(nwarps);
     dim3 grid((unsigned)ceil_div64(R, nwarps), (unsigned)((C + CC - 1) / CC));
-    if (CC == 4) {
+    if (CC == 4 && ways == 1) {
+        GNAN_CUDA(cudaFuncSetAttribute(agg_rows_bins_kernel<4, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        agg_rows_bins_kernel<4, 1><<<grid, BINS_WARPS * 32, smem, st>>>(a, nwarps, out, Bsum);
+    } else if (CC == 4) {
         GNAN_CUDA(cudaFuncSetAttribute(agg_rows_bins_kernel<4, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         agg_rows_bins_kernel<4, 2><<<grid, BINS_WARPS * 32, smem, st>>>(a, nwarps, out, Bsum);
     } else if (CC == 2) {
@@ -738,8 +750,21 @@ extern "C" int gnan_aggregate_blockdiag_bwd(const uint8_t *hop, const int64_t *h
         GNAN_LAUNCH_OK();
         return GNAN_OK;
     }
-    const size_t smem = sizeof(float) * (size_t)nbins * Cr * (table_per_row ? 8 : 1);
-    agg_blockdiag_bwd_kernel<<<blocks, 256, smem, st>>>(a, g, dS, dT);
+    // dT bins: one table per CTA (global) or per warp (per-row) in shared memory. Where 8 per-row tables do not fit, a CTA has
+    // fewer warps and the grid as many more CTAs; a table larger than shared memory accumulates in dT itself.
+    const size_t bins_bytes = sizeof(float) * (size_t)nbins * Cr;
+    if (bins_bytes > MAX_SMEM) {
+        agg_blockdiag_bwd_kernel<false><<<blocks, 256, 0, st>>>(a, g, dS, dT);
+        GNAN_LAUNCH_OK();
+        return GNAN_OK;
+    }
+    int warps = 8;
+    while (table_per_row && warps * bins_bytes > MAX_SMEM) warps >>= 1;
+    const size_t smem = bins_bytes * (table_per_row ? warps : 1);
+    if (smem > 48 * 1024)
+        GNAN_CUDA(cudaFuncSetAttribute(agg_blockdiag_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const int bwd_blocks = (int)std::min<int64_t>(ceil_div64(B, warps), 4 * gnan_sm_count() * (8 / warps));
+    agg_blockdiag_bwd_kernel<true><<<bwd_blocks, warps * 32, smem, st>>>(a, g, dS, dT);
     GNAN_LAUNCH_OK();
     return GNAN_OK;
 }

@@ -530,7 +530,11 @@ def test_mlp_dropout_matches_oracle_with_the_same_masks(precision):
 @pytest.mark.parametrize("R,N,C,Cr,nbins,per_row,scale", [
     (5, 7, 1, 1, 3, False, False), (37, 100, 3, 3, 6, True, False), (64, 2500, 7, 7, 12, False, True),
     (33, 4099, 4, 1, 40, False, True), (20, 300, 2, 2, 70, True, True), (129, 515, 40, 40, 9, False, False),
-    (300, 300, 5, 1, 5, True, False)])
+    (300, 300, 5, 1, 5, True, False),
+    # nbins 210 / 211 / 256 with 4-channel chunks: two lane-private bin copies per warp up to 210, one from 211 on
+    (24, 300, 4, 4, 210, False, True), (24, 300, 4, 1, 211, True, True), (12, 4099, 4, 4, 256, False, True),
+    (17, 530, 5, 5, 211, False, True), (17, 530, 5, 1, 256, True, True),
+    (9, 260, 40, 40, 210, True, True), (9, 260, 40, 40, 211, False, True), (9, 260, 40, 40, 256, True, True)])
 def test_aggregate_rows_vs_oracle(R, N, C, Cr, nbins, per_row, scale):
     from gnan_b200 import ops
     rng = np.random.default_rng(R + N)
@@ -557,6 +561,10 @@ def test_aggregate_rows_vs_oracle(R, N, C, Cr, nbins, per_row, scale):
     assert G.rel_err(Tg.grad.cpu().numpy(), Td.grad.numpy()) < TOL
     with torch.no_grad():                                   # inference path (no bin sums saved)
         assert torch.equal(ops.aggregate_rows(hop, Tg, Sg, rscale=None if rs is None else rs.to(DEV), per_row=per_row), got.detach())
+        # backward without saved bin sums: rebuilt by one extra forward pass
+        dS, dT = ops.agg_rows_bwd(hop, Tg, None if rs is None else rs.to(DEV), Sg, per_row, gO.to(DEV), torch.empty(0, device=DEV))
+    assert G.rel_err(dS.cpu().numpy(), Sd.grad.numpy()) < TOL
+    assert G.rel_err(dT.cpu().numpy(), Td.grad.numpy()) < TOL
 
 
 # tensor-core form (csrc/agg_tc.cu): TMA-streamed hop tiles, on-the-fly 0/1 operand in TMEM, tcgen05 kind::i8 against the

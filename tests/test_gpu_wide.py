@@ -80,13 +80,18 @@ def test_wide_aggregation_vs_float64(R, N, C, Cr, nbins, per_row, scale):
     assert G.rel_err(Tg.grad.cpu().numpy(), Td.grad.numpy()) < TOL
 
 
-@pytest.mark.parametrize("variant", ["GNAN.TensorGNAN", "models.TensorGNAN"])
-def test_deep_graph_module_step_vs_float64_restatement(variant):
-    """A whole forward + backward on a graph of diameter > 254 (input- and output-normalised rho), against oracle/gnan_lut.py."""
+@pytest.mark.parametrize("variant,n_chain,C", [
+    pytest.param("GNAN.TensorGNAN", 300, 3, id="GNAN.TensorGNAN"), pytest.param("models.TensorGNAN", 300, 3, id="models.TensorGNAN"),
+    # diameter 209-254: still uint8 hops, nbins > 210 on the CUDA-core row kernels with 4-channel chunks
+    pytest.param("GNAN.TensorGNAN", 230, 5, id="GNAN.TensorGNAN-uint8"),
+    pytest.param("models.TensorGNAN", 230, 5, id="models.TensorGNAN-uint8")])
+def test_deep_graph_module_step_vs_float64_restatement(variant, n_chain, C):
+    """A whole forward + backward on a graph of diameter > 254 (int16 hops), or 209-254 (uint8 hops, nbins > 210), with input-
+    and output-normalised rho, against oracle/gnan_lut.py."""
     from gnan_b200.preprocess import apsp
     rng = np.random.default_rng(11)
-    ei, n = deep_graph(rng, n_chain=300, n_extra=60)
-    K, C, H, L = 5, 3, 64, 3
+    ei, n = deep_graph(rng, n_chain=n_chain, n_extra=60)
+    K, H, L = 5, 64, 3
     x = torch.tensor(rng.normal(size=(n, K))).float()
     w = torch.tensor(rng.normal(size=(n, C))).float()
     torch.manual_seed(0)
@@ -100,7 +105,7 @@ def test_deep_graph_module_step_vs_float64_restatement(variant):
         mode, rl = "output", 2
     m.fs.xavier_normal_(1.0); m.rho.xavier_normal_(1.0)
     hd = apsp(torch.tensor(ei), n, device=DEV)
-    assert hd.wide
+    assert hd.wide if n_chain > 256 else (not hd.wide and hd.nbins > 210)
     out = m.forward(SimpleNamespace(x=x, hop_data=hd))
     (out * w.to(DEV)).sum().backward()
     hop = torch.tensor(oapsp.apsp(ei, n)).long()
